@@ -9,7 +9,7 @@ genome, every block with its own generator) is split evenly over the ranks by co
 m-mer owner (peer stores over NVLink), every rank groups the buckets it owns.  The sum of the owners' table digests is
 printed and checked against profiles/expected_digests.json: it must be the same at every N.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2] [--impl reference] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  `value` is device-resident throughput (inputs in HBM when the
 timed region starts), `e2e` goes through the public host-buffer call (pinned H2D + pipeline + D2H of
@@ -54,7 +54,14 @@ def parse_args():
     ap.add_argument("--e2e-overlapped", action="store_true", help="(default now; kept so that older command lines still parse)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the table of the last timed step as DIR/<name>.npy (float64, see dump_outputs)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's table; --impl reference computes none")
+    return a
 
 
 READ_BLOCK = 250_000  # reads per generator block of the strong-scaling read sets
@@ -299,6 +306,40 @@ class ClockSampler:
         return out
 
 
+DUMP_ROWS = 1 << 18  # rows kept per dumped array; longer arrays are sampled
+
+
+def dump_outputs(out_dir, binner, table, digest, suffix=""):
+    """Writes the pruned table of the last timed step as float64 .npy files, so that two builds can be compared output for
+    output: counts.npy (n_instances, n_distinct, n_buckets, n_kmers, n_ids), table_digest.npy (gbin_table_digest, which
+    covers the whole table), and the table's arrays mmer_codes, mmer_kmer_off, kmer_codes, kmer_id_off and read_ids.  64-bit
+    codes are split into 32-bit limbs, most significant first, so that float64 holds them exactly: kmer_codes has
+    2 * kmer_words columns.  An array longer than DUMP_ROWS rows is cut to a fixed, seeded sample of DUMP_ROWS rows, whose
+    indices go to <name>_rows.npy.  At most about 26 MiB in all."""
+    import numpy as np
+    h = binner.table_to_host(table)
+    os.makedirs(out_dir, exist_ok=True)
+
+    def limbs(x):
+        x = np.asarray(x, dtype=np.uint64)
+        return np.stack([x >> np.uint64(32), x & np.uint64(0xFFFFFFFF)], axis=-1).reshape(len(x), 2)
+
+    def save(name, a):
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+    save("counts", [h.n_instances, h.n_distinct, h.n_buckets, h.n_kmers, h.n_ids])
+    save("table_digest", limbs([digest])[0])
+    arrays = {"mmer_codes": h.mmer_codes, "mmer_kmer_off": h.mmer_kmer_off, "kmer_codes": limbs(h.kmer_codes).reshape(h.n_kmers, 2 * h.kw),
+              "kmer_id_off": h.kmer_id_off, "read_ids": h.read_ids}
+    for name, a in arrays.items():
+        assert a.dtype != np.uint64 or a.size == 0 or int(a.max()) < (1 << 53), name  # exact in float64
+        if len(a) > DUMP_ROWS:
+            rows = np.sort(np.random.default_rng(0).choice(len(a), DUMP_ROWS, replace=False))
+            save(f"{name}_rows", rows)
+            a = a[rows]
+        save(name, a)
+
+
 _REAL_STDOUT = None
 
 
@@ -452,6 +493,8 @@ def main():
                    "what": "gbin_table_digest: order-independent hash of every (m-mer, k-mer, ordered id list), summed over the owners"}
     if expected and digest != expected and rank == 0:
         print(f"bench.py: table digest {digest} differs from profiles/expected_digests.json[{dkey}] = {expected}", file=sys.stderr)
+    if a.dump_outputs:  # before the e2e leg, which reuses the context's buffers that hold the device table
+        dump_outputs(a.dump_outputs, binner, table, dg, f"_rank{rank}" if world > 1 else "")
 
     # ---- e2e: public host-buffer call, pinned H2D + pipeline + D2H of the table inside the timed region
     e2e = None
@@ -477,7 +520,7 @@ def main():
             for bb in group:
                 bb.bin_host_raw(rd_host)
             torch.cuda.synchronize()
-            per_thread = max(a.steps, 2)
+            per_thread = a.steps
 
             def worker(bb):
                 for _ in range(per_thread):
