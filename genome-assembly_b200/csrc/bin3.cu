@@ -1198,7 +1198,6 @@ uint64_t v3_max_units(uint64_t n_inst, uint64_t n_runs, int cap) {
 }
 size_t v3_unit_bytes() { return sizeof(Unit3); }
 size_t v3_unit_out_bytes() { return sizeof(UnitOut3); }
-size_t v3_counters_bytes() { return sizeof(G3Counters); }
 
 struct PtrIn64 {
     const uint64_t *p;

@@ -21,9 +21,13 @@ using namespace gbin;
 
 namespace {
 
-struct DevBuf {
+struct DevBuf {  // frees its memory when destroyed (with the context that holds it)
     void *p = nullptr;
     size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    ~DevBuf() { release(); }
     cudaError_t ensure(size_t bytes) {
         if (bytes <= cap) return cudaSuccess;
         if (p) cudaFree(p);
@@ -63,9 +67,13 @@ struct DevBuf {
     T *as() const { return static_cast<T *>(p); }
 };
 
-struct HostBuf {  // page-locked
+struct HostBuf {  // page-locked; freed when destroyed
     void *p = nullptr;
     size_t cap = 0;
+    HostBuf() = default;
+    HostBuf(const HostBuf &) = delete;
+    HostBuf &operator=(const HostBuf &) = delete;
+    ~HostBuf() { release(); }
     cudaError_t ensure(size_t bytes) {
         if (bytes <= cap) return cudaSuccess;
         if (p) cudaFreeHost(p);
@@ -83,27 +91,40 @@ struct HostBuf {  // page-locked
     }
 };
 
-struct Misc {  // small device-resident scalars
-    GroupCounts counts;
-    unsigned long long bad_bases;
-    unsigned long long total_windows;
-    unsigned int max_len;
-    unsigned int pad;
+// Small device-resident scalars (ctx->misc) and their pinned host mirror (ctx->h_misc).  Values the host needs at the same
+// point are grouped into one member, so that read_back() fetches them in one copy.
+struct Misc {
+    struct {
+        GroupCounts counts;
+        unsigned long long bad_bases;  // of pipeline 1's scan
+    } grp;
+    struct {
+        unsigned long long total_windows;
+        unsigned int max_len;
+    } reads;
     uint64_t part_counts[256];
-    // pipeline v2
+    // super-k-mer pipelines (2 and 3)
     unsigned long long skr_counters[4];  // [0] bad bases, [1] records, [2] instances
-    SkrGroupCounters gc;
-    uint32_t skr_ticket, n_inst_dev, n_runs_dev, n_buckets_dev;
-    uint32_t chunk_tickets[SKR_MAX_CHUNKS];
+    uint32_t skr_ticket, n_buckets_dev;
+    struct {
+        uint32_t n_inst, n_runs;
+    } plan;
     unsigned long long chunk_totals[SKR_MAX_CHUNKS];
-    uint32_t split_n_nl, split_n_reads;
-    // pipeline v3
+    // pipeline 2
+    SkrGroupCounters gc;
+    uint32_t chunk_tickets[SKR_MAX_CHUNKS];
+    // pipeline 3
     V3Counters gc3;
-    unsigned long long n_real_entries;
+    unsigned long long n_mmers;         // distinct m-mer codes of a batch (automatic key layout)
+    unsigned long long n_real_entries;  // entries of the sort that are not empty pieces
     uint32_t chunk_bounds[SKR_MAX_CHUNKS + 1];
     uint32_t v3_tickets[2 * SKR_MAX_CHUNKS];
     unsigned long long lsd_totals[SKR_MAX_CHUNKS];
     uint64_t v3_chunk_sum;
+    // file path and table digest
+    uint32_t split_n_nl, split_n_reads;
+    char last_byte;                     // of the file image
+    unsigned long long digest;
 };
 
 // Host path only.  HostFeed: the reads are still in host memory; the scan stage copies them chunk by chunk on the copy
@@ -123,6 +144,9 @@ struct HostSink {
     int chunks;
 };
 
+// Timing events of one call, in the order they are recorded.
+enum : int { EV_START, EV_READS_ON_DEVICE, EV_SCANNED, EV_SORTED, EV_GROUPED, EV_TABLE_ON_HOST, EV_COUNT };
+
 }  // namespace
 
 struct gbin_ctx {
@@ -137,16 +161,16 @@ struct gbin_ctx {
     int host_chunks;              // GBIN_HOST_CHUNKS (default 8; 1 = no overlap)
     char err[512];
     gbin_timings tm;
-    cudaEvent_t ev[6];
+    cudaEvent_t ev[EV_COUNT];
     // inputs staged by the host path
     DevBuf d_reads, d_starts, d_lens, d_ids;
     // pipeline workspace
     DevBuf rec_a, rec_b, radix_scratch, win_counts, rec_off, scan_scratch;
     DevBuf group_of, run_start, surv_index, id_offset, surv_group, bucket_of;
     DevBuf misc;
-    // pipeline v2 workspace
+    // workspace of the super-k-mer pipelines (2 and 3)
     DevBuf skr_a, skr_b, tile_state, inst_prefix, run_excl, skr_run_start, small_prefix, unit_base, units, unit_state, o_kmer_mmer, bucket_excl, big_list, big_k0, big_k1, big_arr, stg_ids, stg_codes, stg_mmer, stg_off, skr_side;
-    // pipeline v3 workspace
+    // pipeline 3 workspace
     DevBuf ent_a, ent_b, piece_n, sorted_info, v3_base64, v3_head_run, v3_unit_out, v3_unit_excl, v3_atoms, v3_lsd_aux, v3_bitmap;
     DevBuf x_list_off, x_ids;         // gbin_expand_read_ids_device's result
     void *donated = nullptr;          // gbin_donate_scratch: caller-owned device memory the next grouping call may use for its sort buffers
@@ -161,8 +185,8 @@ struct gbin_ctx {
     int xchg_timeout_ms = 120000;  // gbin_set_tuning "xchg_timeout_ms" / GBIN_XCHG_TIMEOUT_MS
     int pipeline;        // 3: sort by reference + warp units, falling back to 2, then 1 (default); 2: super-k-mer path with v1 as fallback; 1: v1 only
     int last_pipeline;   // which one produced the last table
-    uint32_t fallbacks;  // v2 -> v1 fallbacks since creation
-    gbin_run_stats rs;   // sizes seen by the last pipeline-2 run
+    uint32_t fallbacks;  // fallbacks to the next pipeline (3 -> 2 -> 1) since creation
+    gbin_run_stats rs;   // sizes seen by the last pipeline-2 or pipeline-3 run
     // owner exchange over peer memory (multi-GPU, one process per GPU)
     struct {
         bool created = false, attached = false;
@@ -214,6 +238,113 @@ int check_config(const gbin_config *c) {
     return GBIN_OK;
 }
 
+// Makes the context's device current and picks the call's stream: the caller's, else the context's own.
+cudaError_t begin_call(gbin_ctx *ctx, void *stream, cudaStream_t *st) {
+    *st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    return cudaSetDevice(ctx->cfg.device);
+}
+
+// Copies one member of the device scalars into the pinned mirror and waits for it: one host round trip.
+template <typename T>
+cudaError_t read_back(gbin_ctx *ctx, T Misc::*field, cudaStream_t st) {
+    Misc *dm = ctx->misc.as<Misc>();
+    Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
+    const cudaError_t e = cudaMemcpyAsync(&(hm->*field), &(dm->*field), sizeof(T), cudaMemcpyDeviceToHost, st);
+    return e == cudaSuccess ? cudaStreamSynchronize(st) : e;
+}
+
+// The device table over the context's output arrays.
+gbin_table device_table(const gbin_ctx *ctx, uint64_t n_instances, uint64_t n_distinct, uint64_t S, uint64_t NS, uint64_t B) {
+    gbin_table t;
+    memset(&t, 0, sizeof t);
+    t.kmer_size = ctx->cfg.kmer_size;
+    t.mmer_size = ctx->cfg.mmer_size;
+    t.abundance_cutoff = ctx->cfg.abundance_cutoff;
+    t.kmer_words = ctx->KW;
+    t.on_device = 1;
+    t.ctx_owned = 1;
+    t.n_instances = n_instances;
+    t.n_distinct = n_distinct;
+    t.n_kmers = S;
+    t.n_ids = NS;
+    t.n_buckets = B;
+    t.mmer_codes = ctx->o_mmer_codes.as<uint32_t>();
+    t.mmer_kmer_off = ctx->o_mmer_kmer_off.as<uint64_t>();
+    t.kmer_codes = ctx->o_kmer_codes.as<uint64_t>();
+    t.kmer_id_off = ctx->o_kmer_id_off.as<uint64_t>();
+    t.read_ids = ctx->o_read_ids.as<int32_t>();
+    return t;
+}
+
+// Bucket directory of the super-k-mer pipelines over the S surviving k-mers in ctx->o_kmer_mmer; *B receives the bucket count.
+int emit_bucket_directory(gbin_ctx *ctx, uint64_t S, uint64_t NS, cudaStream_t st, int *launches, uint64_t *B) {
+    Misc *dm = ctx->misc.as<Misc>();
+    Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
+    CU(ctx->bucket_excl.ensure((S + 1) * 4));
+    CU(ctx->o_mmer_codes.ensure((S + 1) * sizeof(uint32_t)));
+    CU(ctx->o_mmer_kmer_off.ensure((S + 2) * sizeof(uint64_t)));
+    CU(ctx->scan_scratch.ensure(group_scan_scratch_bytes(S + 1024)));
+    const bool on = ctx->prof.begin(KK_EMIT, st);
+    const int lp = skr_emit_buckets(ctx->o_kmer_mmer.as<uint32_t>(), S, NS, ctx->bucket_excl.as<uint32_t>(), ctx->scan_scratch.as<uint32_t>(),
+                                    ctx->o_mmer_codes.as<uint32_t>(), ctx->o_mmer_kmer_off.as<uint64_t>(), ctx->o_kmer_id_off.as<uint64_t>(),
+                                    &dm->n_buckets_dev, st);
+    ctx->prof.end(on, lp, st);
+    *launches += lp;
+    CU(cudaGetLastError());
+    CU(read_back(ctx, &Misc::n_buckets_dev, st));
+    *B = hm->n_buckets_dev;
+    return GBIN_OK;
+}
+
+// Host path: streams the finished part of the table to the host while later chunks are grouped.  The table is written in
+// unit order, and what the units of chunk c wrote is final once ctx->ev_chunk[c] has fired; totals_host[c] then holds
+// {k-mers << shift | ids} written up to the end of chunk c.  A chunk with k-mers left to pipeline 3's global sort for long spans
+// (lsd_totals_host[c] != 0) ends the streaming, as does an arena too small: the rest is copied at the end.
+int stream_finished_chunks(gbin_ctx *ctx, HostSink *sink, uint32_t n, const unsigned long long *totals_host, int shift,
+                           const unsigned long long *lsd_totals_host) {
+    const int KW = ctx->KW;
+    for (uint32_t c = 0; c < n; c++) {
+        CU(cudaEventSynchronize(ctx->ev_chunk[c]));
+        if (lsd_totals_host && lsd_totals_host[c]) break;
+        const unsigned long long tot = totals_host[c];
+        const uint64_t s1 = tot >> shift, n1 = tot & ((1ull << shift) - 1);
+        if (s1 > sink->kmer_cap || n1 > sink->id_cap || s1 < sink->kmers_done || n1 < sink->ids_done) break;
+        const uint64_t s0 = sink->kmers_done, n0 = sink->ids_done;
+        if (s1 > s0) {
+            CU(cudaMemcpyAsync(sink->kmer_codes + s0 * KW, ctx->o_kmer_codes.as<uint64_t>() + s0 * KW, (s1 - s0) * KW * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->st_d2h));
+            CU(cudaMemcpyAsync(sink->kmer_id_off + s0, ctx->o_kmer_id_off.as<uint64_t>() + s0, (s1 - s0) * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->st_d2h));
+        }
+        if (n1 > n0) CU(cudaMemcpyAsync(sink->read_ids + n0, ctx->o_read_ids.as<int32_t>() + n0, (n1 - n0) * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->st_d2h));
+        sink->kmers_done = s1;
+        sink->ids_done = n1;
+    }
+    return GBIN_OK;
+}
+
+// What was streamed into the sink belongs to an abandoned attempt: wait until nothing is in flight into the arenas, then start over.
+int abandon_sink(gbin_ctx *ctx, HostSink *sink) {
+    if (!sink) return GBIN_OK;
+    CU(cudaStreamSynchronize(ctx->st_d2h));
+    sink->kmers_done = sink->ids_done = 0;
+    return GBIN_OK;
+}
+
+// Partition of n records by owner: launch(scratch, d_counts, st) runs the partition kernels and returns how many it launched.
+template <typename Launch>
+int partition_by_owner(gbin_ctx *ctx, uint64_t n, uint32_t n_parts, void *stream, uint64_t *counts_host, Launch launch) {
+    if (!ctx || !counts_host || n_parts == 0 || n_parts > 256) return GBIN_E_INVALID_ARG;
+    if (n >= (1ull << 32) - 8192) return fail(ctx, GBIN_E_TOO_LARGE, "too many records in one partition call");
+    cudaStream_t st;
+    CU(begin_call(ctx, stream, &st));
+    CU(ctx->radix_scratch.ensure(radix_scratch_bytes(n)));
+    const int launches = launch(ctx->radix_scratch.p, ctx->misc.as<Misc>()->part_counts, st);
+    CU(cudaGetLastError());
+    CU(read_back(ctx, &Misc::part_counts, st));
+    memcpy(counts_host, static_cast<Misc *>(ctx->h_misc.p)->part_counts, sizeof(uint64_t) * n_parts);
+    ctx->tm.kernel_launches = (uint32_t)launches;
+    return GBIN_OK;
+}
+
 __global__ void max_len_kernel(const uint32_t *__restrict__ lens, uint64_t n, unsigned int *__restrict__ out) {
     const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     unsigned int v = i < n ? lens[i] : 0u;
@@ -252,29 +383,28 @@ int plan_reads(gbin_ctx *ctx, const gbin_reads *rd, cudaStream_t st, uint64_t *n
     CU(ctx->win_counts.ensure(rd->n_reads * sizeof(uint32_t)));
     CU(ctx->rec_off.ensure((rd->n_reads + 1) * sizeof(uint64_t)));
     CU(ctx->scan_scratch.ensure(group_scan_scratch_bytes(rd->n_reads)));
-    CU(cudaMemsetAsync(&dm->max_len, 0, sizeof(unsigned int), st));
+    CU(cudaMemsetAsync(&dm->reads.max_len, 0, sizeof(unsigned int), st));
     if (rd->max_read_len == 0) {
-        max_len_kernel<<<(unsigned)((rd->n_reads + 255) / 256), 256, 0, st>>>(rd->lens, rd->n_reads, &dm->max_len);
+        max_len_kernel<<<(unsigned)((rd->n_reads + 255) / 256), 256, 0, st>>>(rd->lens, rd->n_reads, &dm->reads.max_len);
         (*launches)++;
     }
     *launches += launch_count_windows(rv, K, ctx->win_counts.as<uint32_t>(), st);
     *launches += exclusive_scan<uint64_t, WinCountIn>(WinCountIn{ctx->win_counts.as<uint32_t>()}, ctx->rec_off.as<uint64_t>(), rd->n_reads,
                                                       ctx->scan_scratch.as<uint64_t>(),
-                                                      reinterpret_cast<uint64_t *>(&dm->total_windows), st);
-    CU(cudaMemcpyAsync(&hm->total_windows, &dm->total_windows, sizeof(unsigned long long) + sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    *n_inst = hm->total_windows;
-    *max_len = rd->max_read_len ? rd->max_read_len : hm->max_len;
+                                                      reinterpret_cast<uint64_t *>(&dm->reads.total_windows), st);
+    CU(read_back(ctx, &Misc::reads, st));
+    *n_inst = hm->reads.total_windows;
+    *max_len = rd->max_read_len ? rd->max_read_len : hm->reads.max_len;
     return GBIN_OK;
 }
 
 int run_scan(gbin_ctx *ctx, const gbin_reads *rd, uint32_t arrival_base, void *d_records, uint32_t max_len, cudaStream_t st, int *launches) {
     Misc *dm = ctx->misc.as<Misc>();
     ReadsView rv{reinterpret_cast<const uint8_t *>(rd->data), rd->data_bytes, rd->n_reads, rd->stride, rd->read_len, rd->starts, rd->lens};
-    CU(cudaMemsetAsync(&dm->bad_bases, 0, sizeof(unsigned long long), st));
+    CU(cudaMemsetAsync(&dm->grp.bad_bases, 0, sizeof(unsigned long long), st));
     const bool on = ctx->prof.begin(KK_SCAN, st);
     const int ls = launch_scan_reads(rv, rd->starts ? ctx->rec_off.as<uint64_t>() : nullptr, ctx->cfg.kmer_size, ctx->cfg.mmer_size, ctx->KW,
-                                     arrival_base, max_len ? max_len : 1, d_records, &dm->bad_bases, ctx->sm_count, st);
+                                     arrival_base, max_len ? max_len : 1, d_records, &dm->grp.bad_bases, ctx->sm_count, st);
     ctx->prof.end(on, ls < 0 ? 0 : ls, st);
     if (ls < 0) return fail(ctx, GBIN_E_TOO_LARGE, "a read of %u bases does not fit the scan kernel's shared memory (limit %u bases)", max_len, gbin_max_read_len());
     *launches += ls;
@@ -288,15 +418,6 @@ int run_group(gbin_ctx *ctx, void *recs, void *twin, uint64_t n, const int32_t *
     const int KW = ctx->KW, K = ctx->cfg.kmer_size, M = ctx->cfg.mmer_size, cutoff = ctx->cfg.abundance_cutoff;
     Misc *dm = ctx->misc.as<Misc>();
     Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
-    memset(out, 0, sizeof *out);
-    out->kmer_size = K;
-    out->mmer_size = M;
-    out->abundance_cutoff = cutoff;
-    out->kmer_words = KW;
-    out->on_device = 1;
-    out->ctx_owned = 1;
-    out->n_instances = n;
-
     CU(ctx->radix_scratch.ensure(radix_scratch_bytes(n)));
     bool in_b = false;
     int passes = 0;
@@ -313,7 +434,7 @@ int run_group(gbin_ctx *ctx, void *recs, void *twin, uint64_t n, const int32_t *
     ws.group_of = ctx->group_of.as<uint32_t>();
     ws.run_start = ctx->run_start.as<uint32_t>();
     ws.scan_scratch = ctx->scan_scratch.p;
-    ws.counts = &dm->counts;
+    ws.counts = &dm->grp.counts;
     ws.cutoff = cutoff;
 
     bool on = ctx->prof.begin(KK_RUNS, st);
@@ -321,11 +442,9 @@ int run_group(gbin_ctx *ctx, void *recs, void *twin, uint64_t n, const int32_t *
     ctx->prof.end(on, lg, st);
     *launches += lg;
     CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(hm, dm, sizeof(GroupCounts) + sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    if (hm->bad_bases) return fail(ctx, GBIN_E_NON_ACGT, "%llu bases other than A/C/G/T in the batch", hm->bad_bases);
-    const uint64_t G = hm->counts.n_distinct;
-    out->n_distinct = G;
+    CU(read_back(ctx, &Misc::grp, st));
+    if (hm->grp.bad_bases) return fail(ctx, GBIN_E_NON_ACGT, "%llu bases other than A/C/G/T in the batch", hm->grp.bad_bases);
+    const uint64_t G = hm->grp.counts.n_distinct;
 
     uint64_t S = 0, NS = 0, B = 0;
     if (G) {
@@ -338,10 +457,9 @@ int run_group(gbin_ctx *ctx, void *recs, void *twin, uint64_t n, const int32_t *
         ctx->prof.end(on, lg, st);
         *launches += lg;
         CU(cudaGetLastError());
-        CU(cudaMemcpyAsync(&hm->counts, &dm->counts, sizeof(GroupCounts), cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        S = hm->counts.n_kmers;
-        NS = hm->counts.n_ids;
+        CU(read_back(ctx, &Misc::grp, st));
+        S = hm->grp.counts.n_kmers;
+        NS = hm->grp.counts.n_ids;
     }
     if (S) {
         CU(ctx->surv_group.ensure(S * sizeof(uint32_t)));
@@ -353,9 +471,8 @@ int run_group(gbin_ctx *ctx, void *recs, void *twin, uint64_t n, const int32_t *
         ctx->prof.end(on, lg, st);
         *launches += lg;
         CU(cudaGetLastError());
-        CU(cudaMemcpyAsync(&hm->counts, &dm->counts, sizeof(GroupCounts), cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        B = hm->counts.n_buckets;
+        CU(read_back(ctx, &Misc::grp, st));
+        B = hm->grp.counts.n_buckets;
     }
     CU(ctx->o_mmer_codes.ensure((B + 1) * sizeof(uint32_t)));
     CU(ctx->o_mmer_kmer_off.ensure((B + 1) * sizeof(uint64_t)));
@@ -369,24 +486,17 @@ int run_group(gbin_ctx *ctx, void *recs, void *twin, uint64_t n, const int32_t *
     ctx->prof.end(on, lg, st);
     *launches += lg;
     CU(cudaGetLastError());
-    out->n_kmers = S;
-    out->n_ids = NS;
-    out->n_buckets = B;
-    out->mmer_codes = to.mmer_codes;
-    out->mmer_kmer_off = to.mmer_kmer_off;
-    out->kmer_codes = to.kmer_codes;
-    out->kmer_id_off = to.kmer_id_off;
-    out->read_ids = to.read_ids;
+    *out = device_table(ctx, n, G, S, NS, B);
     return GBIN_OK;
 }
 
-// ---- pipeline v2: super-k-mer records -> stable sort by m-mer -> grouping in shared memory
+// ---- super-k-mer pipelines.  Pipeline 2: super-k-mer records -> stable sort by m-mer -> grouping in shared memory.
 
-// Scan stage: one record per signature segment, in arrival order, into ctx->skr_a (own == true) or into the
+// Scan stage of pipelines 2 and 3: one record per signature segment, in arrival order, into ctx->skr_a (own == true) or into the
 // caller's buffer `ext` of `ext_cap` records.  *n_skr receives the record count.  With a feed (host path, fixed-stride
 // reads) the reads arrive over PCIe in chunks on the copy stream and every chunk is scanned as soon as it is there.
-int run_v2_scan(gbin_ctx *ctx, const gbin_reads *rd, uint64_t n, uint32_t max_len, uint32_t arrival_base, void *ext, uint64_t ext_cap,
-                cudaStream_t st, uint64_t *n_skr_out, int *launches, const HostFeed *feed = nullptr) {
+int run_skr_scan(gbin_ctx *ctx, const gbin_reads *rd, uint64_t n, uint32_t max_len, uint32_t arrival_base, void *ext, uint64_t ext_cap,
+                 cudaStream_t st, uint64_t *n_skr_out, int *launches, const HostFeed *feed = nullptr) {
     const int K = ctx->cfg.kmer_size, M = ctx->cfg.mmer_size;
     const int NW = K <= 32 ? 8 : 12;
     Misc *dm = ctx->misc.as<Misc>();
@@ -409,7 +519,7 @@ int run_v2_scan(gbin_ctx *ctx, const gbin_reads *rd, uint64_t n, uint32_t max_le
                 if (b1 > b0) CU(cudaMemcpyAsync(feed->dst + b0, feed->src + b0, b1 - b0, cudaMemcpyHostToDevice, ctx->st_h2d));
                 CU(cudaEventRecord(ctx->ev_feed[c], ctx->st_h2d));
                 CU(cudaStreamWaitEvent(st, ctx->ev_feed[c], 0));
-                if (c + 1 == chunks) CU(cudaEventRecord(ctx->ev[1], st));  // every byte of the reads is on the device
+                if (c + 1 == chunks) CU(cudaEventRecord(ctx->ev[EV_READS_ON_DEVICE], st));  // every byte of the reads is on the device
             }
             const int l1 = launch_skr_scan(rv, r0, r1, K, M, arrival_base, max_len, ext ? ext : ctx->skr_a.p, cap, ctx->tile_state.as<unsigned long long>(),
                                            &dm->skr_ticket, dm->skr_counters, ctx->sm_count, st);
@@ -422,8 +532,7 @@ int run_v2_scan(gbin_ctx *ctx, const gbin_reads *rd, uint64_t n, uint32_t max_le
         ctx->prof.end(on, ls, st);
         *launches += ls;
         CU(cudaGetLastError());
-        CU(cudaMemcpyAsync(hm->skr_counters, dm->skr_counters, sizeof dm->skr_counters, cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
+        CU(read_back(ctx, &Misc::skr_counters, st));
         if (hm->skr_counters[0]) return fail(ctx, GBIN_E_NON_ACGT, "%llu bases other than A/C/G/T in the batch", hm->skr_counters[0]);
         n_skr = hm->skr_counters[1];
         if (hm->skr_counters[2] != n)
@@ -455,7 +564,7 @@ int run_v2_group(gbin_ctx *ctx, void *skr, void *twin, uint64_t n_skr, const int
     CU(cudaGetLastError());
     ctx->tm.sort_passes = (uint32_t)passes;
     const void *sorted = in_b ? twin : skr;
-    CU(cudaEventRecord(ctx->ev[3], st));
+    CU(cudaEventRecord(ctx->ev[EV_SORTED], st));
 
     // ---- plan: instance prefix, m-mer runs, units
     CU(ctx->inst_prefix.ensure((n_skr + 2) * 4));
@@ -464,13 +573,12 @@ int run_v2_group(gbin_ctx *ctx, void *skr, void *twin, uint64_t n_skr, const int
     CU(ctx->scan_scratch.ensure(group_scan_scratch_bytes(n_skr)));
     bool on = ctx->prof.begin(KK_SKR_PLAN, st);
     int lp = skr_plan_runs(ctx->skr_side.as<uint64_t>(), n_skr, ctx->inst_prefix.as<uint32_t>(), ctx->run_excl.as<uint64_t>(), ctx->skr_run_start.as<uint32_t>(),
-                           ctx->scan_scratch.as<uint64_t>(), &dm->n_inst_dev, &dm->n_runs_dev, st);
+                           ctx->scan_scratch.as<uint64_t>(), &dm->plan.n_inst, &dm->plan.n_runs, st);
     ctx->prof.end(on, lp, st);
     *launches += lp;
     CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(&hm->n_inst_dev, &dm->n_inst_dev, 2 * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    const uint64_t n_runs = hm->n_runs_dev, n = hm->n_inst_dev;
+    CU(read_back(ctx, &Misc::plan, st));
+    const uint64_t n_runs = hm->plan.n_runs, n = hm->plan.n_inst;
     *n_inst_out = n;
     ctx->rs.n_super_kmers = n_skr;
     ctx->rs.n_mmer_runs = n_runs;
@@ -517,69 +625,26 @@ int run_v2_group(gbin_ctx *ctx, void *skr, void *twin, uint64_t n_skr, const int
     ctx->prof.end(on, lp, st);
     *launches += lp;
     CU(cudaGetLastError());
-    if (ch.done) {
-        // Stream the finished part of the table to the host while later chunks are grouped: the output of units [0, u) is
-        // final once they have completed, and the flat table is written in unit order.
-        for (uint32_t c = 0; c < ch.n; c++) {
-            CU(cudaEventSynchronize(ctx->ev_chunk[c]));
-            const unsigned long long tot = hm->chunk_totals[c];
-            const uint64_t s1 = tot >> 31, n1 = tot & 0x7fffffffull;
-            if (s1 > sink->kmer_cap || n1 > sink->id_cap || s1 < sink->kmers_done || n1 < sink->ids_done) break;  // arena too small: the rest is copied at the end
-            const uint64_t s0 = sink->kmers_done, n0 = sink->ids_done;
-            if (s1 > s0) {
-                CU(cudaMemcpyAsync(sink->kmer_codes + s0 * KW, ctx->o_kmer_codes.as<uint64_t>() + s0 * KW, (s1 - s0) * KW * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->st_d2h));
-                CU(cudaMemcpyAsync(sink->kmer_id_off + s0, ctx->o_kmer_id_off.as<uint64_t>() + s0, (s1 - s0) * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->st_d2h));
-            }
-            if (n1 > n0) CU(cudaMemcpyAsync(sink->read_ids + n0, ctx->o_read_ids.as<int32_t>() + n0, (n1 - n0) * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->st_d2h));
-            sink->kmers_done = s1;
-            sink->ids_done = n1;
-        }
+    if (ch.done) {  // the grouping kernels pack each chunk's totals as {k-mers << 31 | ids}
+        const int rc = stream_finished_chunks(ctx, sink, ch.n, hm->chunk_totals, 31, nullptr);
+        if (rc) return rc;
     }
-    CU(cudaMemcpyAsync(&hm->gc, &dm->gc, sizeof(SkrGroupCounters), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
+    CU(read_back(ctx, &Misc::gc, st));
     ctx->rs.n_units = hm->gc.n_units;
     if (hm->gc.overflow) {  // a unit did not fit shared memory: this batch goes through pipeline v1
         ctx->fallbacks++;
         return GBIN_OK;
     }
     const uint64_t S = hm->gc.total_kmers, NS = hm->gc.total_ids;
-
-    // ---- bucket directory
-    CU(ctx->bucket_excl.ensure((S + 1) * 4));
-    CU(ctx->o_mmer_codes.ensure((S + 1) * sizeof(uint32_t)));
-    CU(ctx->o_mmer_kmer_off.ensure((S + 2) * sizeof(uint64_t)));
-    on = ctx->prof.begin(KK_EMIT, st);
-    lp = skr_emit_buckets(ctx->o_kmer_mmer.as<uint32_t>(), S, NS, ctx->bucket_excl.as<uint32_t>(), ctx->scan_scratch.as<uint32_t>(),
-                          ctx->o_mmer_codes.as<uint32_t>(), ctx->o_mmer_kmer_off.as<uint64_t>(), ctx->o_kmer_id_off.as<uint64_t>(),
-                          &dm->n_buckets_dev, st);
-    ctx->prof.end(on, lp, st);
-    *launches += lp;
-    CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(&hm->n_buckets_dev, &dm->n_buckets_dev, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-
-    memset(out, 0, sizeof *out);
-    out->kmer_size = K;
-    out->mmer_size = M;
-    out->abundance_cutoff = cutoff;
-    out->kmer_words = KW;
-    out->on_device = 1;
-    out->ctx_owned = 1;
-    out->n_instances = n;
-    out->n_distinct = hm->gc.distinct;
-    out->n_kmers = S;
-    out->n_ids = NS;
-    out->n_buckets = hm->n_buckets_dev;
-    out->mmer_codes = ctx->o_mmer_codes.as<uint32_t>();
-    out->mmer_kmer_off = ctx->o_mmer_kmer_off.as<uint64_t>();
-    out->kmer_codes = ctx->o_kmer_codes.as<uint64_t>();
-    out->kmer_id_off = ctx->o_kmer_id_off.as<uint64_t>();
-    out->read_ids = ctx->o_read_ids.as<int32_t>();
+    uint64_t B = 0;
+    const int rc = emit_bucket_directory(ctx, S, NS, st, launches, &B);
+    if (rc) return rc;
+    *out = device_table(ctx, n, hm->gc.distinct, S, NS, B);
     *done = true;
     return GBIN_OK;
 }
 
-// ---- pipeline v3: entries sorted by reference, one warp per unit, staging + finalize (bin3.cu)
+// ---- pipeline 3: entries sorted by reference, one warp per unit, staging + finalize (bin3.cu)
 // The records in `skr` are read, not moved.  *done = false when the batch does not fit (a (bucket, d) class larger than a unit);
 // it then goes through pipeline 2, which sorts the records themselves.
 
@@ -610,11 +675,10 @@ int v3_choose_layout(gbin_ctx *ctx, const void *skr, uint64_t n_skr, cudaStream_
     Misc *dm = ctx->misc.as<Misc>();
     Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
     CU(ctx->v3_bitmap.ensure(v3_mmer_bitmap_bytes(M)));
-    *launches += v3_count_mmers(skr, K <= 32 ? 8 : 12, n_skr, M, ctx->v3_bitmap.as<uint32_t>(), &dm->n_real_entries, st);
+    *launches += v3_count_mmers(skr, K <= 32 ? 8 : 12, n_skr, M, ctx->v3_bitmap.as<uint32_t>(), &dm->n_mmers, st);
     CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(&hm->n_real_entries, &dm->n_real_entries, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    const double buckets = hm->n_real_entries ? (double)hm->n_real_entries : 1.0;
+    CU(read_back(ctx, &Misc::n_mmers, st));
+    const double buckets = hm->n_mmers ? (double)hm->n_mmers : 1.0;
     const double mean_inst = (double)n_skr / buckets * ((K - M + 2) / 2.0);  // a record holds about (K-M+2)/2 windows
     int nc = 1, h = 0;
     const int cap1 = ctx->v3_cap ? ctx->v3_cap : 1024, cap2 = ctx->v3_cap ? ctx->v3_cap : 512;
@@ -650,13 +714,12 @@ int run_v3_pass(gbin_ctx *ctx, const void *skr, const uint64_t *ent, const uint1
     CU(ctx->scan_scratch.ensure(group_scan_scratch_bytes(n_ent)));
     bool on = ctx->prof.begin(KK_SKR_PLAN, st);
     int lp = v3_plan_runs(ent, sorted_info, n_ent, ctx->inst_prefix.as<uint32_t>(), ctx->run_excl.as<uint64_t>(), ctx->skr_run_start.as<uint32_t>(),
-                          ctx->scan_scratch.as<uint64_t>(), &dm->n_inst_dev, &dm->n_runs_dev, st);
+                          ctx->scan_scratch.as<uint64_t>(), &dm->plan.n_inst, &dm->plan.n_runs, st);
     ctx->prof.end(on, lp, st);
     *launches += lp;
     CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(&hm->n_inst_dev, &dm->n_inst_dev, 2 * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    const uint64_t n_runs = hm->n_runs_dev, n = hm->n_inst_dev;
+    CU(read_back(ctx, &Misc::plan, st));
+    const uint64_t n_runs = hm->plan.n_runs, n = hm->plan.n_inst;
     *n_inst = n;
     ctx->rs.n_mmer_runs += n_runs;
     const uint64_t max_units = v3_max_units(n, n_runs, ctx->v3_cap_eff);
@@ -721,27 +784,11 @@ int run_v3_pass(gbin_ctx *ctx, const void *skr, const uint64_t *ent, const uint1
                          lsd_view(lsd_cap), false, ctx->sm_count, &ctx->prof, st);
     *launches += lp;
     CU(cudaGetLastError());
-    if (ch.done) {
-        // Stream the finished part of the table to the host while later chunks are grouped: the output of the units of a chunk
-        // is final once the chunk's launches have completed — unless the chunk holds long spans, which wait for the global sort.
-        for (uint32_t c = 0; c < ch.n; c++) {
-            CU(cudaEventSynchronize(ctx->ev_chunk[c]));
-            if (hm->lsd_totals[c]) break;
-            const unsigned long long tot = hm->chunk_totals[c];
-            const uint64_t s1 = tot >> 32, n1 = tot & 0xffffffffull;
-            if (s1 > sink->kmer_cap || n1 > sink->id_cap || s1 < sink->kmers_done || n1 < sink->ids_done) break;  // arena too small: the rest is copied at the end
-            const uint64_t s0 = sink->kmers_done, n0 = sink->ids_done;
-            if (s1 > s0) {
-                CU(cudaMemcpyAsync(sink->kmer_codes + s0 * KW, ctx->o_kmer_codes.as<uint64_t>() + s0 * KW, (s1 - s0) * KW * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->st_d2h));
-                CU(cudaMemcpyAsync(sink->kmer_id_off + s0, ctx->o_kmer_id_off.as<uint64_t>() + s0, (s1 - s0) * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->st_d2h));
-            }
-            if (n1 > n0) CU(cudaMemcpyAsync(sink->read_ids + n0, ctx->o_read_ids.as<int32_t>() + n0, (n1 - n0) * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->st_d2h));
-            sink->kmers_done = s1;
-            sink->ids_done = n1;
-        }
+    if (ch.done) {  // the grouping kernels pack each chunk's totals as {k-mers << 32 | ids}
+        rc = stream_finished_chunks(ctx, sink, ch.n, hm->chunk_totals, 32, hm->lsd_totals);
+        if (rc) return rc;
     }
-    CU(cudaMemcpyAsync(&hm->gc3, &dm->gc3, sizeof(V3Counters), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
+    CU(read_back(ctx, &Misc::gc3, st));
     if (hm->gc3.overflow == 6u && hm->gc3.lsd_kmers > lsd_cap) {
         // long spans met no (or too small) sort arrays: allocate them and redo their placement (the staged results are still there)
         ctx->v3_lsd_seen = true;
@@ -758,8 +805,7 @@ int run_v3_pass(gbin_ctx *ctx, const void *skr, const uint64_t *ent, const uint1
                              lsd_view(lsd_cap), true, ctx->sm_count, &ctx->prof, st);
         *launches += lp;
         CU(cudaGetLastError());
-        CU(cudaMemcpyAsync(&hm->gc3, &dm->gc3, sizeof(V3Counters), cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
+        CU(read_back(ctx, &Misc::gc3, st));
     }
     ctx->rs.n_units += hm->gc3.n_units;
     ctx->rs.n_lsd_kmers += hm->gc3.lsd_kmers;
@@ -787,7 +833,7 @@ int run_v3_pass(gbin_ctx *ctx, const void *skr, const uint64_t *ent, const uint1
 int run_v3_group(gbin_ctx *ctx, const void *skr, uint64_t n_skr, const int32_t *d_ids, int32_t id_base, cudaStream_t st, gbin_table *out, int *launches,
                  bool *done, uint64_t *n_inst_out, HostSink *sink = nullptr) {
     *done = false;
-    const int K = ctx->cfg.kmer_size, M = ctx->cfg.mmer_size, cutoff = ctx->cfg.abundance_cutoff, KW = ctx->KW;
+    const int K = ctx->cfg.kmer_size, M = ctx->cfg.mmer_size;
     Misc *dm = ctx->misc.as<Misc>();
     Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
     KeyLayout kl;
@@ -835,11 +881,10 @@ int run_v3_group(gbin_ctx *ctx, const void *skr, uint64_t n_skr, const int32_t *
     CU(cudaGetLastError());
     ctx->tm.sort_passes = (uint32_t)passes;
     const uint64_t *ent = in_b ? ent_b_p : ent_a_p;
-    CU(cudaEventRecord(ctx->ev[3], st));
+    CU(cudaEventRecord(ctx->ev[EV_SORTED], st));
     uint64_t n_ent = n_slots;
     if (kl.nc == 2) {  // empty pieces carry the all-ones key and sort behind everything: plan over the real ones only
-        CU(cudaMemcpyAsync(&hm->n_real_entries, &dm->n_real_entries, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
+        CU(read_back(ctx, &Misc::n_real_entries, st));
         n_ent = hm->n_real_entries;
     }
 
@@ -895,39 +940,10 @@ int run_v3_group(gbin_ctx *ctx, const void *skr, uint64_t n_skr, const int32_t *
     ctx->rs.n_passes = (uint32_t)(bounds.size() - 1);
     const uint64_t S = S_off, NS = N_off;
     if (S >= (1ull << 32)) return fail(ctx, GBIN_E_TOO_LARGE, "%llu surviving k-mers in one batch (limit 2^32)", (unsigned long long)S);
-
-    // ---- bucket directory
-    CU(ctx->bucket_excl.ensure((S + 1) * 4));
-    CU(ctx->o_mmer_codes.ensure((S + 1) * sizeof(uint32_t)));
-    CU(ctx->o_mmer_kmer_off.ensure((S + 2) * sizeof(uint64_t)));
-    CU(ctx->scan_scratch.ensure(group_scan_scratch_bytes(S + 1024)));
-    on = ctx->prof.begin(KK_EMIT, st);
-    lp = skr_emit_buckets(ctx->o_kmer_mmer.as<uint32_t>(), S, NS, ctx->bucket_excl.as<uint32_t>(), ctx->scan_scratch.as<uint32_t>(),
-                          ctx->o_mmer_codes.as<uint32_t>(), ctx->o_mmer_kmer_off.as<uint64_t>(), ctx->o_kmer_id_off.as<uint64_t>(),
-                          &dm->n_buckets_dev, st);
-    ctx->prof.end(on, lp, st);
-    *launches += lp;
-    CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(&hm->n_buckets_dev, &dm->n_buckets_dev, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-
-    memset(out, 0, sizeof *out);
-    out->kmer_size = K;
-    out->mmer_size = M;
-    out->abundance_cutoff = cutoff;
-    out->kmer_words = KW;
-    out->on_device = 1;
-    out->ctx_owned = 1;
-    out->n_instances = n_total;
-    out->n_distinct = distinct;
-    out->n_kmers = S;
-    out->n_ids = NS;
-    out->n_buckets = hm->n_buckets_dev;
-    out->mmer_codes = ctx->o_mmer_codes.as<uint32_t>();
-    out->mmer_kmer_off = ctx->o_mmer_kmer_off.as<uint64_t>();
-    out->kmer_codes = ctx->o_kmer_codes.as<uint64_t>();
-    out->kmer_id_off = ctx->o_kmer_id_off.as<uint64_t>();
-    out->read_ids = ctx->o_read_ids.as<int32_t>();
+    uint64_t B = 0;
+    rc = emit_bucket_directory(ctx, S, NS, st, launches, &B);
+    if (rc) return rc;
+    *out = device_table(ctx, n_total, distinct, S, NS, B);
     *done = true;
     return GBIN_OK;
 }
@@ -945,10 +961,8 @@ int run_skr_group(gbin_ctx *ctx, void *skr, uint64_t n_skr, const int32_t *d_ids
             return GBIN_OK;
         }
         ctx->fallbacks++;
-        if (sink) {  // what was streamed belongs to the abandoned attempt
-            CU(cudaStreamSynchronize(ctx->st_d2h));
-            sink->kmers_done = sink->ids_done = 0;
-        }
+        rc = abandon_sink(ctx, sink);
+        if (rc) return rc;
     }
     if (n_skr * (uint64_t)(ctx->cfg.kmer_size - ctx->cfg.mmer_size + 1) >= (1ull << 31))  // pipeline 2 holds instance coordinates in 31 bits
         return fail(ctx, GBIN_E_TOO_LARGE, "the batch is too large for pipeline 2 (%llu super-k-mer records) and pipeline 3 %s", (unsigned long long)n_skr,
@@ -960,18 +974,18 @@ int run_skr_group(gbin_ctx *ctx, void *skr, uint64_t n_skr, const int32_t *d_ids
     return GBIN_OK;
 }
 
-int run_v2(gbin_ctx *ctx, const gbin_reads *rd, uint64_t n, uint32_t max_len, cudaStream_t st, gbin_table *out, int *launches, bool *done,
-           const HostFeed *feed, HostSink *sink, int *used) {
+int run_skr_pipelines(gbin_ctx *ctx, const gbin_reads *rd, uint64_t n, uint32_t max_len, cudaStream_t st, gbin_table *out, int *launches, bool *done,
+                      const HostFeed *feed, HostSink *sink, int *used) {
     *done = false;
     if (n == 0 || (ctx->pipeline < 3 && n >= (1ull << 31))) return GBIN_OK;
     uint64_t n_skr = 0, n_chk = 0;
-    int rc = run_v2_scan(ctx, rd, n, max_len, 0, nullptr, 0, st, &n_skr, launches, feed);
+    int rc = run_skr_scan(ctx, rd, n, max_len, 0, nullptr, 0, st, &n_skr, launches, feed);
     if (rc == GBIN_E_TOO_LARGE) {  // reads longer than the super-k-mer scan holds in shared memory: pipeline 1 takes the batch
         ctx->fallbacks++;
         return GBIN_OK;
     }
     if (rc) return rc;
-    CU(cudaEventRecord(ctx->ev[2], st));
+    CU(cudaEventRecord(ctx->ev[EV_SCANNED], st));
     rc = run_skr_group(ctx, ctx->skr_a.p, n_skr, rd->read_ids, rd->id_base, st, out, launches, done, &n_chk, sink, used);
     if (rc) return rc;
     if (!*done) return GBIN_OK;
@@ -992,23 +1006,21 @@ int bin_device_impl(gbin_ctx *ctx, const gbin_reads *rd, cudaStream_t st, gbin_t
     const bool v2 = ctx->pipeline >= 2 && n != 0 && (ctx->pipeline >= 3 || n < (1ull << 31));
     if (feed && (!v2 || max_len > 1500)) {  // nobody downstream streams the reads in (long reads go to pipeline 1's scan): copy them in one piece
         CU(cudaMemcpyAsync(feed->dst, feed->src, feed->bytes, cudaMemcpyHostToDevice, st));
-        CU(cudaEventRecord(ctx->ev[1], st));
+        CU(cudaEventRecord(ctx->ev[EV_READS_ON_DEVICE], st));
         feed = nullptr;
     }
     if (v2) {
         bool done = false;
         int used = 2;
-        rc = run_v2(ctx, rd, n, max_len, st, out, launches, &done, feed, sink, &used);
+        rc = run_skr_pipelines(ctx, rd, n, max_len, st, out, launches, &done, feed, sink, &used);
         if (rc) return rc;
         if (done) {
             ctx->last_pipeline = used;
-            CU(cudaEventRecord(ctx->ev[4], st));
+            CU(cudaEventRecord(ctx->ev[EV_GROUPED], st));
             return GBIN_OK;
         }
-        if (sink) {  // what was streamed belongs to the abandoned attempt; nothing may still be in flight into the arenas
-            CU(cudaStreamSynchronize(ctx->st_d2h));
-            sink->kmers_done = sink->ids_done = 0;
-        }
+        rc = abandon_sink(ctx, sink);
+        if (rc) return rc;
     }
     if (n >= (1ull << 32) - 8192) return fail(ctx, GBIN_E_TOO_LARGE, "%llu k-mer instances: too many for the pipeline-1 fallback", (unsigned long long)n);
     ctx->last_pipeline = 1;
@@ -1018,10 +1030,10 @@ int bin_device_impl(gbin_ctx *ctx, const gbin_reads *rd, cudaStream_t st, gbin_t
     CU(ctx->rec_b.ensure((n + 1) * rb));
     rc = run_scan(ctx, rd, 0, ctx->rec_a.p, max_len, st, launches);
     if (rc) return rc;
-    CU(cudaEventRecord(ctx->ev[2], st));
-    rc = run_group(ctx, ctx->rec_a.p, ctx->rec_b.p, n, rd->read_ids, rd->id_base, st, out, launches, ctx->ev[3]);
+    CU(cudaEventRecord(ctx->ev[EV_SCANNED], st));
+    rc = run_group(ctx, ctx->rec_a.p, ctx->rec_b.p, n, rd->read_ids, rd->id_base, st, out, launches, ctx->ev[EV_SORTED]);
     if (rc) return rc;
-    CU(cudaEventRecord(ctx->ev[4], st));
+    CU(cudaEventRecord(ctx->ev[EV_GROUPED], st));
     return GBIN_OK;
 }
 
@@ -1095,7 +1107,7 @@ int gbin_create(const gbin_config *cfg, gbin_ctx **out) {
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking);
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&ctx->st_h2d, cudaStreamNonBlocking);
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&ctx->st_d2h, cudaStreamNonBlocking);
-    for (int i = 0; i < 6 && e == cudaSuccess; i++) e = cudaEventCreate(&ctx->ev[i]);
+    for (int i = 0; i < EV_COUNT && e == cudaSuccess; i++) e = cudaEventCreate(&ctx->ev[i]);
     for (int i = 0; i < SKR_MAX_CHUNKS && e == cudaSuccess; i++) e = cudaEventCreateWithFlags(&ctx->ev_feed[i], cudaEventDisableTiming);
     for (int i = 0; i < SKR_MAX_CHUNKS && e == cudaSuccess; i++) e = cudaEventCreateWithFlags(&ctx->ev_chunk[i], cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_copy, cudaEventDisableTiming);
@@ -1122,25 +1134,8 @@ void gbin_destroy(gbin_ctx *ctx) {
     cudaSetDevice(ctx->cfg.device);
     cudaStreamSynchronize(ctx->stream);
     gbin_xchg_destroy(ctx);
-    DevBuf *bufs[] = {&ctx->d_reads, &ctx->d_starts, &ctx->d_lens, &ctx->d_ids, &ctx->rec_a, &ctx->rec_b, &ctx->radix_scratch,
-                      &ctx->win_counts, &ctx->rec_off, &ctx->scan_scratch, &ctx->group_of, &ctx->run_start, &ctx->surv_index,
-                      &ctx->id_offset, &ctx->surv_group, &ctx->bucket_of, &ctx->misc, &ctx->o_mmer_codes, &ctx->o_mmer_kmer_off,
-                      &ctx->o_kmer_codes, &ctx->o_kmer_id_off, &ctx->o_read_ids, &ctx->skr_a, &ctx->skr_b, &ctx->tile_state,
-                      &ctx->inst_prefix, &ctx->run_excl, &ctx->skr_run_start, &ctx->small_prefix, &ctx->unit_base, &ctx->units,
-                      &ctx->unit_state, &ctx->o_kmer_mmer, &ctx->bucket_excl, &ctx->big_list, &ctx->big_k0, &ctx->big_k1, &ctx->big_arr, &ctx->stg_ids, &ctx->stg_codes, &ctx->stg_mmer, &ctx->stg_off, &ctx->skr_side,
-                      &ctx->ent_a, &ctx->ent_b, &ctx->piece_n, &ctx->sorted_info, &ctx->v3_base64, &ctx->v3_head_run, &ctx->v3_unit_out, &ctx->v3_unit_excl, &ctx->v3_atoms, &ctx->v3_lsd_aux, &ctx->v3_bitmap, &ctx->x_list_off, &ctx->x_ids};
-    for (DevBuf *b : bufs) b->release();
-    ctx->h_misc.release();
-    ctx->h_result.release();
-    ctx->h_kmer_codes.release();
-    ctx->h_kmer_id_off.release();
-    ctx->h_read_ids.release();
-    ctx->h_file.release();
-    ctx->split_nl.release();
-    ctx->split_tiles_buf.release();
-    ctx->split_base.release();
     ctx->prof.destroy();
-    for (int i = 0; i < 6; i++) cudaEventDestroy(ctx->ev[i]);
+    for (int i = 0; i < EV_COUNT; i++) cudaEventDestroy(ctx->ev[i]);
     for (int i = 0; i < SKR_MAX_CHUNKS; i++) {
         cudaEventDestroy(ctx->ev_feed[i]);
         cudaEventDestroy(ctx->ev_chunk[i]);
@@ -1152,7 +1147,7 @@ void gbin_destroy(gbin_ctx *ctx) {
     cudaStreamDestroy(ctx->st_h2d);
     cudaStreamDestroy(ctx->st_d2h);
     cudaStreamDestroy(ctx->stream);
-    delete ctx;
+    delete ctx;  // the buffers free their memory
 }
 
 int gbin_get_config(const gbin_ctx *ctx, gbin_config *out) {
@@ -1195,12 +1190,12 @@ static void finish_timings(gbin_ctx *ctx, int launches, bool host_path) {
         }
         return t;
     };
-    ctx->tm.h2d_ms = host_path ? ms(0, 1) : 0.f;
-    ctx->tm.scan_ms = ms(1, 2);
-    ctx->tm.sort_ms = ms(2, 3);
-    ctx->tm.group_ms = ms(3, 4);
-    ctx->tm.d2h_ms = host_path ? ms(4, 5) : 0.f;
-    ctx->tm.total_ms = ms(0, host_path ? 5 : 4);
+    ctx->tm.h2d_ms = host_path ? ms(EV_START, EV_READS_ON_DEVICE) : 0.f;
+    ctx->tm.scan_ms = ms(EV_READS_ON_DEVICE, EV_SCANNED);
+    ctx->tm.sort_ms = ms(EV_SCANNED, EV_SORTED);
+    ctx->tm.group_ms = ms(EV_SORTED, EV_GROUPED);
+    ctx->tm.d2h_ms = host_path ? ms(EV_GROUPED, EV_TABLE_ON_HOST) : 0.f;
+    ctx->tm.total_ms = ms(EV_START, host_path ? EV_TABLE_ON_HOST : EV_GROUPED);
     ctx->tm.kernel_launches = (uint32_t)launches;
     ctx->prof.collect();
 }
@@ -1284,11 +1279,11 @@ const char *gbin_kernel_kind_name(int kind) {
 
 int gbin_bin_reads_device(gbin_ctx *ctx, const gbin_reads *reads, void *stream, gbin_table *out) {
     if (!ctx || !reads || !out) return GBIN_E_INVALID_ARG;
-    CU(cudaSetDevice(ctx->cfg.device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    cudaStream_t st;
+    CU(begin_call(ctx, stream, &st));
     int launches = 0;
-    CU(cudaEventRecord(ctx->ev[0], st));
-    CU(cudaEventRecord(ctx->ev[1], st));
+    CU(cudaEventRecord(ctx->ev[EV_START], st));
+    CU(cudaEventRecord(ctx->ev[EV_READS_ON_DEVICE], st));
     int rc = bin_device_impl(ctx, reads, st, out, &launches);
     if (rc) return rc;
     CU(cudaStreamSynchronize(st));
@@ -1335,13 +1330,13 @@ static int table_to_pinned(gbin_ctx *ctx, const gbin_table &dev, HostSink *sink,
 
 int gbin_bin_reads_host(gbin_ctx *ctx, const gbin_reads *reads, gbin_table *out) {
     if (!ctx || !reads || !out) return GBIN_E_INVALID_ARG;
-    CU(cudaSetDevice(ctx->cfg.device));
-    cudaStream_t st = ctx->stream;
+    cudaStream_t st;
+    CU(begin_call(ctx, nullptr, &st));
     int launches = 0;
     gbin_reads d = *reads;
     HostFeed feed{};
     bool use_feed = false;
-    CU(cudaEventRecord(ctx->ev[0], st));
+    CU(cudaEventRecord(ctx->ev[EV_START], st));
     if (reads->n_reads) {
         if (!reads->data || reads->data_bytes == 0) return fail(ctx, GBIN_E_INVALID_ARG, "host reads need data and data_bytes");
         CU(ctx->d_reads.ensure(reads->data_bytes + 64));
@@ -1351,7 +1346,7 @@ int gbin_bin_reads_host(gbin_ctx *ctx, const gbin_reads *reads, gbin_table *out)
             feed = HostFeed{reads->data, ctx->d_reads.as<char>(), reads->data_bytes, ctx->host_chunks};
             if (reads->n_reads < 4096u * (uint64_t)feed.chunks) feed.chunks = 1;
             use_feed = true;
-            CU(cudaStreamWaitEvent(ctx->st_h2d, ctx->ev[0], 0));
+            CU(cudaStreamWaitEvent(ctx->st_h2d, ctx->ev[EV_START], 0));
         } else {
             CU(cudaMemcpyAsync(ctx->d_reads.p, reads->data, reads->data_bytes, cudaMemcpyHostToDevice, st));
         }
@@ -1379,7 +1374,7 @@ int gbin_bin_reads_host(gbin_ctx *ctx, const gbin_reads *reads, gbin_table *out)
             d.read_ids = ctx->d_ids.as<int32_t>();
         }
     }
-    if (!use_feed) CU(cudaEventRecord(ctx->ev[1], st));
+    if (!use_feed) CU(cudaEventRecord(ctx->ev[EV_READS_ON_DEVICE], st));
     // the big arrays of the table are streamed into the pinned arenas as far as these reach (they are sized by the previous
     // call, so the first call on a context copies everything at the end and later calls of similar size overlap the copy)
     HostSink sink{static_cast<uint64_t *>(ctx->h_kmer_codes.p), static_cast<uint64_t *>(ctx->h_kmer_id_off.p), static_cast<int32_t *>(ctx->h_read_ids.p),
@@ -1396,7 +1391,7 @@ int gbin_bin_reads_host(gbin_ctx *ctx, const gbin_reads *reads, gbin_table *out)
     }
     rc = table_to_pinned(ctx, dev, &sink, st, out);
     if (rc) return rc;
-    CU(cudaEventRecord(ctx->ev[5], st));
+    CU(cudaEventRecord(ctx->ev[EV_TABLE_ON_HOST], st));
     CU(cudaStreamSynchronize(st));
     CU(cudaStreamSynchronize(ctx->st_d2h));
     finish_timings(ctx, launches, true);
@@ -1405,8 +1400,8 @@ int gbin_bin_reads_host(gbin_ctx *ctx, const gbin_reads *reads, gbin_table *out)
 
 int gbin_table_to_pinned(gbin_ctx *ctx, const gbin_table *dev, void *stream, gbin_table *host) {
     if (!ctx || !dev || !host || !dev->on_device) return GBIN_E_INVALID_ARG;
-    CU(cudaSetDevice(ctx->cfg.device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    cudaStream_t st;
+    CU(begin_call(ctx, stream, &st));
     int rc = table_to_pinned(ctx, *dev, nullptr, st, host);
     if (rc) return rc;
     CU(cudaStreamSynchronize(st));
@@ -1433,14 +1428,11 @@ int split_reads_impl(gbin_ctx *ctx, const char *d_data, uint64_t size, int read_
     uint32_t *tile_counts = ctx->split_tiles_buf.as<uint32_t>();
     *launches += split_find_newlines(data, size, tile_counts, tile_counts + tiles, nullptr, &dm->split_n_nl, false, st);
     CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(&hm->split_n_nl, &dm->split_n_nl, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     // the last line may lack its newline: it still is a line for fgets
-    char last = 0;
-    CU(cudaMemcpyAsync(&hm->pad, d_data + size - 1, 1, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    memcpy(&last, &hm->pad, 1);
+    CU(cudaMemcpyAsync(&hm->last_byte, d_data + size - 1, 1, cudaMemcpyDeviceToHost, st));
+    CU(read_back(ctx, &Misc::split_n_nl, st));
     const uint64_t n_nl = hm->split_n_nl;
-    const uint64_t n_lines = n_nl + (last != '\n' ? 1 : 0);
+    const uint64_t n_lines = n_nl + (hm->last_byte != '\n' ? 1 : 0);
     if (n_lines >= (1ull << 32) - 1) return fail(ctx, GBIN_E_TOO_LARGE, "more than 2^32-1 lines in one file image");
     CU(ctx->split_nl.ensure((n_nl + 1) * sizeof(uint64_t)));
     *launches += split_find_newlines(data, size, tile_counts, nullptr, ctx->split_nl.as<uint64_t>(), nullptr, true, st);
@@ -1449,8 +1441,7 @@ int split_reads_impl(gbin_ctx *ctx, const char *d_data, uint64_t size, int read_
     *launches += split_count_reads(ctx->split_nl.as<uint64_t>(), n_nl, size, cap, n_lines, ctx->split_base.as<uint32_t>(),
                                    ctx->scan_scratch.as<uint32_t>(), &dm->split_n_reads, st);
     CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(&hm->split_n_reads, &dm->split_n_reads, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
+    CU(read_back(ctx, &Misc::split_n_reads, st));
     const uint64_t n_reads = hm->split_n_reads;
     CU(ctx->d_starts.ensure((n_reads + 1) * sizeof(uint64_t)));
     CU(ctx->d_lens.ensure((n_reads + 1) * sizeof(uint32_t)));
@@ -1475,8 +1466,8 @@ int gbin_copy_to_host(gbin_ctx *ctx, void *host_dst, const void *device_src, uin
 
 int gbin_split_reads_device(gbin_ctx *ctx, const char *d_data, uint64_t data_bytes, int read_length_define, void *stream, gbin_reads *out) {
     if (!ctx || !out || (data_bytes && !d_data)) return GBIN_E_INVALID_ARG;
-    CU(cudaSetDevice(ctx->cfg.device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    cudaStream_t st;
+    CU(begin_call(ctx, stream, &st));
     int launches = 0;
     int rc = split_reads_impl(ctx, d_data, data_bytes, read_length_define, st, out, &launches);
     if (rc) return rc;
@@ -1487,8 +1478,8 @@ int gbin_split_reads_device(gbin_ctx *ctx, const char *d_data, uint64_t data_byt
 
 int gbin_bin_file_host(gbin_ctx *ctx, const char *path, int read_length_define, gbin_table *out) {
     if (!ctx || !path || !out) return GBIN_E_INVALID_ARG;
-    CU(cudaSetDevice(ctx->cfg.device));
-    cudaStream_t st = ctx->stream;
+    cudaStream_t st;
+    CU(begin_call(ctx, nullptr, &st));
     FILE *f = fopen(path, "rb");
     if (!f) return fail(ctx, GBIN_E_IO, "cannot open %s", path);
     if (fseek(f, 0, SEEK_END) != 0) {
@@ -1513,9 +1504,9 @@ int gbin_bin_file_host(gbin_ctx *ctx, const char *path, int read_length_define, 
     fclose(f);
     if (got != size) return fail(ctx, GBIN_E_IO, "short read on %s", path);
     int launches = 0;
-    CU(cudaEventRecord(ctx->ev[0], st));
+    CU(cudaEventRecord(ctx->ev[EV_START], st));
     if (size) CU(cudaMemcpyAsync(ctx->d_reads.p, ctx->h_file.p, size, cudaMemcpyHostToDevice, st));
-    CU(cudaEventRecord(ctx->ev[1], st));
+    CU(cudaEventRecord(ctx->ev[EV_READS_ON_DEVICE], st));
     gbin_reads rd;
     int rc = split_reads_impl(ctx, ctx->d_reads.as<char>(), size, read_length_define, st, &rd, &launches);
     if (rc) return rc;
@@ -1524,7 +1515,7 @@ int gbin_bin_file_host(gbin_ctx *ctx, const char *path, int read_length_define, 
     if (rc) return rc;
     rc = table_to_pinned(ctx, dev, nullptr, st, out);
     if (rc) return rc;
-    CU(cudaEventRecord(ctx->ev[5], st));
+    CU(cudaEventRecord(ctx->ev[EV_TABLE_ON_HOST], st));
     CU(cudaStreamSynchronize(st));
     finish_timings(ctx, launches, true);
     return GBIN_OK;
@@ -1537,22 +1528,19 @@ int gbin_table_digest(gbin_ctx *ctx, const gbin_table *t, void *stream, uint64_t
         return GBIN_OK;
     }
     if (!ctx) return GBIN_E_INVALID_ARG;
-    CU(cudaSetDevice(ctx->cfg.device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
-    Misc *dm = ctx->misc.as<Misc>();
-    Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
-    table_digest_device(t, &dm->n_real_entries, st);
+    cudaStream_t st;
+    CU(begin_call(ctx, stream, &st));
+    table_digest_device(t, &ctx->misc.as<Misc>()->digest, st);
     CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(&hm->n_real_entries, &dm->n_real_entries, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    *digest_out = hm->n_real_entries;
+    CU(read_back(ctx, &Misc::digest, st));
+    *digest_out = static_cast<Misc *>(ctx->h_misc.p)->digest;
     return GBIN_OK;
 }
 
 int gbin_expand_read_ids_device(gbin_ctx *ctx, const gbin_table *t, void *stream, gbin_expanded *out) {
     if (!ctx || !t || !out || !t->on_device) return GBIN_E_INVALID_ARG;
-    CU(cudaSetDevice(ctx->cfg.device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    cudaStream_t st;
+    CU(begin_call(ctx, stream, &st));
     const uint64_t K = (uint64_t)t->kmer_size, S = t->n_kmers, N = t->n_ids;
     size_t free_b = 0, total_b = 0;
     CU(cudaMemGetInfo(&free_b, &total_b));
@@ -1623,8 +1611,8 @@ int gbin_table_to_host(gbin_ctx *ctx, const gbin_table *dev, gbin_table *host) {
 
 int gbin_count_instances_device(gbin_ctx *ctx, const gbin_reads *reads, void *stream, uint64_t *n_out) {
     if (!ctx || !reads || !n_out) return GBIN_E_INVALID_ARG;
-    CU(cudaSetDevice(ctx->cfg.device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    cudaStream_t st;
+    CU(begin_call(ctx, stream, &st));
     uint32_t max_len = 0;
     int launches = 0;
     return plan_reads(ctx, reads, st, n_out, &max_len, &launches);
@@ -1633,8 +1621,8 @@ int gbin_count_instances_device(gbin_ctx *ctx, const gbin_reads *reads, void *st
 int gbin_scan_reads_device(gbin_ctx *ctx, const gbin_reads *reads, uint32_t arrival_base, void *d_records, uint64_t capacity,
                            void *stream, uint64_t *n_out) {
     if (!ctx || !reads || !n_out) return GBIN_E_INVALID_ARG;
-    CU(cudaSetDevice(ctx->cfg.device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    cudaStream_t st;
+    CU(begin_call(ctx, stream, &st));
     uint64_t n = 0;
     uint32_t max_len = 0;
     int launches = 0;
@@ -1645,12 +1633,10 @@ int gbin_scan_reads_device(gbin_ctx *ctx, const gbin_reads *reads, uint32_t arri
     if (n && !d_records) return GBIN_E_INVALID_ARG;
     rc = run_scan(ctx, reads, arrival_base, d_records, max_len, st, &launches);
     if (rc) return rc;
-    Misc *dm = ctx->misc.as<Misc>();
-    Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
-    CU(cudaMemcpyAsync(&hm->bad_bases, &dm->bad_bases, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
+    CU(read_back(ctx, &Misc::grp, st));
     ctx->prof.collect();
-    if (hm->bad_bases) return fail(ctx, GBIN_E_NON_ACGT, "%llu bases other than A/C/G/T in the batch", hm->bad_bases);
+    const unsigned long long bad = static_cast<Misc *>(ctx->h_misc.p)->grp.bad_bases;
+    if (bad) return fail(ctx, GBIN_E_NON_ACGT, "%llu bases other than A/C/G/T in the batch", bad);
     *n_out = n;
     ctx->tm.kernel_launches = (uint32_t)launches;
     return GBIN_OK;
@@ -1658,20 +1644,9 @@ int gbin_scan_reads_device(gbin_ctx *ctx, const gbin_reads *reads, uint32_t arri
 
 int gbin_partition_records_device(gbin_ctx *ctx, const void *d_records, uint64_t n, uint32_t n_parts, void *d_out, void *stream,
                                   uint64_t *counts_host) {
-    if (!ctx || !counts_host || n_parts == 0 || n_parts > 256) return GBIN_E_INVALID_ARG;
-    if (n >= (1ull << 32) - 8192) return fail(ctx, GBIN_E_TOO_LARGE, "too many records in one partition call");
-    CU(cudaSetDevice(ctx->cfg.device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
-    Misc *dm = ctx->misc.as<Misc>();
-    Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
-    CU(ctx->radix_scratch.ensure(radix_scratch_bytes(n)));
-    int launches = radix_partition_by_owner(d_records, d_out, n, ctx->KW, n_parts, ctx->radix_scratch.p, dm->part_counts, st);
-    CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(hm->part_counts, dm->part_counts, sizeof(uint64_t) * n_parts, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    memcpy(counts_host, hm->part_counts, sizeof(uint64_t) * n_parts);
-    ctx->tm.kernel_launches = (uint32_t)launches;
-    return GBIN_OK;
+    return partition_by_owner(ctx, n, n_parts, stream, counts_host, [&](void *scratch, uint64_t *d_counts, cudaStream_t st) {
+        return radix_partition_by_owner(d_records, d_out, n, ctx->KW, n_parts, scratch, d_counts, st);
+    });
 }
 
 // ---------------------------------------------------------------- owner exchange over peer memory
@@ -1685,6 +1660,18 @@ struct XchgHandle {  // what a rank publishes: GBIN_XCHG_HANDLE_BYTES
 };
 static_assert(sizeof(XchgHandle) <= GBIN_XCHG_HANDLE_BYTES, "handle blob size");
 constexpr uint32_t XCHG_MAGIC = 0x67786331u;
+
+// Starts the context's exchange plan over its own buffers; the caller fills in the peers' (cap, peer_recv, peer_sh).
+void init_xchg_plan(gbin_ctx *ctx) {
+    auto &x = ctx->xg;
+    if (x.n_opened) gbin_xchg_detach(ctx);  // a second attach replaces the first one's mappings
+    memset(&x.plan, 0, sizeof x.plan);
+    x.plan.timeout_cycles = (long long)ctx->xchg_timeout_ms * 2000000ll;  // about 2 GHz
+    x.plan.rank = x.rank;
+    x.plan.world = x.world;
+    x.plan.dst_tab = x.dst_tab;
+    x.plan.result = x.result;
+}
 }  // namespace
 
 int gbin_xchg_create(gbin_ctx *ctx, uint32_t rank, uint32_t world, uint64_t capacity_records, void *handle_out) {
@@ -1722,13 +1709,7 @@ int gbin_xchg_attach(gbin_ctx *ctx, const void *all_handles) {
     if (!ctx || !all_handles || !ctx->xg.created) return GBIN_E_INVALID_ARG;
     CU(cudaSetDevice(ctx->cfg.device));
     auto &x = ctx->xg;
-    if (x.n_opened) gbin_xchg_detach(ctx);  // a second attach replaces the first one's mappings
-    memset(&x.plan, 0, sizeof x.plan);
-    x.plan.timeout_cycles = (long long)ctx->xchg_timeout_ms * 2000000ll;  // about 2 GHz
-    x.plan.rank = x.rank;
-    x.plan.world = x.world;
-    x.plan.dst_tab = x.dst_tab;
-    x.plan.result = x.result;
+    init_xchg_plan(ctx);
     for (uint32_t r = 0; r < x.world; r++) {
         XchgHandle h;
         memcpy(&h, static_cast<const char *>(all_handles) + (size_t)r * GBIN_XCHG_HANDLE_BYTES, sizeof h);
@@ -1786,8 +1767,8 @@ int gbin_xchg_exchange_skr(gbin_ctx *ctx, const void *d_skr, uint64_t n, void *s
     if (!ctx || !d_recv_out || !n_recv_out || (n && !d_skr)) return GBIN_E_INVALID_ARG;
     if (!ctx->xg.attached) return fail(ctx, GBIN_E_STATE, "gbin_xchg_exchange_skr before gbin_xchg_create / gbin_xchg_attach");
     if (n >= (1ull << 32) - 8192) return fail(ctx, GBIN_E_TOO_LARGE, "too many records in one exchange call");
-    CU(cudaSetDevice(ctx->cfg.device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    cudaStream_t st;
+    CU(begin_call(ctx, stream, &st));
     auto &x = ctx->xg;
     CU(ctx->radix_scratch.ensure(radix_scratch_bytes(n)));
     x.plan.epoch = ++x.epoch;
@@ -1813,8 +1794,8 @@ uint32_t gbin_skr_record_bytes(const gbin_ctx *ctx) { return ctx ? (ctx->cfg.kme
 int gbin_scan_skr_device(gbin_ctx *ctx, const gbin_reads *reads, uint32_t arrival_base, void *d_skr, uint64_t capacity, void *stream,
                          uint64_t *n_skr_out, uint64_t *n_instances_out) {
     if (!ctx || !reads || !n_skr_out) return GBIN_E_INVALID_ARG;
-    CU(cudaSetDevice(ctx->cfg.device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    cudaStream_t st;
+    CU(begin_call(ctx, stream, &st));
     uint64_t n = 0, n_skr = 0;
     uint32_t max_len = 0;
     int launches = 0;
@@ -1823,7 +1804,7 @@ int gbin_scan_skr_device(gbin_ctx *ctx, const gbin_reads *reads, uint32_t arriva
     if (max_len > GBIN_MAX_READ_LEN) return fail(ctx, GBIN_E_TOO_LARGE, "read length %u exceeds GBIN_MAX_READ_LEN", max_len);
     if (n && !d_skr) return GBIN_E_INVALID_ARG;
     if (n) {
-        rc = run_v2_scan(ctx, reads, n, max_len, arrival_base, d_skr, capacity, st, &n_skr, &launches);
+        rc = run_skr_scan(ctx, reads, n, max_len, arrival_base, d_skr, capacity, st, &n_skr, &launches);
         if (rc) return rc;
     }
     ctx->prof.collect();
@@ -1834,33 +1815,22 @@ int gbin_scan_skr_device(gbin_ctx *ctx, const gbin_reads *reads, uint32_t arriva
 }
 
 int gbin_partition_skr_device(gbin_ctx *ctx, const void *d_skr, uint64_t n, uint32_t n_parts, void *d_out, void *stream, uint64_t *counts_host) {
-    if (!ctx || !counts_host || n_parts == 0 || n_parts > 256) return GBIN_E_INVALID_ARG;
-    if (n >= (1ull << 32) - 8192) return fail(ctx, GBIN_E_TOO_LARGE, "too many records in one partition call");
-    CU(cudaSetDevice(ctx->cfg.device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
-    Misc *dm = ctx->misc.as<Misc>();
-    Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
-    CU(ctx->radix_scratch.ensure(radix_scratch_bytes(n)));
-    int launches = radix_partition_skr_by_owner(d_skr, d_out, n, ctx->cfg.kmer_size <= 32 ? 8 : 12, n_parts, ctx->radix_scratch.p, dm->part_counts, st);
-    CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(hm->part_counts, dm->part_counts, sizeof(uint64_t) * n_parts, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    memcpy(counts_host, hm->part_counts, sizeof(uint64_t) * n_parts);
-    ctx->tm.kernel_launches = (uint32_t)launches;
-    return GBIN_OK;
+    return partition_by_owner(ctx, n, n_parts, stream, counts_host, [&](void *scratch, uint64_t *d_counts, cudaStream_t st) {
+        return radix_partition_skr_by_owner(d_skr, d_out, n, ctx->cfg.kmer_size <= 32 ? 8 : 12, n_parts, scratch, d_counts, st);
+    });
 }
 
 int gbin_group_skr_device(gbin_ctx *ctx, void *d_skr, uint64_t n_skr, const int32_t *d_ids_by_arrival, int32_t id_base, void *stream,
                           gbin_table *out, int *used_fallback) {
     if (!ctx || !out || (n_skr && !d_skr)) return GBIN_E_INVALID_ARG;
     if (n_skr >= (1ull << 31)) return fail(ctx, GBIN_E_TOO_LARGE, "too many super-k-mer records in one call");
-    CU(cudaSetDevice(ctx->cfg.device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    cudaStream_t st;
+    CU(begin_call(ctx, stream, &st));
     int launches = 0;
     if (used_fallback) *used_fallback = 0;
-    CU(cudaEventRecord(ctx->ev[0], st));
-    CU(cudaEventRecord(ctx->ev[1], st));
-    CU(cudaEventRecord(ctx->ev[2], st));
+    CU(cudaEventRecord(ctx->ev[EV_START], st));
+    CU(cudaEventRecord(ctx->ev[EV_READS_ON_DEVICE], st));
+    CU(cudaEventRecord(ctx->ev[EV_SCANNED], st));
     bool done = false;
     uint64_t n = 0;
     int used = 2;
@@ -1874,12 +1844,11 @@ int gbin_group_skr_device(gbin_ctx *ctx, void *d_skr, uint64_t n_skr, const int3
             return fail(ctx, GBIN_E_STATE, "a shared-memory unit overflowed; re-run this batch through gbin_group_records_device");
         }
     } else {
-        Misc *dm = ctx->misc.as<Misc>();
-        CU(cudaMemsetAsync(&dm->bad_bases, 0, sizeof(unsigned long long), st));
-        int rc = run_group(ctx, nullptr, nullptr, 0, d_ids_by_arrival, id_base, st, out, &launches, ctx->ev[3]);
+        CU(cudaMemsetAsync(&ctx->misc.as<Misc>()->grp.bad_bases, 0, sizeof(unsigned long long), st));
+        int rc = run_group(ctx, nullptr, nullptr, 0, d_ids_by_arrival, id_base, st, out, &launches, ctx->ev[EV_SORTED]);
         if (rc) return rc;
     }
-    CU(cudaEventRecord(ctx->ev[4], st));
+    CU(cudaEventRecord(ctx->ev[EV_GROUPED], st));
     CU(cudaStreamSynchronize(st));
     finish_timings(ctx, launches, false);
     ctx->last_pipeline = used;
@@ -1890,19 +1859,18 @@ int gbin_group_records_device(gbin_ctx *ctx, void *d_records, uint64_t n, const 
                               void *stream, gbin_table *out) {
     if (!ctx || !out || (n && !d_records)) return GBIN_E_INVALID_ARG;
     if (n >= (1ull << 32) - 8192) return fail(ctx, GBIN_E_TOO_LARGE, "%llu records in one group call (limit 2^32)", (unsigned long long)n);
-    CU(cudaSetDevice(ctx->cfg.device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    cudaStream_t st;
+    CU(begin_call(ctx, stream, &st));
     const size_t rb = sizeof(uint64_t) * ctx->KW + 8;
     CU(ctx->rec_b.ensure((n + 1) * rb));
     int launches = 0;
-    Misc *dm = ctx->misc.as<Misc>();
-    CU(cudaMemsetAsync(&dm->bad_bases, 0, sizeof(unsigned long long), st));
-    CU(cudaEventRecord(ctx->ev[0], st));
-    CU(cudaEventRecord(ctx->ev[1], st));
-    CU(cudaEventRecord(ctx->ev[2], st));
-    int rc = run_group(ctx, d_records, ctx->rec_b.p, n, d_ids_by_arrival, id_base, st, out, &launches, ctx->ev[3]);
+    CU(cudaMemsetAsync(&ctx->misc.as<Misc>()->grp.bad_bases, 0, sizeof(unsigned long long), st));
+    CU(cudaEventRecord(ctx->ev[EV_START], st));
+    CU(cudaEventRecord(ctx->ev[EV_READS_ON_DEVICE], st));
+    CU(cudaEventRecord(ctx->ev[EV_SCANNED], st));
+    int rc = run_group(ctx, d_records, ctx->rec_b.p, n, d_ids_by_arrival, id_base, st, out, &launches, ctx->ev[EV_SORTED]);
     if (rc) return rc;
-    CU(cudaEventRecord(ctx->ev[4], st));
+    CU(cudaEventRecord(ctx->ev[EV_GROUPED], st));
     CU(cudaStreamSynchronize(st));
     finish_timings(ctx, launches, false);
     return GBIN_OK;
@@ -1939,13 +1907,7 @@ namespace {
 int multi_attach_local(gbin_multi *m, int g) {
     gbin_ctx *ctx = m->ctx[g];
     auto &x = ctx->xg;
-    if (x.n_opened) gbin_xchg_detach(ctx);  // a second attach replaces the first one's mappings
-    memset(&x.plan, 0, sizeof x.plan);
-    x.plan.timeout_cycles = (long long)ctx->xchg_timeout_ms * 2000000ll;  // about 2 GHz
-    x.plan.rank = x.rank;
-    x.plan.world = x.world;
-    x.plan.dst_tab = x.dst_tab;
-    x.plan.result = x.result;
+    init_xchg_plan(ctx);
     for (int r = 0; r < m->n; r++) {
         x.plan.cap[r] = m->ctx[r]->xg.cap;
         x.plan.peer_recv[r] = m->ctx[r]->xg.recv;

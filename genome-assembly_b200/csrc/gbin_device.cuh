@@ -78,15 +78,4 @@ __host__ __device__ inline uint32_t owner_of_mmer(uint32_t mmer_code, uint32_t p
     return (uint32_t)(((uint64_t)(mmer_code * 0x9E3779B1u) * parts) >> 32);
 }
 
-// getval (binning.c:91-111): T0 G1 C2 A3, anything else 3.
-__device__ __forceinline__ uint32_t base_code(uint32_t c, bool &valid) {
-    uint32_t v = 3;
-    valid = true;
-    if (c == 'C') v = 2;
-    else if (c == 'G') v = 1;
-    else if (c == 'T') v = 0;
-    else if (c != 'A') valid = false;
-    return v;
-}
-
 }  // namespace gbin

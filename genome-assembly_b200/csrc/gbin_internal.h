@@ -60,7 +60,6 @@ int launch_count_windows(const ReadsView &rv, int K, uint32_t *counts, cudaStrea
 int launch_scan_reads(const ReadsView &rv, const uint64_t *rec_off, int K, int M, int KW, uint32_t arrival_base, uint32_t max_len,
                       void *out, unsigned long long *bad_bases, int sm_count, cudaStream_t st);
 uint32_t scan_reads_max_len();
-int launch_pack_reads(const ReadsView &rv, uint32_t words_per_read, uint32_t *packed, unsigned long long *bad_bases, cudaStream_t st);
 
 // ---- radix_sort.cu
 // Stable LSD radix sort of n records by (mmer, kmer) ascending.  The result lands in `a` or `b`;
@@ -156,7 +155,6 @@ int v3_plan_runs(const uint64_t *ent, const uint16_t *sorted_info, uint64_t n_en
 uint64_t v3_max_units(uint64_t n_inst, uint64_t n_runs, int cap);
 size_t v3_unit_bytes();
 size_t v3_unit_out_bytes();
-size_t v3_counters_bytes();
 struct V3Counters {  // mirror of G3Counters in bin3.cu
     unsigned long long distinct, total_kmers, total_ids;
     unsigned int overflow, n_units, n_spans, pad;

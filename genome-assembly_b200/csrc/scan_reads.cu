@@ -108,33 +108,6 @@ __global__ void __launch_bounds__(SCAN_WARPS * 32)
     if (nbad) atomicAdd(bad_bases, (unsigned long long)nbad);
 }
 
-// ---- standalone pack kernel: ASCII -> 2-bit packed reads in HBM (16 bases per u32, MSB first),
-// row r at packed[r * words_per_read].  Not on the fused path above (which packs in shared
-// memory); exported for consumers that want the packed form and for packing parity tests.
-__global__ void pack_reads_kernel(ReadsView rv, uint32_t words_per_read, uint32_t *__restrict__ packed,
-                                  unsigned long long *__restrict__ bad_bases) {
-    const uint64_t gw = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const uint64_t r = gw / words_per_read;
-    const uint32_t j = (uint32_t)(gw % words_per_read);
-    if (r >= rv.n_reads) return;
-    const uint32_t L = rv.len(r);
-    const uint8_t *src = rv.data + rv.start(r);
-    uint32_t word = 0, nbad = 0;
-#pragma unroll
-    for (int t = 0; t < 16; t++) {
-        const uint32_t p = 16 * j + t;
-        uint32_t v = 0;
-        if (p < L) {
-            bool ok;
-            v = base_code(src[p], ok);
-            nbad += ok ? 0 : 1;
-        }
-        word = (word << 2) | v;
-    }
-    packed[gw] = word;
-    if (nbad) atomicAdd(bad_bases, (unsigned long long)nbad);
-}
-
 // ------------------------------------------------------------------ host launchers
 
 int launch_count_windows(const ReadsView &rv, int K, uint32_t *counts, cudaStream_t st) {
@@ -185,13 +158,6 @@ uint32_t scan_reads_max_len() {
         else hi = mid - 1;
     }
     return lo;
-}
-
-int launch_pack_reads(const ReadsView &rv, uint32_t words_per_read, uint32_t *packed, unsigned long long *bad_bases, cudaStream_t st) {
-    const uint64_t total = rv.n_reads * words_per_read;
-    if (total == 0) return 0;
-    pack_reads_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(rv, words_per_read, packed, bad_bases);
-    return 1;
 }
 
 }  // namespace gbin

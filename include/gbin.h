@@ -151,13 +151,16 @@ int gbin_table_digest(gbin_ctx *ctx, const gbin_table *table, void *stream, uint
 
 int gbin_get_timings(const gbin_ctx *ctx, gbin_timings *out);
 
-/* Two device pipelines produce the same table:
- *   2 (default): super-k-mer records -> stable sort by m-mer -> grouping/prune/emit in shared memory; a batch
+/* Three device pipelines produce the same table:
+ *   3 (default): super-k-mer records -> entries sorted by a reference to their record -> grouping/prune/emit, one warp per
+ *                unit; a batch with a (bucket, d) class larger than a unit is transparently redone by pipeline 2;
+ *   2          : super-k-mer records -> stable sort by m-mer -> grouping/prune/emit in shared memory; a batch
  *                that does not fit its shared-memory units (e.g. one k-mer with thousands of instances)
  *                is transparently redone by pipeline 1;
  *   1          : expanded k-mer instance records -> stable radix sort on (m-mer, k-mer) in HBM -> run-length/prune/emit.
- * The environment variable GBIN_PIPELINE=1 selects pipeline 1 at context creation. */
-/* Sizes of the intermediate structures of the last pipeline-2 run (0 when pipeline 1 produced the table). */
+ * So the fallback order is 3 -> 2 -> 1.  The environment variable GBIN_PIPELINE=1|2|3 selects the pipeline at context
+ * creation. */
+/* Sizes of the intermediate structures of the last pipeline-2 or pipeline-3 run (0 when pipeline 1 produced the table). */
 typedef struct gbin_run_stats {
     uint64_t n_super_kmers; /* records emitted by the scan stage */
     uint64_t n_mmer_runs;   /* distinct m-mer codes before the prune (level-1 buckets) */
