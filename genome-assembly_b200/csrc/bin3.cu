@@ -1171,15 +1171,8 @@ __global__ void v3_chunk_bounds_kernel(const Unit3 *__restrict__ units, const G3
 // ------------------------------------------------------------------ host side
 
 // cap: instances per unit, 512 or 1024 (gbin_set_tuning "v3_cap")
-// Two grouping launches (see group3_kernel's size_class): for one-word k-mers at capacity 1024, unless GBIN_V3_HYBRID=0.
-static bool v3_hybrid(const KeyLayout &kl, int cap_i) {
-    static int on = -1;
-    if (on < 0) {
-        const char *e = getenv("GBIN_V3_HYBRID");
-        on = e ? atoi(e) : 1;
-    }
-    return on && cap_i != 512 && kl.K <= 32;
-}
+// Two grouping launches (see group3_kernel's size_class): for one-word k-mers at capacity 1024.
+static bool v3_hybrid(const KeyLayout &kl, int cap_i) { return cap_i != 512 && kl.K <= 32; }
 static Plan3 v3_plan_params(const KeyLayout &kl, int cap_i) {
     const uint32_t cap = cap_i == 512 ? 512u : 1024u;
     Plan3 pp{cap, cap / 8, cap / 4, (uint32_t)(kl.K - kl.M + 1), cap, cap / 8, cap / 4};  // NB_MAX and ECAP of WarpLayout
@@ -1255,15 +1248,6 @@ int v3_group_launch(const void *skr, const uint64_t *ent, const void *units, con
     int per_sm_s = (int)((size_t)(227 * 1024) / (smem_s + 1024));
     if (per_sm_s < 1) per_sm_s = 1;
     int launches = 0;
-    static int sbs = -1, l_per_sm = 2;  // GBIN_V3_SBS=0: the two launches one after the other; GBIN_V3_LPS: CTAs per SM of the large-unit kernel
-    if (sbs < 0) {
-        const char *e = getenv("GBIN_V3_SBS");
-        sbs = e ? atoi(e) : 1;
-        const char *f = getenv("GBIN_V3_LPS");
-        l_per_sm = f ? atoi(f) : 2;
-        if (l_per_sm < 1 || l_per_sm > 2) l_per_sm = 2;
-    }
-    const bool side_by_side = sbs && ch.aux && ch.ev_fork && ch.ev_join;
     auto launch = [&](auto kern, auto kern_small, auto fin_kern) {
         cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (hybrid) cudaFuncSetAttribute(kern_small, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_s);
@@ -1272,15 +1256,12 @@ int v3_group_launch(const void *skr, const uint64_t *ent, const void *units, con
                 bool on = prof && prof->begin(KK_SKR_GROUP, st);
                 if (!hybrid) {
                     kern<<<sm_count * per_sm, WARPS * 32, smem, st>>>(sk, ent, un, kl, cutoff, ids_by_arrival, id_base, stg, gc, ch.bounds, c, ch.tickets, 0u);
-                } else if (!side_by_side) {
-                    kern<<<sm_count * per_sm, WARPS * 32, smem, st>>>(sk, ent, un, kl, cutoff, ids_by_arrival, id_base, stg, gc, ch.bounds, c, ch.tickets, 2u);
-                    kern_small<<<sm_count * per_sm_s, WARPS * 32, smem_s, st>>>(sk, ent, un, kl, cutoff, ids_by_arrival, id_base, stg, gc, ch.bounds, c, ch.tickets + ch.n, 1u);
                 } else {
-                    // side by side: the large-unit kernel goes first, the small-unit kernel's CTAs take what is left of
+                    // side by side: the large-unit kernel goes first at 2 CTAs per SM, the small-unit kernel's CTAs take what is left of
                     // every SM and, being persistent, the room the other kernel leaves when it runs out of units (its tail is covered)
                     cudaEventRecord(ch.ev_fork, st);
                     cudaStreamWaitEvent(ch.aux, ch.ev_fork, 0);
-                    kern<<<sm_count * l_per_sm, WARPS * 32, smem, st>>>(sk, ent, un, kl, cutoff, ids_by_arrival, id_base, stg, gc, ch.bounds, c, ch.tickets, 2u);
+                    kern<<<sm_count * 2, WARPS * 32, smem, st>>>(sk, ent, un, kl, cutoff, ids_by_arrival, id_base, stg, gc, ch.bounds, c, ch.tickets, 2u);
                     kern_small<<<sm_count * per_sm_s, WARPS * 32, smem_s, ch.aux>>>(sk, ent, un, kl, cutoff, ids_by_arrival, id_base, stg, gc, ch.bounds, c, ch.tickets + ch.n, 1u);
                     cudaEventRecord(ch.ev_join, ch.aux);
                     cudaStreamWaitEvent(st, ch.ev_join, 0);
@@ -1304,25 +1285,14 @@ int v3_group_launch(const void *skr, const uint64_t *ent, const void *units, con
             if (ch.done) cudaEventRecord(ch.done[c], st);
         }
     };
-    static int uu = 0;  // GBIN_V3_U = 1|2|4: instances per lane in flight (experiments)
-    if (!uu) {
-        const char *e = getenv("GBIN_V3_U");
-        uu = e ? atoi(e) : 0;
-        if (uu != 1 && uu != 2 && uu != 4) uu = -1;
-    }
-    const int u_sel = uu > 0 ? uu : (cap == 512 ? 2 : 4);  // more warps per SM at 512: less need for instruction-level parallelism, smaller code
-#define G3_LAUNCH(PW_, KW_, CAP_) \
-    (u_sel == 1 ? launch(group3_kernel<PW_, KW_, CAP_, WARPS, 1>, group3_kernel<PW_, KW_, 512, WARPS, 2>, finalize3_kernel<KW_>) \
-             : (u_sel == 2 ? launch(group3_kernel<PW_, KW_, CAP_, WARPS, 2>, group3_kernel<PW_, KW_, 512, WARPS, 2>, finalize3_kernel<KW_>) \
-                           : launch(group3_kernel<PW_, KW_, CAP_, WARPS, 4>, group3_kernel<PW_, KW_, 512, WARPS, 2>, finalize3_kernel<KW_>)))
+    // instances per lane in flight: 4 at capacity 1024, 2 at 512 (more warps per SM there: less need for instruction-level parallelism, smaller code)
     if (KW == 1) {
-        if (cap == 512) G3_LAUNCH(2, 1, 512);
-        else G3_LAUNCH(2, 1, 1024);
+        if (cap == 512) launch(group3_kernel<2, 1, 512, WARPS, 2>, group3_kernel<2, 1, 512, WARPS, 2>, finalize3_kernel<1>);
+        else launch(group3_kernel<2, 1, 1024, WARPS, 4>, group3_kernel<2, 1, 512, WARPS, 2>, finalize3_kernel<1>);
     } else {
-        if (cap == 512) G3_LAUNCH(4, 2, 512);
-        else G3_LAUNCH(4, 2, 1024);
+        if (cap == 512) launch(group3_kernel<4, 2, 512, WARPS, 2>, group3_kernel<4, 2, 512, WARPS, 2>, finalize3_kernel<2>);
+        else launch(group3_kernel<4, 2, 1024, WARPS, 4>, group3_kernel<4, 2, 512, WARPS, 2>, finalize3_kernel<2>);
     }
-#undef G3_LAUNCH
     return launches;
 }
 
@@ -1630,13 +1600,8 @@ int v3_lsd_finish(const KeyLayout &kl, uint64_t n, void *rec_a, void *rec_b, voi
     bool in_b = false;
     int passes = 0;
     int l = 0;
-    static int span_sort_on = -1;  // GBIN_V3_SPAN_SORT=0: always the global sort (experiments)
-    if (span_sort_on < 0) {
-        const char *e = getenv("GBIN_V3_SPAN_SORT");
-        span_sort_on = e ? atoi(e) : 1;
-    }
     bool need_global = true;
-    if (span_sort_on && n < (1ull << 31)) {
+    if (n < (1ull << 31)) {
         uint32_t *work32 = reinterpret_cast<uint32_t *>(dnew);  // [n + 2] u64 = [2 n + 4] u32; free until the list-length scan below
         bool on = prof && prof->begin(KK_V3_SPAN, st);
         const int ls_ = KW == 1 ? v3_span_sort<1>(rec_a, rec_b, n, work32, scan_scratch, sm_count, st) : v3_span_sort<2>(rec_a, rec_b, n, work32, scan_scratch, sm_count, st);

@@ -731,10 +731,8 @@ int run_v3_pass(gbin_ctx *ctx, const void *skr, const uint64_t *ent, const uint1
     CU(ctx->v3_unit_out.ensure(max_units * v3_unit_out_bytes()));
     CU(ctx->v3_unit_excl.ensure((2 * max_units + 2) * 8));
     CU(ctx->scan_scratch.ensure(group_scan_scratch_bytes(n_runs + max_units + 1024)));
-    V3Chunks ch{1u, dm->v3_tickets, dm->chunk_bounds, &dm->v3_chunk_sum, dm->chunk_totals, dm->lsd_totals, nullptr, nullptr, nullptr};
-    ch.aux = ctx->st_aux;
-    ch.ev_fork = ctx->ev_fork;
-    ch.ev_join = ctx->ev_join;
+    V3Chunks ch{1u, dm->v3_tickets, dm->chunk_bounds, &dm->v3_chunk_sum, dm->chunk_totals, dm->lsd_totals, nullptr, nullptr, nullptr,
+                ctx->st_aux, ctx->ev_fork, ctx->ev_join};
     if (single_pass && sink && sink->chunks > 1) {
         ch.n = (uint32_t)sink->chunks;
         ch.totals_host = hm->chunk_totals;

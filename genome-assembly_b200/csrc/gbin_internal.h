@@ -192,8 +192,8 @@ struct V3Chunks {
     unsigned long long *lsd_totals_dev;  // device, [n]: the same for the k-mers handed to the global sort
     unsigned long long *totals_host, *lsd_totals_host;  // pinned, [n] or nullptr
     cudaEvent_t *done;                // [n] or nullptr
-    cudaStream_t aux = nullptr;       // second stream + two events (no timing): the two grouping launches of a chunk run side by side
-    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
+    cudaStream_t aux;                 // second stream + two events (no timing): the two grouping launches of a chunk run side by side
+    cudaEvent_t ev_fork, ev_join;
 };
 size_t v3_group_smem_bytes(int KW, int cap);
 int v3_group_launch(const void *skr, const uint64_t *ent, const void *units, const KeyLayout &kl, int cap, int cutoff, const int32_t *ids_by_arrival, int32_t id_base,

@@ -27,15 +27,16 @@
 
 namespace gbin {
 
-// A unit holds at most CAP k-mer instances (template parameter of the kernel: 1280 by default, 2048 or 4096).
-//   small buckets (<= t = CAP/4 instances) are packed into windows of win = 3*CAP/4 instances of the small-bucket
-//   prefix space, so a packed unit holds less than win + t = CAP instances and is about 75 % full on average;
+// A unit holds at most CAP = G_UNIT_CAP k-mer instances (1280: four CTAs per SM).
+//   small buckets (<= t = CAP/2 instances) are packed into windows of win = CAP/2 instances of the small-bucket
+//   prefix space, so a packed unit holds less than win + t = CAP instances and is about half full on average;
 //   a bucket with t < c <= CAP is a unit of its own; a larger one is cut into slices of about tsub = CAP/2.
+constexpr uint32_t G_UNIT_CAP = 1280;
 struct PlanParams {
     uint32_t cap, t, win, tsub;
 };
 constexpr int G_RANK_MAX = 512;  // up to this many survivors per unit are ordered by counting instead of a bitonic sort
-                                 // (their keys, 20 B each for 128-bit codes, plus a u16 rank array must fit the dead hash table: 16 KB at CAP 1280 and 2048)
+                                 // (their keys, 20 B each for 128-bit codes, plus a u16 rank array must fit the dead hash table: 16 KB at CAP 1280)
 
 struct __align__(16) Unit {
     uint32_t skr_begin, skr_end;  // range of sorted super-k-mer records; UNIT_RECORDS: range of expanded instance records
@@ -900,36 +901,17 @@ __global__ void empty_table_kernel2(uint64_t *mmer_kmer_off, uint64_t *kmer_id_o
 
 // ------------------------------------------------------------------ host side
 
-static int g_unit_cap() {  // GBIN_V2_CAP=1280|2048|4096 selects the unit capacity (default 1280: four CTAs per SM; 2048: three)
-    static int cap = 0;
-    if (!cap) {
-        const char *e = getenv("GBIN_V2_CAP");
-        const int v = e ? atoi(e) : 1280;
-        cap = (v == 4096 || v == 2048) ? v : 1280;
-    }
-    return cap;
-}
-static PlanParams plan_params() {
-    const uint32_t cap = (uint32_t)g_unit_cap();
-    static int eighths = 0;  // GBIN_V2_TSMALL = 1..4: small-bucket threshold in eighths of the capacity (default 4)
-    if (!eighths) {
-        const char *e = getenv("GBIN_V2_TSMALL");
-        eighths = e ? atoi(e) : 4;
-        if (eighths < 1 || eighths > 4) eighths = 4;
-    }
-    const uint32_t t = cap * eighths / 8;
-    return PlanParams{cap, t, cap - t, cap / 2};
-}
+static PlanParams plan_params() { return PlanParams{G_UNIT_CAP, G_UNIT_CAP / 2, G_UNIT_CAP / 2, G_UNIT_CAP / 2}; }
 
 size_t skr_group_smem_bytes(int KW) {
-    const size_t cap = (size_t)g_unit_cap();
+    const size_t cap = G_UNIT_CAP;
     const size_t hs = cap > 2048 ? 8192 : (cap > 1024 ? 4096 : 2048);  // hash slots, as in the kernel
     return KW * cap * 8 + cap * 4 * 2 + hs * 4 + cap * 4 + cap * 2 * 3 + 64;
 }
 
-uint64_t skr_max_units(uint64_t n_inst, uint64_t n_runs) { return n_inst / (g_unit_cap() / 4) + 2 * n_runs + 8; }
+uint64_t skr_max_units(uint64_t n_inst, uint64_t n_runs) { return n_inst / (G_UNIT_CAP / 4) + 2 * n_runs + 8; }
 size_t skr_unit_bytes() { return sizeof(Unit); }
-uint64_t skr_max_big_runs(uint64_t n_inst) { return n_inst / (uint64_t)g_unit_cap() + 2; }
+uint64_t skr_max_big_runs(uint64_t n_inst) { return n_inst / (uint64_t)G_UNIT_CAP + 2; }
 
 // Phase A (needs n_skr on the host): instance prefix and m-mer run starts in one fused scan.
 // both64: [n_skr + 1] u64 scratch; scratch64: prefix-scan scratch. *n_inst_dev / *n_runs_dev receive the totals.
@@ -1002,16 +984,8 @@ int skr_group_launch(const void *skr_sorted, int K, int cutoff, const uint32_t *
         }
     };
     const int per_sm = (int)((size_t)(227 * 1024) / (smem + 1024));  // CTAs per SM that shared memory allows
-    if (g_unit_cap() == 4096) {
-        if (KW == 1) launch(skr_group_kernel<2, 1, 4096, 512>, 512, 1);
-        else launch(skr_group_kernel<4, 2, 4096, 512>, 512, 1);
-    } else if (g_unit_cap() == 1280) {
-        if (KW == 1) launch(skr_group_kernel<2, 1, 1280, 256>, 256, per_sm < 4 ? per_sm : 4);
-        else launch(skr_group_kernel<4, 2, 1280, 256>, 256, per_sm < 4 ? per_sm : 4);
-    } else {
-        if (KW == 1) launch(skr_group_kernel<2, 1, 2048, 256>, 256, per_sm < 3 ? per_sm : 3);
-        else launch(skr_group_kernel<4, 2, 2048, 256>, 256, per_sm < 3 ? per_sm : 3);
-    }
+    if (KW == 1) launch(skr_group_kernel<2, 1, G_UNIT_CAP, 256>, 256, per_sm < 4 ? per_sm : 4);
+    else launch(skr_group_kernel<4, 2, G_UNIT_CAP, 256>, 256, per_sm < 4 ? per_sm : 4);
     return (int)(ch.totals_dev ? 2 * ch.n : ch.n);
 }
 

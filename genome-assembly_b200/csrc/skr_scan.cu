@@ -10,7 +10,6 @@
 // records leave the SM as one contiguous run of 16-byte stores.
 // The output is therefore in arrival order (read-major, segment-minor) and deterministic — the
 // later stable sort by m-mer keeps arrival order per bucket.
-#include <cstdlib>
 #include <type_traits>
 
 #include "gbin_device.cuh"
@@ -388,9 +387,7 @@ struct Scan2Shape {
 };
 static Scan2Shape skr_scan2_shape(int K, int M, uint32_t max_len) {
     Scan2Shape sh{0, false, 0, 0};
-    static int disabled = -1;
-    if (disabled < 0) disabled = getenv("GBIN_SCAN_HOPS") ? 1 : 0;  // experiments: keep the hop-chain kernel
-    if (disabled || max_len < (uint32_t)K) return sh;
+    if (max_len < (uint32_t)K) return sh;
     const uint32_t npos = max_len - M + 1;
     if (npos > 256u) return sh;
     sh.nj = npos <= 96u ? 3 : (npos <= 160u ? 5 : 8);
@@ -409,28 +406,27 @@ static Scan2Shape skr_scan2_shape(int K, int M, uint32_t max_len) {
 }
 
 // Tile shape: rpw reads per warp and a staging area of seg_cap records, sized for 1.6x the expected number of segments
-// (a segment covers about (K-M+2)/2 windows) within a 6 KB budget per warp; tiles that exceed it are redone in place.
+// (a segment covers about (K-M+2)/2 windows) within a budget of SKR_STAGE_BYTES per warp; tiles that exceed it are redone in place.
+constexpr uint32_t SKR_STAGE_BYTES = 6144;
 static void skr_tile_shape(int K, int M, uint32_t max_len, uint32_t *rpw_out, uint32_t *seg_cap_out) {
     const int NW = skr_words(K);
     const uint32_t W = max_len >= (uint32_t)K ? max_len - K + 1 : 1;
-    static uint32_t stage_bytes = 0;  // GBIN_SCAN_STAGE_BYTES: staging budget per warp (experiments)
-    if (!stage_bytes) {
-        const char *e = getenv("GBIN_SCAN_STAGE_BYTES");
-        stage_bytes = e ? (uint32_t)atoi(e) : 6144u;
-        if (stage_bytes < 1024u || stage_bytes > 16384u) stage_bytes = 6144u;
-    }
-    const uint32_t budget = stage_bytes / (NW * 4u);  // records
+    const uint32_t budget = SKR_STAGE_BYTES / (NW * 4u);  // records
     uint32_t per_read = (uint32_t)(1.6 * (double)W / ((K - M + 2) / 2.0)) + 2;
     if (per_read > W) per_read = W;
     uint32_t rpw = budget / per_read;
     if (rpw < 1) rpw = 1;
-    if (rpw > stage_bytes / 512u) rpw = stage_bytes / 512u;  // 12 reads per tile at the default budget
+    if (rpw > SKR_STAGE_BYTES / 512u) rpw = SKR_STAGE_BYTES / 512u;  // 12 reads per tile
     uint32_t cap = rpw * per_read;
     if (cap > budget) cap = budget;
     if (cap < 4) cap = 4;
     *rpw_out = rpw;
     *seg_cap_out = cap;
 }
+
+// ns between polls of a predecessor tile that has not published yet: the kernel is bound by instruction issue, so a
+// spinning warp takes issue slots from the warps that still compute
+constexpr uint32_t SKR_POLL_SLEEP_NS = 800;
 
 // Host launcher.  tile_state must hold skr_scan_tiles() u64 (zeroed here), ticket one u32 (zeroed here).
 // Returns kernels launched.
@@ -442,11 +438,6 @@ int launch_skr_scan(const ReadsView &rv_all, uint64_t read_begin, uint64_t read_
     rv.n_reads = read_end;  // the kernel treats n_reads as the end of its read range
     const int PW = skr_payload_units(K);
     const int NW = 4 + 2 * PW;
-    static int lkb_sleep = -1;
-    if (lkb_sleep < 0) {
-        const char *e = getenv("GBIN_SCAN_SLEEP");
-        lkb_sleep = e ? atoi(e) : 800;
-    }
     const Scan2Shape s2 = skr_scan2_shape(K, M, max_len);
     if (s2.nj) {
         const uint32_t ntiles = (uint32_t)((read_end - read_begin + s2.rpw - 1) / s2.rpw);
@@ -463,7 +454,7 @@ int launch_skr_scan(const ReadsView &rv_all, uint64_t read_begin, uint64_t read_
                 return;
             }
             kern<<<blocks, SKR_WARPS * 32, smem, st>>>(rv, read_begin, K, M, arrival_base, max_len, s2.rpw, s2.seg_cap, ntiles, static_cast<uint32_t *>(out),
-                                                       capacity, tile_state, ticket, counters, (uint32_t)lkb_sleep);
+                                                       capacity, tile_state, ticket, counters, SKR_POLL_SLEEP_NS);
         };
         auto pick_nj = [&](auto pw, auto key) {
             constexpr int P = decltype(pw)::value;
@@ -499,8 +490,6 @@ int launch_skr_scan(const ReadsView &rv_all, uint64_t read_begin, uint64_t read_
     if (blocks > (ntiles + warps - 1) / warps) blocks = (ntiles + warps - 1) / warps;
     // one-REDUX hops need score, inverted offset and strand bit in 32 bits (read_pack.cuh)
     const bool packed = 2 * M + 1 + ((K - M + 1) <= 32 ? 5 : 6) <= 32;
-    // ns between polls of a predecessor tile that has not published yet: the kernel is bound by instruction issue, so a
-    // spinning warp takes issue slots from the warps that still compute (GBIN_SCAN_SLEEP overrides, for experiments)
     bool attr_failed = false;
     auto launch = [&](auto kern) {
         if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
@@ -509,7 +498,7 @@ int launch_skr_scan(const ReadsView &rv_all, uint64_t read_begin, uint64_t read_
             return;
         }
         kern<<<blocks, warps * 32, smem, st>>>(rv, read_begin, K, M, arrival_base, max_len, rpw, seg_cap, ntiles, static_cast<uint32_t *>(out),
-                                                   capacity, tile_state, ticket, counters, (uint32_t)lkb_sleep);
+                                                   capacity, tile_state, ticket, counters, SKR_POLL_SLEEP_NS);
     };
     if (PW == 2) {
         if (packed) launch(skr_scan_kernel<2, true>);
