@@ -1883,20 +1883,25 @@ struct gbin_multi {
     std::vector<int> dev;
     uint64_t xchg_cap = 0;
     char err[512] = {0};
-    // a reusable barrier for the worker threads of one call
+    // A reusable barrier for the worker threads of one call.  It returns the OR of the flags all threads passed in, so that every
+    // thread takes the same decision after it, even while another thread already records its status of the next step.
     std::mutex mu;
     std::condition_variable cv;
-    int waiting = 0, generation = 0;
-    void barrier() {
+    int waiting = 0, generation = 0, flags_in = 0, flags_out = 0;
+    int barrier(int flags = 0) {
         std::unique_lock<std::mutex> lk(mu);
         const int gen = generation;
+        flags_in |= flags;
         if (++waiting == n) {
+            flags_out = flags_in;
+            flags_in = 0;
             waiting = 0;
             generation++;
             cv.notify_all();
         } else {
             cv.wait(lk, [&] { return gen != generation; });
         }
+        return flags_out;  // the next generation cannot complete before this thread has arrived at it
     }
 };
 
@@ -1982,6 +1987,7 @@ int gbin_multi_bin_reads_host(gbin_multi *m, const gbin_reads *reads, gbin_table
     if (reads->starts && !reads->lens) return GBIN_E_INVALID_ARG;
     std::vector<int> rcs(G, GBIN_OK);
     std::vector<uint64_t> n_skr(G, 0);
+    std::vector<uint64_t> part_counts((size_t)G * G, 0);  // [g * G + o]: instance records GPU g holds for owner o (overflow redo)
     std::vector<std::string> errs(G);
     m->err[0] = 0;
     auto work = [&](int g) {
@@ -2063,14 +2069,10 @@ int gbin_multi_bin_reads_host(gbin_multi *m, const gbin_reads *reads, gbin_table
         } else if (!rc) {
             n_skr[g] = 0;
         }
-        m->barrier();  // ---- every rank knows every rank's record count (and whether somebody failed)
-        bool any = false;
+        if (m->barrier(rc != GBIN_OK)) return;  // ---- somebody failed; else every rank knows every rank's record count
         uint64_t mx = 0;
-        for (int r = 0; r < G; r++) {
-            any = any || rcs[r] != GBIN_OK;
+        for (int r = 0; r < G; r++)
             if (n_skr[r] > mx) mx = n_skr[r];
-        }
-        if (any) return;
         void *d_recv = nullptr;
         uint64_t n_recv = 0;
         const uint64_t want = mx + mx / 3 + 65536;
@@ -2083,28 +2085,72 @@ int gbin_multi_bin_reads_host(gbin_multi *m, const gbin_reads *reads, gbin_table
             const int r2 = gbin_xchg_create(ctx, (uint32_t)g, (uint32_t)G, want + want / 8, blob);
             if (r2) failed(r2, "exchange buffers");
         }
-        m->barrier();  // ---- all buffers exist
-        for (int r = 0; r < G; r++) any = any || rcs[r] != GBIN_OK;
-        if (any) return;
+        if (m->barrier(rc != GBIN_OK)) return;  // ---- all buffers exist
         multi_attach_local(m, g);
         m->barrier();
         // ---- owner exchange (collective)
         const int rx = gbin_xchg_exchange_skr(ctx, ctx->skr_a.p, n_skr[g], st, &d_recv, &n_recv, nullptr);
-        if (rx) {
-            failed(rx, "owner exchange");
-            return;
-        }
+        if (rx) failed(rx, "owner exchange");
         }
         // ---- grouping of this GPU's buckets
-        int r2 = GBIN_OK;
         gbin_table dev;
-        int fell = 0;
-        r2 = gbin_group_skr_device(ctx, d_recv, n_recv, d_ids, reads->id_base, st, &dev, &fell);
-        if (r2) {
-            failed(r2, "grouping");
-            return;
+        int overflow = 0;
+        if (!rc) {
+            const int r2 = gbin_group_skr_device(ctx, d_recv, n_recv, d_ids, reads->id_base, st, &dev, &overflow);
+            if (r2 && !(r2 == GBIN_E_STATE && overflow)) failed(r2, "grouping");
         }
-        r2 = gbin_table_to_pinned(ctx, &dev, st, &tables_out[g]);
+        const int flags = m->barrier((rc != GBIN_OK) | (overflow ? 2 : 0));  // ---- did some rank fail, did some unit overflow
+        if (flags & 1) return;
+        if (flags & 2) {
+            // One k-mer had more instances than a unit holds and the super-k-mer records were consumed by the sort: every GPU redoes
+            // its shard in instance-record form (pipeline 1), which groups in HBM and cannot overflow.  Scan into rec_a, partition
+            // into skr_a (dead now), then every owner gathers its part of every GPU's partition, in rank order, into its rec_a.
+            const size_t rb = gbin_record_bytes(ctx);
+            uint64_t n_rec = 0;
+            if (ctx->rec_a.ensure((ninst + 1) * rb) != cudaSuccess) {
+                (void)cudaGetLastError();
+                failed(GBIN_E_NOMEM, "instance-record buffer");
+            }
+            if (!rc) {
+                const int r3 = gbin_scan_reads_device(ctx, &d, (uint32_t)lo, ctx->rec_a.p, ninst, st, &n_rec);
+                if (r3) failed(r3, "instance-record scan");
+            }
+            if (!rc && G > 1) {
+                if (ctx->skr_a.ensure((n_rec + 1) * rb) != cudaSuccess) {
+                    (void)cudaGetLastError();
+                    failed(GBIN_E_NOMEM, "partition buffer");
+                } else {
+                    const int r3 = gbin_partition_records_device(ctx, ctx->rec_a.p, n_rec, (uint32_t)G, ctx->skr_a.p, st, &part_counts[(size_t)g * G]);
+                    if (r3) failed(r3, "instance-record partition");
+                }
+            }
+            if (G > 1) {
+                if (m->barrier(rc != GBIN_OK)) return;  // ---- every rank's parts are in its skr_a, their sizes in part_counts
+                n_rec = 0;
+                for (int r = 0; r < G; r++) n_rec += part_counts[(size_t)r * G + g];
+                e = ctx->rec_a.ensure((n_rec + 1) * rb);
+                uint64_t at = 0;
+                for (int r = 0; r < G && e == cudaSuccess; r++) {
+                    uint64_t off = 0;
+                    for (int o = 0; o < g; o++) off += part_counts[(size_t)r * G + o];
+                    const uint64_t c = part_counts[(size_t)r * G + g];
+                    if (c) e = cudaMemcpyAsync(ctx->rec_a.as<char>() + at * rb, m->ctx[r]->skr_a.as<char>() + off * rb, c * rb, cudaMemcpyDefault, st);
+                    at += c;
+                }
+                if (e == cudaSuccess) e = cudaStreamSynchronize(st);  // (no rank writes its skr_a again in this call)
+                if (e != cudaSuccess) {
+                    (void)cudaGetLastError();
+                    failed(e == cudaErrorMemoryAllocation ? GBIN_E_NOMEM : GBIN_E_CUDA, "gathering the owner's records");
+                }
+            }
+            if (rc) return;
+            const int r3 = gbin_group_records_device(ctx, ctx->rec_a.p, n_rec, d_ids, reads->id_base, st, &dev);
+            if (r3) {
+                failed(r3, "grouping (instance records)");
+                return;
+            }
+        }
+        const int r2 = gbin_table_to_pinned(ctx, &dev, st, &tables_out[g]);
         if (r2) failed(r2, "table to host");
     };
     std::vector<std::thread> th;

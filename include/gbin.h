@@ -263,7 +263,10 @@ void gbin_xchg_destroy(gbin_ctx *ctx);
  * gbin_multi_bin_reads_host: reads in HOST memory; GPU g takes the contiguous read range [g*n/G, (g+1)*n/G), runs the scan, sends
  * every record to the owner of its m-mer bucket (gbin_owner_of; peer stores over NVLink, gbin_xchg_* with the peers' buffers passed
  * by address), groups what it received.  tables_out[g] (host arrays in context g's pinned arena, valid until the next call) is the
- * part of the table GPU g owns: disjoint m-mer buckets, together the table of a single-GPU run (their digests add up to its digest). */
+ * part of the table GPU g owns: disjoint m-mer buckets, together the table of a single-GPU run (their digests add up to its digest).
+ * When a shared-memory unit overflows on any GPU (one k-mer with more instances than a unit holds, e.g. homopolymer-rich reads), every
+ * GPU redoes its shard in instance-record form (gbin_scan_reads_device, gbin_partition_records_device, a gather of every GPU's part
+ * by its owner, gbin_group_records_device): same result. */
 typedef struct gbin_multi gbin_multi;
 int gbin_multi_create(const gbin_config *cfg, const int *devices, int n_devices, gbin_multi **out);
 void gbin_multi_destroy(gbin_multi *m);
