@@ -1,4 +1,4 @@
-// bin3.cu — pipeline v3: level 1 by reference, level 2 by one warp per unit.
+// bin3.cu — pipeline v3: level 1 by reference, level 2 by one warp (or one pair of warps) per unit.
 //
 // Input: the super-k-mer records of the scan stage, in arrival order (skr.cuh).  Stages:
 //   1. make_entries_kernel: one 8-byte entry {key << 32 | slot} per piece of a record (bin3.cuh) and the piece's
@@ -7,9 +7,9 @@
 //      two-level store (binning.c:1044-1049); inside a key entries stay in arrival order.
 //   3. planning (no atomics, no host round trip inside): instance prefix + atoms (runs of equal key) in one scan;
 //      units = packs of whole small atoms, single atoms, or the d-rounds of an atom larger than a unit.
-//   4. group3_kernel: every WARP owns one unit at a time — no CTA barrier anywhere.  The warp expands the windows of
-//      its pieces (rolling 2-bit shift, complement when is_rev — binning.c:1029-1040) into shared memory, groups
-//      equal (bucket, k-mer) keys with a hash whose slots hold instance indices (level-2 insert + ll_node push,
+//   4. group3_kernel: every WARP (512-instance units) or PAIR of warps (1024-instance units, synchronised by the pair's own
+//      named barrier) owns one unit at a time — no CTA barrier anywhere.  It expands the windows of its pieces (rolling
+//      2-bit shift, complement when is_rev — binning.c:1029-1040) into shared memory, groups equal (bucket, k-mer) keys with a hash whose slots hold instance indices (level-2 insert + ll_node push,
 //      binning.c:1052-1069), counts, prunes (count > ABUNDANCE_CUTOFF, binning.c:1094-1102), orders the survivors of
 //      every bucket by k-mer, orders every id list newest-first, obtains its place in the table from a two-level chained
 //      scan over units (aggregates are published right after the count, long before they are needed) and writes its part
@@ -444,12 +444,14 @@ __device__ __forceinline__ void front_kmer(const Payload<PW> &pl, int K, bool re
 }
 
 template <int WCAP, int KW>
-struct WarpLayout {  // per-warp shared memory; every region is a multiple of 16 bytes
+struct UnitLayout {  // shared memory of one unit in flight; every region is a multiple of 16 bytes
+    static constexpr int W = WCAP == 1024 ? 2 : 1;  // warps per unit: one at 512 instances, a pair at 1024
     static constexpr int NB_MAX = WCAP / 8;  // buckets of a packed unit
     static constexpr int ECAP = WCAP / 4;    // entries of a packed unit (an atom with more entries is a unit of its own)
     static constexpr int BSTART_BYTES = ((NB_MAX + 1) * 2 + 15) / 16 * 16;
-    static constexpr int BYTES = KW * WCAP * 8 /*keys*/ + WCAP * 4 /*table*/ + WCAP * 2 /*cnt*/ + WCAP * 2 /*grp*/ + WCAP * 2 /*rk*/ + WCAP /*eix*/ + BSTART_BYTES +
-                                 NB_MAX * 4 /*bmm*/ + ECAP * 4 /*eid*/ + ECAP /*ebk*/;
+    static constexpr int XCH_BYTES = W == 2 ? 64 : 0;  // the pair's exchange words: [2 slots][2 warps][4] u32
+    static constexpr int BYTES = KW * WCAP * 8 /*keys*/ + WCAP * 4 /*table*/ + W * WCAP * 2 /*cnt (+ cnt_lo)*/ + WCAP * 2 /*grp*/ + WCAP * 2 /*rk*/ + WCAP /*eix*/ +
+                                 BSTART_BYTES + NB_MAX * 4 /*bmm*/ + ECAP * 4 /*eid*/ + ECAP /*ebk*/ + XCH_BYTES;
 };
 
 __device__ __forceinline__ uint32_t warp_incl_scan_u32(uint32_t v, uint32_t lane) {
@@ -461,42 +463,102 @@ __device__ __forceinline__ uint32_t warp_incl_scan_u32(uint32_t v, uint32_t lane
     return v;
 }
 
-constexpr int G3_WARPS = 5;  // warps (= units in flight) per CTA
+// Synchronises the warps of one unit: __syncwarp for one warp, the pair's own named barrier (bar.sync id, 64) for two — never the
+// whole CTA, so a warp waits for its partner only.
+template <int W>
+__device__ __forceinline__ void unit_sync(uint32_t bar_id) {
+    if (W == 1) __syncwarp();
+    else asm volatile("bar.sync %0, 64;" ::"r"(bar_id) : "memory");
+}
+
+// A pair's exchange of warp-uniform values: lane 0 of every warp writes up to three values into the current slot, the pair syncs,
+// and both warps read both sets (slot[0..2]: warp 0's, slot[4..6]: warp 1's).  Two slots are used in turn: a warp writes a slot again
+// two exchanges later, after the barrier of the exchange in between, which its partner reaches only after reading that slot.
+struct PairXch {
+    uint32_t *x;
+    uint32_t slot;
+    __device__ __forceinline__ const uint32_t *put(uint32_t h, uint32_t lane, uint32_t bar_id, uint32_t a, uint32_t b = 0u, uint32_t c = 0u) {
+        uint32_t *s = x + slot * 8;
+        if (lane == 0) {
+            s[h * 4] = a;
+            s[h * 4 + 1] = b;
+            s[h * 4 + 2] = c;
+        }
+        slot ^= 1u;
+        unit_sync<2>(bar_id);
+        return s;
+    }
+};
+
+// Inclusive scan of v over the unit's 32 * W lanes (warp 1's lanes after warp 0's); *total = the sum over all of them.
+template <int W>
+__device__ __forceinline__ uint32_t unit_incl_scan(uint32_t v, uint32_t lane, uint32_t h, uint32_t bar_id, PairXch &xc, uint32_t *total) {
+    v = warp_incl_scan_u32(v, lane);
+    const uint32_t wt = __shfl_sync(0xffffffffu, v, 31);
+    if (W == 1) {
+        *total = wt;
+        return v;
+    }
+    const uint32_t *s = xc.put(h, lane, bar_id, wt);
+    *total = s[0] + s[4];
+    return v + (h ? s[0] : 0u);
+}
+
+constexpr int G3_WARPS = 5;  // units in flight per CTA of the 512-instance layout (one warp each)
+constexpr int G3_PAIRS = 3;  // units in flight per CTA of the 1024-instance layout (one pair of warps each): 3 CTAs, 18 warps per SM at K <= 32
+// CTAs per SM that a CTA's shared memory allows (227 KB per SM, 1 KB of it reserved per CTA)
+constexpr int g3_ctas_per_sm(size_t smem) {
+    const int n = (int)((size_t)(227 * 1024) / (smem + 1024));
+    return n > 1 ? n : 1;
+}
 constexpr uint32_t G3_SMALL_INST = 512, G3_SMALL_ENT = 128, G3_SMALL_NB = 64;  // what the 512-instance layout holds
 
-template <int PW, int KW, int WCAP, int WARPS, int U>
-__global__ void __launch_bounds__(WARPS * 32)
+// The pair kernel states the CTAs per SM that its shared memory allows, so that ptxas budgets registers for them (and keeps
+// every value in a register); the one-warp kernel leaves the choice to ptxas.
+template <int PW, int KW, int WCAP, int UNITS, int U>
+__global__ void __launch_bounds__(UNITS * UnitLayout<WCAP, KW>::W * 32, WCAP == 1024 ? g3_ctas_per_sm(UNITS * UnitLayout<WCAP, KW>::BYTES) : 0)
     group3_kernel(const uint32_t *__restrict__ skr, const uint64_t *__restrict__ ent, const Unit3 *__restrict__ units, KeyLayout kl, int cutoff,
                   const int32_t *__restrict__ ids_by_arrival, int32_t id_base, G3Stage out, G3Counters *__restrict__ gc,
                   const uint32_t *__restrict__ chunk_bounds, uint32_t chunk, uint32_t *__restrict__ chunk_tickets, uint32_t size_class) {
     // size_class: 0 = every unit; 1 = only the small units (no rounds, at most G3_SMALL_INST instances and G3_SMALL_ENT entries);
-    // 2 = only the others.  Two launches (1024-instance layout for the large units, 512-instance layout — twice the warps per SM —
-    // for the small ones) share the unit list.
+    // 2 = only the others.  Two launches (1024-instance layout for the large units, 512-instance layout for the small ones) share
+    // the unit list.
+    // UNITS units are in flight per CTA.  A unit of the 512-instance layout is worked on by one warp; a unit of the 1024-instance
+    // layout by a PAIR of warps that share its shared memory (h = 0, 1), synchronised by the pair's own named barrier: the unit's
+    // memory fixes how many units an SM holds, not how many warps work on them.  The pair splits every phase: entries and
+    // survivors by ranges of 64, the instance positions in two halves [0, mid) and [mid, n_inst).
+    using WL = UnitLayout<WCAP, KW>;
+    constexpr int W = WL::W;
     constexpr int NW = SkrLayout<PW>::WORDS;
     constexpr int HS = 2 * WCAP;  // hash slots (u16 each)
     constexpr int LOG_HS = WCAP == 512 ? 10 : 11;
     static_assert(WCAP == 512 || WCAP == 1024, "unit capacity");
     static_assert((1 << LOG_HS) == HS, "hash size");
-    using WL = WarpLayout<WCAP, KW>;
     constexpr int NB_MAX = WL::NB_MAX, ECAP = WL::ECAP;
     extern __shared__ __align__(16) uint8_t smem3[];
     const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    uint8_t *wb = smem3 + (size_t)warp * WL::BYTES;
+    const uint32_t h = warp % W, bar_id = 1 + warp / W;  // warp of the unit; named barrier of the pair (0 is __syncthreads')
+    const uint32_t ul = h * 32 + lane;                    // lane inside the unit
+    const bool first = ul == 0;                           // the unit's first lane: takes tickets, reports
+    uint8_t *wb = smem3 + (size_t)(warp / W) * WL::BYTES;
     uint64_t *key0 = reinterpret_cast<uint64_t *>(wb);
     uint64_t *key1 = key0 + (KW == 2 ? WCAP : 0);
     uint16_t *tbl16 = reinterpret_cast<uint16_t *>(key0 + KW * WCAP);  // [2 * WCAP] hash slots: instance index + 1 of the group's leader
     uint32_t *cnt32 = reinterpret_cast<uint32_t *>(tbl16 + 2 * WCAP);  // [WCAP / 2] words = [WCAP] u16: instances per group, later the END of its id list
     uint16_t *cnt16 = reinterpret_cast<uint16_t *>(cnt32);
-    uint16_t *grp = cnt16 + WCAP;                                      // [WCAP] leader (first inserted instance) of every instance's group
-    uint16_t *rk = grp + WCAP;                                         // [WCAP] rank of the instance inside its group, in position order
+    uint32_t *cntlo32 = cnt32 + (W - 1) * WCAP / 2;                    // pair: [WCAP] u16 instances per group in the lower half (the counts
+    uint16_t *cntlo16 = reinterpret_cast<uint16_t *>(cntlo32);         // of warp 0; cnt counts warp 1's, until the survivors pass adds them)
+    uint16_t *grp = cnt16 + W * WCAP;                                  // [WCAP] leader (first inserted instance) of every instance's group
+    uint16_t *rk = grp + WCAP;                                         // [WCAP] rank of the instance inside its group (pair: inside its half)
     uint8_t *eix = reinterpret_cast<uint8_t *>(rk + WCAP);             // [WCAP] entry of the instance (packed units)
     uint16_t *bstart = reinterpret_cast<uint16_t *>(eix + WCAP);       // [NB_MAX + 1] first instance of every bucket of the unit
     uint32_t *bmm = reinterpret_cast<uint32_t *>(reinterpret_cast<uint8_t *>(bstart) + WL::BSTART_BYTES);  // [NB_MAX] its m-mer code
     int32_t *eid = reinterpret_cast<int32_t *>(bmm + NB_MAX);          // [ECAP] read id of every entry
     uint8_t *ebk = reinterpret_cast<uint8_t *>(eid + ECAP);            // [ECAP] bucket ordinal of every entry
+    PairXch xc{reinterpret_cast<uint32_t *>(ebk + ECAP), 0u};          // pair: exchange words
     // after the grouping the hash table is dead: its memory holds the survivor lists, then the unit's ids
     uint16_t *surv = tbl16;                               // [WCAP] instance index of every surviving leader, ascending
-    uint16_t *sorted = surv + WCAP;                       // [WCAP] the same in table order
+    uint16_t *sorted = surv + WCAP;                       // [WCAP] the same in table order (pair: first warp 1's survivors, see below)
     int32_t *idbuf = reinterpret_cast<int32_t *>(tbl16);  // [WCAP] the unit's ids in output order
 
     const int K = kl.K;
@@ -504,10 +566,15 @@ __global__ void __launch_bounds__(WARPS * 32)
     const uint32_t unit_begin = chunk_bounds[chunk], unit_end = chunk_bounds[chunk + 1];
     const uint32_t lt_mask = (1u << lane) - 1u;
     const uint32_t cls_mask = (uint32_t)(kl.nc - 1);
+    // the ticket taken by the unit's first lane, to every lane of the unit (pair: the exchange's barrier also ends the unit)
+    auto share_ticket = [&](uint32_t t) -> uint32_t {
+        if (W == 1) return __shfl_sync(0xffffffffu, t, 0);
+        return xc.put(h, lane, bar_id, __shfl_sync(0xffffffffu, t, 0))[0];
+    };
 
     uint32_t u = 0;
-    if (lane == 0) u = unit_begin + atomicAdd(&chunk_tickets[chunk], 1u);
-    u = __shfl_sync(0xffffffffu, u, 0);
+    if (first) u = unit_begin + atomicAdd(&chunk_tickets[chunk], 1u);
+    u = share_ticket(u);
     while (u < unit_end) {
         Unit3 un;
         {
@@ -522,7 +589,7 @@ __global__ void __launch_bounds__(WARPS * 32)
         }
         // the next ticket is taken now and read at the end of the unit (units do not depend on each other)
         uint32_t u_next = 0;
-        if (lane == 0) u_next = unit_begin + atomicAdd(&chunk_tickets[chunk], 1u);
+        if (first) u_next = unit_begin + atomicAdd(&chunk_tickets[chunk], 1u);
         const uint32_t u_cur = u;
         const bool is_round = un.rounds != 0;
         const uint32_t n_ent = un.ent_end - un.ent_begin;
@@ -532,22 +599,22 @@ __global__ void __launch_bounds__(WARPS * 32)
         if (size_class) {
             const bool small = !is_round && un.n_inst <= G3_SMALL_INST && n_ent <= G3_SMALL_ENT;
             if (small != (size_class == 1u)) {  // the other launch's unit
-                u = __shfl_sync(0xffffffffu, u_next, 0);
+                u = share_ticket(u_next);
                 continue;
             }
         }
         if (is_round && un.n_inst == 0) {  // a round the cut did not need
-            if (lane == 0) out.unit_out[u_cur] = UnitOut3{un.ibase, 0u, 0u, 0u};
-            u = __shfl_sync(0xffffffffu, u_next, 0);
+            if (first) out.unit_out[u_cur] = UnitOut3{un.ibase, 0u, 0u, 0u};
+            u = share_ticket(u_next);
             continue;
         }
 
         // ---- zero the hash table and the counters (contiguous)
         {
             uint4 *z = reinterpret_cast<uint4 *>(tbl16);
-            for (uint32_t i = lane; i < (uint32_t)(WCAP * 4 + WCAP * 2) / 16; i += 32) z[i] = make_uint4(0u, 0u, 0u, 0u);
+            for (uint32_t i = ul; i < (uint32_t)(WCAP * 4 + W * WCAP * 2) / 16; i += 32 * W) z[i] = make_uint4(0u, 0u, 0u, 0u);
         }
-        __syncwarp();
+        unit_sync<W>(bar_id);
 
         // ---- round units: the planner cut the atom's instances by ranges of d; mine is [dlo, dhi]
         int dlo = 0, dhi = 63;
@@ -562,8 +629,8 @@ __global__ void __launch_bounds__(WARPS * 32)
         uint32_t n_inst = 0, n_bkt = 0;
         if (!bad) {
             uint32_t carry_pos = 0, carry_ord = 0, prev_mm = 0xffffffffu;
-            for (uint32_t e0 = 0; e0 < n_ent; e0 += 32) {
-                const uint32_t e = e0 + lane;
+            for (uint32_t e0 = 0; e0 < n_ent; e0 += 32 * W) {
+                const uint32_t e = e0 + ul;
                 uint32_t np = 0, t0 = 0, mm = 0xffffffffu, arrival = 0;
                 bool rev = false;
                 uint4 ha = make_uint4(0u, 0u, 0u, 0u), pa = ha, pb = ha;
@@ -593,19 +660,32 @@ __global__ void __launch_bounds__(WARPS * 32)
                 }
                 // buckets (runs of equal m-mer code) of the unit and instance positions
                 uint32_t pm = __shfl_up_sync(0xffffffffu, mm, 1);
-                if (lane == 0) pm = prev_mm;
+                if (lane == 0) {
+                    if (W == 1) pm = prev_mm;
+                    else pm = (e == 0 || e >= n_ent) ? 0xffffffffu : (uint32_t)(ent[un.ent_begin + e - 1] >> 32) >> kl.mshift;  // the entry before
+                }
                 const bool head = e < n_ent && mm != pm;
-                const uint32_t hs = warp_incl_scan_u32(head ? 1u : 0u, lane);
-                const uint32_t ps = warp_incl_scan_u32(np, lane);
+                uint32_t hs = warp_incl_scan_u32(head ? 1u : 0u, lane);
+                uint32_t ps = warp_incl_scan_u32(np, lane);
+                uint32_t hs_all = __shfl_sync(0xffffffffu, hs, 31), ps_all = __shfl_sync(0xffffffffu, ps, 31);
+                if (W == 2) {  // 64-wide scans: warp 1's lanes follow warp 0's
+                    const uint32_t *s = xc.put(h, lane, bar_id, hs_all, ps_all);
+                    if (h) {
+                        hs += s[0];
+                        ps += s[1];
+                    }
+                    hs_all = s[0] + s[4];
+                    ps_all = s[1] + s[5];
+                }
                 const uint32_t ord = carry_ord + hs - 1;  // bucket ordinal of this entry
                 const uint32_t pos0 = carry_pos + ps - np;
                 if (head && ord < (uint32_t)NB_MAX) {
                     bstart[ord] = (uint16_t)pos0;
                     bmm[ord] = mm;
                 }
-                carry_ord += __shfl_sync(0xffffffffu, hs, 31);
-                carry_pos += __shfl_sync(0xffffffffu, ps, 31);
-                prev_mm = __shfl_sync(0xffffffffu, mm, 31);
+                carry_ord += hs_all;
+                carry_pos += ps_all;
+                if (W == 1) prev_mm = __shfl_sync(0xffffffffu, mm, 31);
                 if (carry_pos > (uint32_t)WCAP || carry_ord > (uint32_t)NB_MAX || (!packed && carry_ord > 1u)) {  // cannot happen with the planner's bounds
                     bad = true;
                     break;
@@ -630,29 +710,38 @@ __global__ void __launch_bounds__(WARPS * 32)
             }
             n_inst = carry_pos;
             n_bkt = carry_ord;
-            if (!bad && lane == 0) bstart[n_bkt] = (uint16_t)n_inst;
+            if (!bad && first) bstart[n_bkt] = (uint16_t)n_inst;
         }
-        __syncwarp();
+        unit_sync<W>(bar_id);
         if (bad) {  // give up on this unit: the batch is redone by another pipeline
-            if (lane == 0) {
+            if (first) {
                 atomicExch(&gc->overflow, 1u);
                 out.unit_out[u_cur] = UnitOut3{ibase, 0u, 0u, 0u};
             }
-            u = __shfl_sync(0xffffffffu, u_next, 0);
+            u = share_ticket(u_next);
             continue;
         }
+        // my instance positions: [pbeg, pend).  Pair: warp 0 the lower half [0, mid), warp 1 the upper half [mid, n_inst).
+        const uint32_t mid = W == 1 ? n_inst : min(n_inst, (n_inst + 63) / 64 * 32);
+        const uint32_t pbeg = h ? mid : 0u, pend = h ? n_inst : mid;
 
         // ---- group: claim a slot with the instance index, compare keys through the instance arrays.  U instances per lane are in
         // flight together.  The rank of an instance inside its group follows position order: 32 positions per step, the peers of a
-        // step are ranked by lane, the steps by the order in which their counter updates are issued.
-        for (uint32_t b0 = 0; b0 < n_inst; b0 += 32 * U) {
+        // step are ranked by lane, the steps by the order in which their counter updates are issued.  A pair inserts into the same
+        // table (the 16-bit CAS works across warps), but each warp counts its own half into its own counters (warp 0: cnt_lo,
+        // warp 1: cnt), so the rank above is the rank inside the half.  Every position of the lower half precedes every position
+        // of the upper half, so an instance's rank in position order = its rank inside its half, plus, in the upper half, the
+        // group's count in the lower half (cnt_lo[leader], complete after the pair's barrier; the id pass adds it).  The result
+        // does not depend on the timing of the two warps' atomics.
+        uint32_t *cntw32 = (W == 2 && h == 0) ? cntlo32 : cnt32;
+        for (uint32_t b0 = pbeg; b0 < pend; b0 += 32 * U) {
             uint64_t k0[U], k1[U];
             uint32_t lo[U], hi[U], idx[U], rep[U], cur[U];
             bool valid[U];
 #pragma unroll
             for (int j = 0; j < U; j++) {
                 const uint32_t p = b0 + j * 32 + lane;
-                valid[j] = p < n_inst;
+                valid[j] = p < pend;
                 k0[j] = valid[j] ? key0[p] : 0ull;
                 k1[j] = (KW == 2 && valid[j]) ? key1[p] : 0ull;
                 uint32_t o = 0;
@@ -716,7 +805,7 @@ __global__ void __launch_bounds__(WARPS * 32)
                 c[j] = 0;
                 if (valid[j] && (int)lane == __ffs(peers[j]) - 1) {
                     const uint32_t sh = 16u * (rep[j] & 1u);
-                    c[j] = (atomicAdd(&cnt32[rep[j] >> 1], (uint32_t)__popc(peers[j]) << sh) >> sh) & 0xffffu;
+                    c[j] = (atomicAdd(&cntw32[rep[j] >> 1], (uint32_t)__popc(peers[j]) << sh) >> sh) & 0xffffu;
                 }
                 __syncwarp();  // the updates of step j must be issued before those of step j + 1 (diverged lanes could run ahead)
             }
@@ -730,27 +819,31 @@ __global__ void __launch_bounds__(WARPS * 32)
                 }
             }
         }
-        __syncwarp();
+        unit_sync<W>(bar_id);
 
-        // ---- leaders and survivors (keep iff count > cutoff, binning.c:1102); survivors are listed by ascending position
+        // ---- leaders and survivors (keep iff count > cutoff, binning.c:1102); survivors are listed by ascending position.  Pair: a
+        // group's count = cnt_lo + cnt, stored into cnt; warp 1 lists its survivors in `sorted` first and moves them behind warp 0's.
         uint32_t S = 0, N = 0, D = 0;
-        for (uint32_t b0 = 0; b0 < n_inst; b0 += 32 * U) {
+        uint16_t *my_surv = h ? sorted : surv;
+        for (uint32_t b0 = pbeg; b0 < pend; b0 += 32 * U) {
             bool leader[U];
             uint32_t c[U];
 #pragma unroll
             for (int j = 0; j < U; j++) {
                 const uint32_t p = b0 + j * 32 + lane;
-                leader[j] = p < n_inst && grp[p] == p;
+                leader[j] = p < pend && grp[p] == p;
             }
 #pragma unroll
-            for (int j = 0; j < U; j++) c[j] = leader[j] ? cnt16[b0 + j * 32 + lane] : 0u;
+            for (int j = 0; j < U; j++) c[j] = leader[j] ? cnt16[b0 + j * 32 + lane] + (W == 2 ? cntlo16[b0 + j * 32 + lane] : 0u) : 0u;
 #pragma unroll
             for (int j = 0; j < U; j++) {
                 const uint32_t p = b0 + j * 32 + lane;
                 const bool sv = leader[j] && (cutoff < 0 || c[j] > (uint32_t)cutoff);
                 const unsigned lm = __ballot_sync(0xffffffffu, leader[j]), sm = __ballot_sync(0xffffffffu, sv);
-                if (sv) surv[S + __popc(sm & lt_mask)] = (uint16_t)p;
-                else if (leader[j]) cnt16[p] = 0xffffu;  // pruned
+                if (sv) {
+                    my_surv[S + __popc(sm & lt_mask)] = (uint16_t)p;
+                    if (W == 2) cnt16[p] = (uint16_t)c[j];
+                } else if (leader[j]) cnt16[p] = 0xffffu;  // pruned
                 S += __popc(sm);
                 D += __popc(lm);
                 N += sv ? c[j] : 0u;
@@ -758,22 +851,34 @@ __global__ void __launch_bounds__(WARPS * 32)
         }
 #pragma unroll
         for (int d = 16; d > 0; d >>= 1) N += __shfl_xor_sync(0xffffffffu, N, d);
+        uint32_t S_lo = S;  // survivors of the lower half
+        if (W == 2) {
+            const uint32_t *s = xc.put(h, lane, bar_id, S, N, D);
+            S_lo = s[0];
+            S = s[0] + s[4];
+            N = s[1] + s[5];
+            D = s[2] + s[6];
+        }
         const uint64_t kbase = ibase / out.kdiv;
         const bool oob = (uint64_t)ibase + N > out.id_cap || kbase + S > out.kmer_cap;  // cannot happen with the caller's bounds; never write out of range
-        if (lane == 0) {
+        if (first) {
             out.unit_out[u_cur] = UnitOut3{ibase, oob ? 0u : S, oob ? 0u : N, 0u};
             atomicAdd(&gc->distinct, (unsigned long long)D);
             if (oob) atomicExch(&gc->overflow, 2u);
         }
-        __syncwarp();
         if (oob) {
-            u = __shfl_sync(0xffffffffu, u_next, 0);
+            u = share_ticket(u_next);
             continue;
         }
+        if (W == 2 && h) {
+            __syncwarp();
+            for (uint32_t x = lane; x < S - S_lo; x += 32) surv[S_lo + x] = sorted[x];
+        }
+        unit_sync<W>(bar_id);
 
         // ---- table order: buckets ascend with position already; inside a bucket every survivor counts the smaller keys
-        for (uint32_t x0 = 0; x0 < S; x0 += 32) {
-            const uint32_t x = x0 + lane;
+        for (uint32_t x0 = 0; x0 < S; x0 += 32 * W) {
+            const uint32_t x = x0 + ul;
             if (x < S) {
                 const uint32_t p = surv[x];
                 uint32_t a = 0, a2 = S;
@@ -806,25 +911,26 @@ __global__ void __launch_bounds__(WARPS * 32)
                 sorted[rank] = (uint16_t)p;
             }
         }
-        __syncwarp();
+        unit_sync<W>(bar_id);
 
         // ---- list offsets in table order: cnt[leader] becomes the END of its list inside the unit
         {
             uint32_t carry = 0;
-            for (uint32_t x0 = 0; x0 < S; x0 += 32) {
-                const uint32_t x = x0 + lane;
+            for (uint32_t x0 = 0; x0 < S; x0 += 32 * W) {
+                const uint32_t x = x0 + ul;
                 const uint32_t p = x < S ? sorted[x] : 0u;
                 const uint32_t c = x < S ? cnt16[p] : 0u;
-                const uint32_t inc = warp_incl_scan_u32(c, lane);
+                uint32_t all;
+                const uint32_t inc = unit_incl_scan<W>(c, lane, h, bar_id, xc, &all);
                 if (x < S) cnt16[p] = (uint16_t)(carry + inc);
-                carry += __shfl_sync(0xffffffffu, inc, 31);
+                carry += all;
             }
         }
-        __syncwarp();
+        unit_sync<W>(bar_id);
 
         // ---- k-mers in table order, staged
-        for (uint32_t x0 = 0; x0 < S; x0 += 32) {
-            const uint32_t x = x0 + lane;
+        for (uint32_t x0 = 0; x0 < S; x0 += 32 * W) {
+            const uint32_t x = x0 + ul;
             if (x < S) {
                 const uint32_t p = sorted[x];
                 const uint32_t beg = x ? cnt16[sorted[x - 1]] : 0u;
@@ -835,13 +941,13 @@ __global__ void __launch_bounds__(WARPS * 32)
                 out.loff[g] = beg;
             }
         }
-        __syncwarp();  // surv / sorted are dead from here on: the table's memory becomes the id buffer
+        unit_sync<W>(bar_id);  // surv / sorted are dead from here on: the table's memory becomes the id buffer
 
         // ---- ids, newest first (binning.c:1059-1069): an instance's place = end of its list - 1 - its rank.  The unit's ids are
         // collected in shared memory and leave as one coalesced run.
         if (N) {
             if (packed) {
-                for (uint32_t b0 = 0; b0 < n_inst; b0 += 32 * U) {
+                for (uint32_t b0 = pbeg; b0 < pend; b0 += 32 * U) {
                     uint32_t end[U], r[U];
                     int32_t id[U];
 #pragma unroll
@@ -850,9 +956,10 @@ __global__ void __launch_bounds__(WARPS * 32)
                         end[j] = 0xffffu;
                         r[j] = 0;
                         id[j] = 0;
-                        if (p < n_inst) {
-                            end[j] = cnt16[grp[p]];
-                            r[j] = rk[p];
+                        if (p < pend) {
+                            const uint32_t g = grp[p];
+                            end[j] = cnt16[g];
+                            r[j] = rk[p] + (W == 2 && h ? cntlo16[g] : 0u);
                             id[j] = eid[eix[p]];
                         }
                     }
@@ -862,8 +969,8 @@ __global__ void __launch_bounds__(WARPS * 32)
                 }
             } else {  // lane = entry (the read id belongs to the record)
                 uint32_t carry_pos = 0;
-                for (uint32_t e0 = 0; e0 < n_ent; e0 += 32) {
-                    const uint32_t e = e0 + lane;
+                for (uint32_t e0 = 0; e0 < n_ent; e0 += 32 * W) {
+                    const uint32_t e = e0 + ul;
                     uint32_t np = 0, arrival = 0;
                     if (e < n_ent) {
                         const uint32_t slot = (uint32_t)ent[un.ent_begin + e];
@@ -880,25 +987,27 @@ __global__ void __launch_bounds__(WARPS * 32)
                             np = (dlo > dhi || b < a) ? 0u : (uint32_t)(b - a + 1);
                         }
                     }
-                    const uint32_t ps = warp_incl_scan_u32(np, lane);
+                    uint32_t all;
+                    const uint32_t ps = unit_incl_scan<W>(np, lane, h, bar_id, xc, &all);
                     const uint32_t pos0 = carry_pos + ps - np;
-                    carry_pos += __shfl_sync(0xffffffffu, ps, 31);
+                    carry_pos += all;
                     if (np) {
                         const int32_t id = ids_by_arrival ? ids_by_arrival[arrival] : id_base + (int32_t)arrival;
                         for (uint32_t i = 0; i < np; i++) {
                             const uint32_t p = pos0 + i;
-                            const uint32_t end = cnt16[grp[p]];
-                            if (end != 0xffffu) idbuf[end - 1u - rk[p]] = id;
+                            const uint32_t g = grp[p];
+                            const uint32_t end = cnt16[g];
+                            if (end != 0xffffu) idbuf[end - 1u - rk[p] - (W == 2 && p >= mid ? cntlo16[g] : 0u)] = id;
                         }
                     }
                 }
             }
-            __syncwarp();
+            unit_sync<W>(bar_id);
             int32_t *dst = out.ids + ibase;
-            for (uint32_t i = lane; i < N; i += 32) dst[i] = idbuf[i];
+            for (uint32_t i = ul; i < N; i += 32 * W) dst[i] = idbuf[i];
         }
-        __syncwarp();
-        u = __shfl_sync(0xffffffffu, u_next, 0);
+        if (W == 1) __syncwarp();
+        u = share_ticket(u_next);
     }
 }
 
@@ -1175,7 +1284,7 @@ __global__ void v3_chunk_bounds_kernel(const Unit3 *__restrict__ units, const G3
 static bool v3_hybrid(const KeyLayout &kl, int cap_i) { return cap_i != 512 && kl.K <= 32; }
 static Plan3 v3_plan_params(const KeyLayout &kl, int cap_i) {
     const uint32_t cap = cap_i == 512 ? 512u : 1024u;
-    Plan3 pp{cap, cap / 8, cap / 4, (uint32_t)(kl.K - kl.M + 1), cap, cap / 8, cap / 4};  // NB_MAX and ECAP of WarpLayout
+    Plan3 pp{cap, cap / 8, cap / 4, (uint32_t)(kl.K - kl.M + 1), cap, cap / 8, cap / 4};  // NB_MAX and ECAP of UnitLayout
     if (v3_hybrid(kl, cap_i)) {
         pp.cap_s = G3_SMALL_INST;
         pp.nb_s = G3_SMALL_NB;
@@ -1221,18 +1330,22 @@ int v3_plan_units(const uint16_t *sorted_info, const uint64_t *ent, const KeyLay
     return l + 1;
 }
 
+// units in flight per CTA of the grouping kernel at capacity cap, and the CTA's threads (UnitLayout::W warps per unit)
+static int v3_group_units(int cap) { return cap == 512 ? G3_WARPS : G3_PAIRS; }
+static int v3_group_threads(int cap) { return v3_group_units(cap) * (cap == 512 ? UnitLayout<512, 1>::W : UnitLayout<1024, 1>::W) * 32; }
+
 size_t v3_group_smem_bytes(int KW, int cap) {
-    const size_t per_warp = cap == 512 ? (KW == 1 ? WarpLayout<512, 1>::BYTES : WarpLayout<512, 2>::BYTES)
-                                       : (KW == 1 ? WarpLayout<1024, 1>::BYTES : WarpLayout<1024, 2>::BYTES);
-    return per_warp * G3_WARPS;
+    const size_t per_unit = cap == 512 ? (KW == 1 ? UnitLayout<512, 1>::BYTES : UnitLayout<512, 2>::BYTES)
+                                       : (KW == 1 ? UnitLayout<1024, 1>::BYTES : UnitLayout<1024, 2>::BYTES);
+    return per_unit * v3_group_units(cap);
 }
 
 int v3_group_launch(const void *skr, const uint64_t *ent, const void *units, const KeyLayout &kl, int cap, int cutoff, const int32_t *ids_by_arrival, int32_t id_base,
                     const V3Out &o, uint64_t max_units, uint64_t *unit_excl, uint64_t *lsd_excl, void *scan_scratch, void *gc_dev, const V3Chunks &ch, const V3Lsd &lsd,
                     bool finalize_only, int sm_count, KernelProf *prof, cudaStream_t st) {
     const int KW = kl.K <= 32 ? 1 : 2;
-    constexpr int WARPS = G3_WARPS;
     const size_t smem = v3_group_smem_bytes(KW, cap);
+    const int threads = v3_group_threads(cap), threads_s = v3_group_threads(512);
     cudaMemsetAsync(ch.tickets, 0, sizeof(uint32_t) * 2 * ch.n, st);
     const uint32_t kdiv = cutoff >= 0 ? (uint32_t)cutoff + 1u : 1u;
     G3Stage stg{o.stg_codes, o.stg_mmer, o.stg_loff, o.stg_ids, static_cast<UnitOut3 *>(o.unit_out), o.kmer_cap, o.id_cap, kdiv};
@@ -1241,12 +1354,10 @@ int v3_group_launch(const void *skr, const uint64_t *ent, const void *units, con
     G3Counters *gc = static_cast<G3Counters *>(gc_dev);
     const uint32_t *sk = static_cast<const uint32_t *>(skr);
     const Unit3 *un = static_cast<const Unit3 *>(units);
-    int per_sm = (int)((size_t)(227 * 1024) / (smem + 1024));
-    if (per_sm < 1) per_sm = 1;
+    const int per_sm = g3_ctas_per_sm(smem);
     const bool hybrid = v3_hybrid(kl, cap);
     const size_t smem_s = v3_group_smem_bytes(KW, 512);
-    int per_sm_s = (int)((size_t)(227 * 1024) / (smem_s + 1024));
-    if (per_sm_s < 1) per_sm_s = 1;
+    const int per_sm_s = g3_ctas_per_sm(smem_s);
     int launches = 0;
     auto launch = [&](auto kern, auto kern_small, auto fin_kern) {
         cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -1255,14 +1366,15 @@ int v3_group_launch(const void *skr, const uint64_t *ent, const void *units, con
             if (!finalize_only) {
                 bool on = prof && prof->begin(KK_SKR_GROUP, st);
                 if (!hybrid) {
-                    kern<<<sm_count * per_sm, WARPS * 32, smem, st>>>(sk, ent, un, kl, cutoff, ids_by_arrival, id_base, stg, gc, ch.bounds, c, ch.tickets, 0u);
+                    kern<<<sm_count * per_sm, threads, smem, st>>>(sk, ent, un, kl, cutoff, ids_by_arrival, id_base, stg, gc, ch.bounds, c, ch.tickets, 0u);
                 } else {
-                    // side by side: the large-unit kernel goes first at 2 CTAs per SM, the small-unit kernel's CTAs take what is left of
-                    // every SM and, being persistent, the room the other kernel leaves when it runs out of units (its tail is covered)
+                    // side by side: the large-unit kernel goes first with as many CTAs as its shared memory lets an SM hold, the
+                    // small-unit kernel's CTAs take what is left of every SM and, being persistent, the room the other kernel leaves when
+                    // it runs out of units (its tail is covered)
                     cudaEventRecord(ch.ev_fork, st);
                     cudaStreamWaitEvent(ch.aux, ch.ev_fork, 0);
-                    kern<<<sm_count * 2, WARPS * 32, smem, st>>>(sk, ent, un, kl, cutoff, ids_by_arrival, id_base, stg, gc, ch.bounds, c, ch.tickets, 2u);
-                    kern_small<<<sm_count * per_sm_s, WARPS * 32, smem_s, ch.aux>>>(sk, ent, un, kl, cutoff, ids_by_arrival, id_base, stg, gc, ch.bounds, c, ch.tickets + ch.n, 1u);
+                    kern<<<sm_count * per_sm, threads, smem, st>>>(sk, ent, un, kl, cutoff, ids_by_arrival, id_base, stg, gc, ch.bounds, c, ch.tickets, 2u);
+                    kern_small<<<sm_count * per_sm_s, threads_s, smem_s, ch.aux>>>(sk, ent, un, kl, cutoff, ids_by_arrival, id_base, stg, gc, ch.bounds, c, ch.tickets + ch.n, 1u);
                     cudaEventRecord(ch.ev_join, ch.aux);
                     cudaStreamWaitEvent(st, ch.ev_join, 0);
                 }
@@ -1286,12 +1398,13 @@ int v3_group_launch(const void *skr, const uint64_t *ent, const void *units, con
         }
     };
     // instances per lane in flight: 4 at capacity 1024, 2 at 512 (more warps per SM there: less need for instruction-level parallelism, smaller code)
+    constexpr int W5 = G3_WARPS, P3 = G3_PAIRS;
     if (KW == 1) {
-        if (cap == 512) launch(group3_kernel<2, 1, 512, WARPS, 2>, group3_kernel<2, 1, 512, WARPS, 2>, finalize3_kernel<1>);
-        else launch(group3_kernel<2, 1, 1024, WARPS, 4>, group3_kernel<2, 1, 512, WARPS, 2>, finalize3_kernel<1>);
+        if (cap == 512) launch(group3_kernel<2, 1, 512, W5, 2>, group3_kernel<2, 1, 512, W5, 2>, finalize3_kernel<1>);
+        else launch(group3_kernel<2, 1, 1024, P3, 4>, group3_kernel<2, 1, 512, W5, 2>, finalize3_kernel<1>);
     } else {
-        if (cap == 512) launch(group3_kernel<4, 2, 512, WARPS, 2>, group3_kernel<4, 2, 512, WARPS, 2>, finalize3_kernel<2>);
-        else launch(group3_kernel<4, 2, 1024, WARPS, 4>, group3_kernel<4, 2, 512, WARPS, 2>, finalize3_kernel<2>);
+        if (cap == 512) launch(group3_kernel<4, 2, 512, W5, 2>, group3_kernel<4, 2, 512, W5, 2>, finalize3_kernel<2>);
+        else launch(group3_kernel<4, 2, 1024, P3, 4>, group3_kernel<4, 2, 512, W5, 2>, finalize3_kernel<2>);
     }
     return launches;
 }

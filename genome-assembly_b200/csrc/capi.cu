@@ -644,7 +644,8 @@ int run_v2_group(gbin_ctx *ctx, void *skr, void *twin, uint64_t n_skr, const int
     return GBIN_OK;
 }
 
-// ---- pipeline 3: entries sorted by reference, one warp per unit, staging + finalize (bin3.cu)
+// ---- pipeline 3: entries sorted by reference, one warp (512-instance units) or one pair of warps (1024-instance units) per unit,
+// staging + finalize (bin3.cu)
 // The records in `skr` are read, not moved.  *done = false when the batch does not fit (a (bucket, d) class larger than a unit);
 // it then goes through pipeline 2, which sorts the records themselves.
 

@@ -142,7 +142,7 @@ int skr_group_launch(const void *skr_sorted, int K, int cutoff, const uint32_t *
 int skr_emit_buckets(const uint32_t *kmer_mmer, uint64_t n_kmers, uint64_t n_ids, uint32_t *bucket_excl, uint32_t *scratch,
                      uint32_t *mmer_codes, uint64_t *mmer_kmer_off, uint64_t *kmer_id_off, uint32_t *n_buckets_dev, cudaStream_t st);
 
-// ---- bin3.cu (pipeline v3: sort by reference, one warp per unit, table written once at its final place)
+// ---- bin3.cu (pipeline v3: sort by reference, one warp or one pair of warps per unit, table written once at its final place)
 // slot_info (per slot) is gathered into sorted_info (per sorted entry) by the last pass
 int radix_sort_entries(void *a, void *b, uint64_t n, int key_bits, void *scratch, bool *result_in_b, int *passes_out, const uint16_t *slot_info,
                        uint16_t *sorted_info, KernelProf *prof, cudaStream_t st, const unsigned long long *n_real_dev = nullptr);
