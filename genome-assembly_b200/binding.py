@@ -70,7 +70,8 @@ EXPORTS = [
     "gbin_strerror", "gbin_last_error", "gbin_version", "gbin_create", "gbin_destroy", "gbin_get_config",
     "gbin_bin_reads_host", "gbin_table_clone", "gbin_table_free", "gbin_pinned_alloc", "gbin_pinned_free",
     "gbin_bin_reads_device", "gbin_table_to_host", "gbin_table_to_pinned", "gbin_get_timings", "gbin_record_bytes",
-    "gbin_set_kernel_profiling", "gbin_get_kernel_profile", "gbin_kernel_kind_name", "gbin_max_read_len", "gbin_multi_create", "gbin_multi_destroy", "gbin_multi_devices", "gbin_multi_context", "gbin_multi_last_error", "gbin_multi_bin_reads_host", "gbin_table_digest", "gbin_set_pipeline", "gbin_set_tuning", "gbin_donate_scratch", "gbin_get_pipeline_info", "gbin_get_run_stats",
+    "gbin_set_kernel_profiling", "gbin_get_kernel_profile", "gbin_kernel_kind_name", "gbin_max_read_len", "gbin_multi_create", "gbin_multi_destroy", "gbin_multi_devices", "gbin_multi_context", "gbin_multi_last_error", "gbin_multi_bin_reads_host",
+    "gbin_bin_reads_host_part", "gbin_bin_reads_device_part", "gbin_plan_parts", "gbin_table_digest", "gbin_set_pipeline", "gbin_set_tuning", "gbin_donate_scratch", "gbin_get_pipeline_info", "gbin_get_run_stats",
     "gbin_count_instances_device", "gbin_scan_reads_device", "gbin_partition_records_device",
     "gbin_group_records_device", "gbin_owner_of", "gbin_xchg_create", "gbin_xchg_attach", "gbin_xchg_exchange_skr", "gbin_xchg_detach", "gbin_xchg_destroy", "gbin_skr_record_bytes", "gbin_scan_skr_device", "gbin_partition_skr_device", "gbin_group_skr_device",
     "gbin_split_reads_device", "gbin_copy_to_host", "gbin_bin_file_host", "gbin_read_file_fgets", "gbin_table_dump", "gbin_table_dump_reference_format", "gbin_table_dump_expanded_format",
@@ -102,6 +103,9 @@ def load_library() -> C.CDLL:
     L.gbin_get_config.argtypes = [vp, C.POINTER(Config)]
     L.gbin_bin_reads_host.argtypes = [vp, C.POINTER(CReads), C.POINTER(CTable)]
     L.gbin_bin_reads_device.argtypes = [vp, C.POINTER(CReads), vp, C.POINTER(CTable)]
+    L.gbin_bin_reads_host_part.argtypes = [vp, C.POINTER(CReads), u32, u32, C.POINTER(CTable)]
+    L.gbin_bin_reads_device_part.argtypes = [vp, C.POINTER(CReads), u32, u32, vp, C.POINTER(CTable)]
+    L.gbin_plan_parts.argtypes = [vp, u64, C.POINTER(u32)]
     L.gbin_table_to_host.argtypes = [vp, C.POINTER(CTable), C.POINTER(CTable)]
     L.gbin_table_to_pinned.argtypes = [vp, C.POINTER(CTable), vp, C.POINTER(CTable)]
     L.gbin_table_clone.argtypes = [C.POINTER(CTable), C.POINTER(CTable)]
@@ -357,7 +361,9 @@ class Binner:
         self._check(self.lib.gbin_bin_reads_host(self.h, C.byref(reads), C.byref(t)))
         return t
 
-    def bin_host(self, data, n_reads, *, stride=0, read_len=0, starts=None, lens=None, read_ids=None, id_base=0) -> HostTable:
+    @staticmethod
+    def _host_reads(data, n_reads, stride, read_len, starts, lens, read_ids, id_base):
+        """-> (CReads over numpy copies of the arguments, the arrays it points into: keep them alive for the call)."""
         if isinstance(data, (bytes, bytearray)):
             data = np.frombuffer(data, dtype=np.uint8)
         data = np.ascontiguousarray(data, dtype=np.uint8)
@@ -369,8 +375,35 @@ class Binner:
         if read_ids is not None:
             read_ids = np.ascontiguousarray(read_ids, dtype=np.int32)
             keep.append(read_ids)
-        rd = self._reads(data, data.size, n_reads, stride, read_len, starts, lens, read_ids, id_base)
+        return Binner._reads(data, data.size, n_reads, stride, read_len, starts, lens, read_ids, id_base), keep
+
+    def bin_host(self, data, n_reads, *, stride=0, read_len=0, starts=None, lens=None, read_ids=None, id_base=0) -> HostTable:
+        rd, _keep = self._host_reads(data, n_reads, stride, read_len, starts, lens, read_ids, id_base)
         return host_table_from_c(self.bin_host_raw(rd))
+
+    # ---- read sets larger than one device: part `part` of `n_parts` owner parts of the table per call
+    def bin_host_part_raw(self, reads: CReads, part: int, n_parts: int) -> CTable:
+        """gbin_bin_reads_host_part: the ctx-owned pinned table of the part (valid until the next call) without copying it."""
+        t = CTable()
+        self._check(self.lib.gbin_bin_reads_host_part(self.h, C.byref(reads), part, n_parts, C.byref(t)))
+        return t
+
+    def bin_host_part(self, data, n_reads, part: int, n_parts: int, *, stride=0, read_len=0, starts=None, lens=None, read_ids=None,
+                      id_base=0) -> HostTable:
+        rd, _keep = self._host_reads(data, n_reads, stride, read_len, starts, lens, read_ids, id_base)
+        return host_table_from_c(self.bin_host_part_raw(rd, part, n_parts))
+
+    def bin_device_part_raw(self, reads: CReads, part: int, n_parts: int, stream: int | None = None) -> CTable:
+        """gbin_bin_reads_device_part: reads in device memory, the part's table in the context's device memory."""
+        t = CTable()
+        self._check(self.lib.gbin_bin_reads_device_part(self.h, C.byref(reads), part, n_parts, stream, C.byref(t)))
+        return t
+
+    def plan_parts(self, n_instances: int) -> int:
+        """gbin_plan_parts: the smallest number of parts whose one part fits the device's free memory now."""
+        p = C.c_uint32()
+        self._check(self.lib.gbin_plan_parts(self.h, int(n_instances), C.byref(p)))
+        return int(p.value)
 
     # ---- device buffers in, device table out
     def bin_device_raw(self, reads: CReads, stream: int | None = None) -> CTable:

@@ -125,6 +125,9 @@ struct Misc {
     uint32_t split_n_nl, split_n_reads;
     char last_byte;                     // of the file image
     unsigned long long digest;
+    // one owner part per call: records and k-mer instances selected so far, and the select kernel's ticket
+    unsigned long long part_sel[2];
+    uint32_t part_ticket;
 };
 
 // Host path only.  HostFeed: the reads are still in host memory; the scan stage copies them chunk by chunk on the copy
@@ -205,6 +208,10 @@ struct gbin_ctx {
     // pinned host arena for results of the host path + small readbacks
     HostBuf h_misc, h_result, h_kmer_codes, h_kmer_id_off, h_read_ids, h_file;
     DevBuf split_nl, split_tiles_buf, split_base;  // device-side fgets splitting
+    // one owner part per call: two read chunks (bytes; rebased starts + lens) of the host form, the part's records, the select's tiles
+    DevBuf part_data[2], part_meta[2], part_rec, part_state;
+    uint64_t part_chunk_bytes = 1ull << 30;  // gbin_set_tuning "part_chunk_kb"
+    cudaEvent_t ev_part_h2d[4];              // [2 * slot + 0 | 1]: around the copy of a chunk into slot 0 | 1 (timed)
     KernelProf prof;
 };
 
@@ -327,6 +334,17 @@ int abandon_sink(gbin_ctx *ctx, HostSink *sink) {
     CU(cudaStreamSynchronize(ctx->st_d2h));
     sink->kmers_done = sink->ids_done = 0;
     return GBIN_OK;
+}
+
+// The big arrays of a host table are streamed into the pinned arenas as far as these reach (they are sized by the previous call,
+// so the first call on a context copies everything at the end and later calls of similar size overlap the copy).
+HostSink host_sink(gbin_ctx *ctx) {
+    HostSink sink{static_cast<uint64_t *>(ctx->h_kmer_codes.p), static_cast<uint64_t *>(ctx->h_kmer_id_off.p), static_cast<int32_t *>(ctx->h_read_ids.p),
+                  0, 0, 0, 0, ctx->host_chunks};
+    sink.kmer_cap = ctx->h_kmer_codes.cap / (sizeof(uint64_t) * ctx->KW);
+    if (ctx->h_kmer_id_off.cap / sizeof(uint64_t) < sink.kmer_cap) sink.kmer_cap = ctx->h_kmer_id_off.cap / sizeof(uint64_t);
+    sink.id_cap = ctx->h_read_ids.cap / sizeof(int32_t);
+    return sink;
 }
 
 // Partition of n records by owner: launch(scratch, d_counts, st) runs the partition kernels and returns how many it launched.
@@ -1110,6 +1128,7 @@ int gbin_create(const gbin_config *cfg, gbin_ctx **out) {
     for (int i = 0; i < SKR_MAX_CHUNKS && e == cudaSuccess; i++) e = cudaEventCreateWithFlags(&ctx->ev_feed[i], cudaEventDisableTiming);
     for (int i = 0; i < SKR_MAX_CHUNKS && e == cudaSuccess; i++) e = cudaEventCreateWithFlags(&ctx->ev_chunk[i], cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_copy, cudaEventDisableTiming);
+    for (int i = 0; i < 4 && e == cudaSuccess; i++) e = cudaEventCreate(&ctx->ev_part_h2d[i]);
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&ctx->st_aux, cudaStreamNonBlocking);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_join, cudaEventDisableTiming);
@@ -1140,6 +1159,7 @@ void gbin_destroy(gbin_ctx *ctx) {
         cudaEventDestroy(ctx->ev_chunk[i]);
     }
     cudaEventDestroy(ctx->ev_copy);
+    for (int i = 0; i < 4; i++) cudaEventDestroy(ctx->ev_part_h2d[i]);
     cudaEventDestroy(ctx->ev_fork);
     cudaEventDestroy(ctx->ev_join);
     cudaStreamDestroy(ctx->st_aux);
@@ -1240,6 +1260,9 @@ int gbin_set_tuning(gbin_ctx *ctx, const char *name, int value) {
     } else if (!strcmp(name, "host_chunks")) {
         if (value < 1 || value > SKR_MAX_CHUNKS) return GBIN_E_INVALID_ARG;
         ctx->host_chunks = value;
+    } else if (!strcmp(name, "part_chunk_kb")) {
+        if (value < 1) return GBIN_E_INVALID_ARG;
+        ctx->part_chunk_bytes = (uint64_t)value << 10;
     } else {
         return GBIN_E_INVALID_ARG;
     }
@@ -1374,13 +1397,7 @@ int gbin_bin_reads_host(gbin_ctx *ctx, const gbin_reads *reads, gbin_table *out)
         }
     }
     if (!use_feed) CU(cudaEventRecord(ctx->ev[EV_READS_ON_DEVICE], st));
-    // the big arrays of the table are streamed into the pinned arenas as far as these reach (they are sized by the previous
-    // call, so the first call on a context copies everything at the end and later calls of similar size overlap the copy)
-    HostSink sink{static_cast<uint64_t *>(ctx->h_kmer_codes.p), static_cast<uint64_t *>(ctx->h_kmer_id_off.p), static_cast<int32_t *>(ctx->h_read_ids.p),
-                  0, 0, 0, 0, ctx->host_chunks};
-    sink.kmer_cap = ctx->h_kmer_codes.cap / (sizeof(uint64_t) * ctx->KW);
-    if (ctx->h_kmer_id_off.cap / sizeof(uint64_t) < sink.kmer_cap) sink.kmer_cap = ctx->h_kmer_id_off.cap / sizeof(uint64_t);
-    sink.id_cap = ctx->h_read_ids.cap / sizeof(int32_t);
+    HostSink sink = host_sink(ctx);
     gbin_table dev;
     int rc = bin_device_impl(ctx, &d, st, &dev, &launches, use_feed ? &feed : nullptr, &sink);
     if (rc) {
@@ -1394,6 +1411,301 @@ int gbin_bin_reads_host(gbin_ctx *ctx, const gbin_reads *reads, gbin_table *out)
     CU(cudaStreamSynchronize(st));
     CU(cudaStreamSynchronize(ctx->st_d2h));
     finish_timings(ctx, launches, true);
+    return GBIN_OK;
+}
+
+// ---------------------------------------------------------------- the table in owner parts, one part per call
+
+namespace {
+// A chunk of a part call: reads [r0, r1), which span bytes [b0, b1) of reads->data.
+struct PartChunk {
+    uint64_t r0, r1, b0, b1;
+    uint32_t max_len;  // 0: not known on the host (plan_reads finds it)
+};
+
+// Cuts the reads into chunks of whole reads whose byte span is at most ctx->part_chunk_bytes, with at least one read each.
+// Fixed-stride reads: contiguous byte ranges.  Ragged reads in host memory: the span [min start, max end) of the chunk's reads, which
+// is copied whole and exceeds the budget only for a single read longer than it (the chunk buffer then grows to fit).  Reads laid out
+// out of order make more, shorter chunks.
+// Ragged reads in device memory are scanned where they are, so they are cut by read count, at the mean bytes per read.
+int plan_part_chunks(gbin_ctx *ctx, const gbin_reads *rd, bool on_host, std::vector<PartChunk> *out) {
+    const uint64_t n = rd->n_reads, budget = ctx->part_chunk_bytes;
+    out->clear();
+    if (n == 0) return GBIN_OK;
+    if (!rd->starts || !on_host) {
+        const uint64_t per_read = rd->starts ? rd->data_bytes / n + 1 : rd->stride;
+        const uint64_t per = per_read == 0 ? n : (budget / per_read ? budget / per_read : 1);
+        for (uint64_t r0 = 0; r0 < n; r0 += per) {
+            const uint64_t r1 = n - r0 > per ? r0 + per : n;
+            if (rd->starts) out->push_back({r0, r1, 0, rd->data_bytes, rd->max_read_len});
+            else out->push_back({r0, r1, r0 * rd->stride, (r1 - 1) * rd->stride + rd->read_len, rd->read_len});
+        }
+        return GBIN_OK;
+    }
+    for (uint64_t i = 0; i < n; i++)
+        if (rd->starts[i] + rd->lens[i] > rd->data_bytes) return fail(ctx, GBIN_E_INVALID_ARG, "read %llu exceeds data_bytes", (unsigned long long)i);
+    for (uint64_t r0 = 0, r1; r0 < n; r0 = r1) {
+        uint64_t lo = rd->starts[r0], hi = lo + rd->lens[r0];
+        uint32_t ml = rd->lens[r0];
+        for (r1 = r0 + 1; r1 < n; r1++) {
+            const uint64_t s = rd->starts[r1], e = s + rd->lens[r1];
+            const uint64_t nlo = s < lo ? s : lo, nhi = e > hi ? e : hi;
+            if (nhi - nlo > budget) break;
+            lo = nlo;
+            hi = nhi;
+            if (rd->lens[r1] > ml) ml = rd->lens[r1];
+        }
+        out->push_back({r0, r1, lo, hi, ml ? ml : 1});
+    }
+    return GBIN_OK;
+}
+
+// Streams every chunk through the device and keeps the records of part `part` in ctx->part_rec, in arrival order: super-k-mer
+// records, or instance records when `inst`.  Host form: chunk c is copied into slot c & 1 on the copy stream while chunk c - 1 is
+// scanned; the slot's previous chunk has been scanned and selected by then (the host waited for both).  *too_long: the
+// super-k-mer scan cannot hold these reads, nothing was selected.  *scan_ms / *h2d_ms: scan + select / copy time summed over chunks.
+int scan_select_part(gbin_ctx *ctx, const gbin_reads *rd, bool on_host, const std::vector<PartChunk> &chunks, uint32_t part, uint32_t n_parts,
+                     bool inst, cudaStream_t st, int *launches, uint64_t *n_sel, uint64_t *n_sel_inst, bool *too_long, float *scan_ms, float *h2d_ms) {
+    const int words = inst ? 2 * ctx->KW + 2 : (ctx->cfg.kmer_size <= 32 ? 8 : 12);
+    const size_t rb = 4u * (size_t)words;
+    Misc *dm = ctx->misc.as<Misc>();
+    Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
+    *n_sel = *n_sel_inst = 0;
+    *too_long = false;
+    CU(cudaMemsetAsync(dm->part_sel, 0, sizeof dm->part_sel, st));
+    std::vector<uint64_t> rebased[2];  // host staging of a slot's starts, relative to its chunk's first byte
+    auto copy_in = [&](size_t c) -> int {
+        const PartChunk &k = chunks[c];
+        const int s = (int)(c & 1);
+        CU(ctx->part_data[s].ensure(k.b1 - k.b0 + 64));
+        CU(cudaEventRecord(ctx->ev_part_h2d[2 * s], ctx->st_h2d));
+        if (k.b1 > k.b0) CU(cudaMemcpyAsync(ctx->part_data[s].p, rd->data + k.b0, k.b1 - k.b0, cudaMemcpyHostToDevice, ctx->st_h2d));
+        if (rd->starts) {
+            const uint64_t m = k.r1 - k.r0;
+            CU(ctx->part_meta[s].ensure(m * (sizeof(uint64_t) + sizeof(uint32_t)) + 16));
+            rebased[s].resize(m);
+            for (uint64_t i = 0; i < m; i++) rebased[s][i] = rd->starts[k.r0 + i] - k.b0;
+            CU(cudaMemcpyAsync(ctx->part_meta[s].p, rebased[s].data(), m * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->st_h2d));
+            CU(cudaMemcpyAsync(ctx->part_meta[s].as<char>() + m * sizeof(uint64_t), rd->lens + k.r0, m * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->st_h2d));
+        }
+        CU(cudaEventRecord(ctx->ev_part_h2d[2 * s + 1], ctx->st_h2d));
+        return GBIN_OK;
+    };
+    auto elapsed = [](cudaEvent_t a, cudaEvent_t b) {
+        float t = 0.f;
+        if (cudaEventElapsedTime(&t, a, b) != cudaSuccess) (void)cudaGetLastError();
+        return t;
+    };
+    int rc = (on_host && !chunks.empty()) ? copy_in(0) : GBIN_OK;
+    for (size_t c = 0; !rc && c < chunks.size(); c++) {
+        const PartChunk &k = chunks[c];
+        const int s = (int)(c & 1);
+        if (on_host && c + 1 < chunks.size() && (rc = copy_in(c + 1))) return rc;
+        gbin_reads v = *rd;  // the chunk as a batch of its own, scanned with arrival_base = its first read
+        v.n_reads = k.r1 - k.r0;
+        v.read_ids = nullptr;
+        v.max_read_len = k.max_len;
+        if (on_host) {
+            v.data = ctx->part_data[s].as<char>();
+            v.data_bytes = k.b1 - k.b0;
+            if (rd->starts) {
+                v.starts = ctx->part_meta[s].as<uint64_t>();
+                v.lens = reinterpret_cast<const uint32_t *>(ctx->part_meta[s].as<char>() + v.n_reads * sizeof(uint64_t));
+            }
+            CU(cudaStreamWaitEvent(st, ctx->ev_part_h2d[2 * s + 1], 0));
+        } else if (rd->starts) {
+            v.starts = rd->starts + k.r0;
+            v.lens = rd->lens + k.r0;
+        } else {
+            v.data = rd->data + k.b0;
+            v.data_bytes = k.b1 - k.b0;
+        }
+        CU(cudaEventRecord(ctx->ev[EV_READS_ON_DEVICE], st));
+        uint64_t n_c = 0, n_src = 0;
+        uint32_t max_len = 0;
+        if ((rc = plan_reads(ctx, &v, st, &n_c, &max_len, launches))) return rc;
+        if (max_len > gbin_max_read_len()) return fail(ctx, GBIN_E_TOO_LARGE, "read length %u exceeds the limit of %u bases", max_len, gbin_max_read_len());
+        const void *src = nullptr;
+        if (n_c && inst) {
+            CU(ctx->rec_b.ensure((n_c + 1) * rb));
+            if ((rc = run_scan(ctx, &v, (uint32_t)k.r0, ctx->rec_b.p, max_len, st, launches))) return rc;
+            CU(read_back(ctx, &Misc::grp, st));
+            if (hm->grp.bad_bases) return fail(ctx, GBIN_E_NON_ACGT, "%llu bases other than A/C/G/T in the batch", hm->grp.bad_bases);
+            src = ctx->rec_b.p;
+            n_src = n_c;
+        } else if (n_c) {
+            rc = run_skr_scan(ctx, &v, n_c, max_len, (uint32_t)k.r0, nullptr, 0, st, &n_src, launches);
+            if (rc == GBIN_E_TOO_LARGE) {  // reads longer than the super-k-mer scan holds in shared memory
+                *too_long = true;
+                return GBIN_OK;
+            }
+            if (rc) return rc;
+            src = ctx->skr_a.p;
+        }
+        if (n_src) {
+            const uint64_t need = *n_sel + n_src;  // every record of the chunk might belong to the part
+            if ((need + 1) * rb > ctx->part_rec.cap) {
+                // grow towards what the whole call is expected to select: the part's records so far, extrapolated over the reads
+                uint64_t want = (uint64_t)((double)(*n_sel + n_src / n_parts + 1) * (double)rd->n_reads / (double)k.r1 * 1.1);
+                if (want < need) want = need;
+                CU(ctx->part_rec.ensure_keep((want + 1) * rb, *n_sel * rb, st));
+            }
+            CU(ctx->part_state.ensure(select_part_state_bytes(n_src)));
+            const bool on = ctx->prof.begin(KK_RADIX_SCATTER, st);
+            const int l = select_part(src, n_src, words, !inst, part, n_parts, ctx->part_rec.as<char>() + *n_sel * rb, ctx->part_state.as<unsigned long long>(),
+                                      &dm->part_ticket, dm->part_sel, st);
+            ctx->prof.end(on, l, st);
+            *launches += l;
+            CU(cudaGetLastError());
+            CU(read_back(ctx, &Misc::part_sel, st));
+            *n_sel = hm->part_sel[0];
+            *n_sel_inst = hm->part_sel[1];
+        }
+        CU(cudaEventRecord(ctx->ev[EV_SCANNED], st));
+        CU(cudaEventSynchronize(ctx->ev[EV_SCANNED]));
+        *scan_ms += elapsed(ctx->ev[EV_READS_ON_DEVICE], ctx->ev[EV_SCANNED]);
+        if (on_host) *h2d_ms += elapsed(ctx->ev_part_h2d[2 * s], ctx->ev_part_h2d[2 * s + 1]);
+    }
+    return rc;
+}
+
+// One part of the table (gbin_bin_reads_host_part / gbin_bin_reads_device_part) into the context's device table.  The part is
+// selected from super-k-mer records and grouped by pipeline 3 (2 when 3 gives it up); it is redone from the reads in instance-record
+// form (pipeline 1) when pipeline 2 overflows too, when the reads are too long for the super-k-mer scan, or when the context is set
+// to pipeline 1.  sink: the host form's pinned arenas.
+int bin_part_impl(gbin_ctx *ctx, const gbin_reads *rd, bool on_host, uint32_t part, uint32_t n_parts, cudaStream_t st, HostSink *sink, gbin_table *out,
+                  int *launches, float *scan_ms, float *h2d_ms) {
+    if (n_parts == 0 || n_parts > 65536 || part >= n_parts) return fail(ctx, GBIN_E_INVALID_ARG, "part %u of %u parts (need part < n_parts <= 65536)", part, n_parts);
+    const uint64_t n = rd->n_reads;
+    if (n >= (1ull << 32)) return fail(ctx, GBIN_E_TOO_LARGE, "more than 2^32-1 reads in one batch");
+    if (n) {
+        if (!rd->data || (on_host && rd->data_bytes == 0)) return fail(ctx, GBIN_E_INVALID_ARG, "reads need data and data_bytes");
+        if (rd->starts && !rd->lens) return fail(ctx, GBIN_E_INVALID_ARG, "ragged reads need lens");
+        if (!rd->starts && rd->stride < rd->read_len) return fail(ctx, GBIN_E_INVALID_ARG, "stride < read_len");
+        if (!rd->starts && rd->data_bytes && (n - 1) * rd->stride + rd->read_len > rd->data_bytes)
+            return fail(ctx, GBIN_E_INVALID_ARG, "fixed-stride reads exceed data_bytes");
+    }
+    std::vector<PartChunk> chunks;
+    int rc = plan_part_chunks(ctx, rd, on_host, &chunks);
+    if (rc) return rc;
+    const int32_t *d_ids = rd->read_ids;  // looked up by arrival = index over all the reads
+    if (on_host && rd->read_ids && n) {
+        CU(ctx->d_ids.ensure(n * sizeof(int32_t)));
+        CU(cudaMemcpyAsync(ctx->d_ids.p, rd->read_ids, n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+        d_ids = ctx->d_ids.as<int32_t>();
+    }
+    bool inst = ctx->pipeline == 1;
+    for (;;) {
+        uint64_t n_sel = 0, n_sel_inst = 0;
+        bool too_long = false;
+        rc = scan_select_part(ctx, rd, on_host, chunks, part, n_parts, inst, st, launches, &n_sel, &n_sel_inst, &too_long, scan_ms, h2d_ms);
+        CU(cudaStreamSynchronize(ctx->st_h2d));  // a copy into a chunk buffer may still be in flight when the loop ended early
+        if (rc) return rc;
+        if (too_long) {
+            ctx->fallbacks++;
+            inst = true;
+            continue;
+        }
+        if (!inst && n_sel) {
+            // the chunks' record buffer is dead: lend it to pipeline 3's entry sort, as gbin_donate_scratch does
+            ctx->donated = ctx->skr_a.p;
+            ctx->donated_bytes = ctx->skr_a.cap;
+            bool done = false;
+            int used = 2;
+            uint64_t n_chk = 0;
+            rc = run_skr_group(ctx, ctx->part_rec.p, n_sel, d_ids, rd->id_base, st, out, launches, &done, &n_chk, sink, &used);
+            ctx->donated = nullptr;
+            ctx->donated_bytes = 0;
+            if (rc) return rc;
+            if (done) {
+                if (n_chk != n_sel_inst)
+                    return fail(ctx, GBIN_E_CUDA, "internal: the part's records hold %llu windows, grouped %llu", (unsigned long long)n_sel_inst, (unsigned long long)n_chk);
+                ctx->last_pipeline = used;
+                break;
+            }
+            if ((rc = abandon_sink(ctx, sink))) return rc;
+            inst = true;  // a shared-memory unit overflowed: this part goes through pipeline 1
+            continue;
+        }
+        // instance records (or an empty part): sort + run-length + prune + emit in HBM
+        if (n_sel >= (1ull << 32) - 8192) return fail(ctx, GBIN_E_TOO_LARGE, "%llu k-mer instances in one part: too many for pipeline 1", (unsigned long long)n_sel);
+        memset(&ctx->rs, 0, sizeof ctx->rs);
+        CU(ctx->rec_b.ensure((n_sel + 1) * (sizeof(uint64_t) * ctx->KW + 8)));
+        CU(cudaMemsetAsync(&ctx->misc.as<Misc>()->grp.bad_bases, 0, sizeof(unsigned long long), st));
+        rc = run_group(ctx, n_sel ? ctx->part_rec.p : nullptr, ctx->rec_b.p, n_sel, d_ids, rd->id_base, st, out, launches, ctx->ev[EV_SORTED]);
+        if (rc) return rc;
+        ctx->last_pipeline = inst ? 1 : ctx->pipeline;
+        break;
+    }
+    CU(cudaEventRecord(ctx->ev[EV_GROUPED], st));
+    return GBIN_OK;
+}
+
+// gbin_plan_parts' model of a part call's device memory (DESIGN.md §5).  PART_BYTES_PER_INSTANCE per k-mer instance of the part: the
+// largest high-water mark per instance measured on a B200 for a one-part call (57.1 B at the config-5 shape; configs 2, 4 and the
+// config-3 shape 46.4 / 56.6 / 53.9 B) — its records, pipeline 3's sort, plan, staging and table with the buffers' slack, and there
+// also the read chunk.  PART_SKEW: the owner hash's imbalance (1.4 % for the busiest of 8 owners, DESIGN.md §6) with room for larger
+// P.  PART_BYTES_PER_CHUNK_BYTE per byte of part_chunk_kb: two read chunks + one chunk's super-k-mer records, which the scan sizes at
+// a quarter of the chunk's instances (+ reads) x 32 B with 1/16 slack: 2 + 0.8 x 0.25 x 32 x 17/16 ~ 9 for 150-base reads.
+constexpr double PART_BYTES_PER_INSTANCE = 58.0, PART_SKEW = 1.05, PART_BYTES_PER_CHUNK_BYTE = 9.0;
+}  // namespace
+
+int gbin_bin_reads_host_part(gbin_ctx *ctx, const gbin_reads *reads, uint32_t part, uint32_t n_parts, gbin_table *out) {
+    if (!ctx || !reads || !out) return GBIN_E_INVALID_ARG;
+    cudaStream_t st;
+    CU(begin_call(ctx, nullptr, &st));
+    int launches = 0;
+    float scan_ms = 0.f, h2d_ms = 0.f;
+    CU(cudaEventRecord(ctx->ev[EV_START], st));
+    HostSink sink = host_sink(ctx);
+    gbin_table dev;
+    int rc = bin_part_impl(ctx, reads, true, part, n_parts, st, &sink, &dev, &launches, &scan_ms, &h2d_ms);
+    if (rc) {
+        cudaStreamSynchronize(ctx->st_h2d);
+        cudaStreamSynchronize(ctx->st_d2h);
+        return rc;
+    }
+    rc = table_to_pinned(ctx, dev, &sink, st, out);
+    if (rc) return rc;
+    CU(cudaEventRecord(ctx->ev[EV_TABLE_ON_HOST], st));
+    CU(cudaStreamSynchronize(st));
+    CU(cudaStreamSynchronize(ctx->st_d2h));
+    finish_timings(ctx, launches, true);
+    ctx->tm.h2d_ms = h2d_ms;
+    ctx->tm.scan_ms = scan_ms;
+    return GBIN_OK;
+}
+
+int gbin_bin_reads_device_part(gbin_ctx *ctx, const gbin_reads *reads, uint32_t part, uint32_t n_parts, void *stream, gbin_table *out) {
+    if (!ctx || !reads || !out) return GBIN_E_INVALID_ARG;
+    cudaStream_t st;
+    CU(begin_call(ctx, stream, &st));
+    int launches = 0;
+    float scan_ms = 0.f, h2d_ms = 0.f;
+    CU(cudaEventRecord(ctx->ev[EV_START], st));
+    int rc = bin_part_impl(ctx, reads, false, part, n_parts, st, nullptr, out, &launches, &scan_ms, &h2d_ms);
+    if (rc) return rc;
+    CU(cudaStreamSynchronize(st));
+    finish_timings(ctx, launches, false);
+    ctx->tm.scan_ms = scan_ms;
+    return GBIN_OK;
+}
+
+int gbin_plan_parts(gbin_ctx *ctx, uint64_t n_instances, uint32_t *n_parts_out) {
+    if (!ctx || !n_parts_out) return GBIN_E_INVALID_ARG;
+    CU(cudaSetDevice(ctx->cfg.device));
+    size_t free_b = 0, total_b = 0;
+    CU(cudaMemGetInfo(&free_b, &total_b));
+    const double room = (double)free_b - PART_BYTES_PER_CHUNK_BYTE * (double)ctx->part_chunk_bytes;
+    auto fits = [&](uint64_t P) { return PART_BYTES_PER_INSTANCE * PART_SKEW * (double)((n_instances + P - 1) / P) <= room; };
+    const double est = room > 0 ? PART_BYTES_PER_INSTANCE * PART_SKEW * (double)n_instances / room : 65537.0;
+    uint64_t P = est < 65537.0 ? (uint64_t)est : 65537;
+    if (P < 1) P = 1;
+    while (P > 1 && fits(P - 1)) P--;
+    while (P <= 65536 && !fits(P)) P++;
+    if (P > 65536)
+        return fail(ctx, GBIN_E_NOMEM, "%llu k-mer instances do not fit %llu free bytes in 65536 parts", (unsigned long long)n_instances, (unsigned long long)free_b);
+    *n_parts_out = (uint32_t)P;
     return GBIN_OK;
 }
 

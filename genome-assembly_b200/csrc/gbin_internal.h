@@ -101,6 +101,12 @@ int radix_sort_skr_by_mmer(void *a, void *b, uint64_t n, int skr_words, int M, v
                            uint64_t *side_out, KernelProf *prof, cudaStream_t st);
 int radix_partition_skr_by_owner(const void *in, void *out, uint64_t n, int skr_words, uint32_t n_parts, void *scratch, uint64_t *d_counts,
                                  cudaStream_t st);
+// Stable select of part `part` of n_parts: the records (super-k-mer records of rec_words 8 | 12 when skr, else instance records of
+// rec_words 4 | 6) with owner_of_mmer(m-mer, n_parts) == part go to out[0..) in input order; counters[0] += their number,
+// counters[1] += their k-mer instances.  tile_state: select_part_state_bytes(n), ticket: one u32 (both zeroed here).
+size_t select_part_state_bytes(uint64_t n);
+int select_part(const void *in, uint64_t n, int rec_words, bool skr, uint32_t part, uint32_t n_parts, void *out, unsigned long long *tile_state,
+                uint32_t *ticket, unsigned long long *counters, cudaStream_t st);
 
 // ---- skr_scan.cu
 // Scans reads [read_begin, read_end) of rv; record offsets continue from counters[1] (zero it before the first launch).

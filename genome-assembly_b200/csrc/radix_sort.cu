@@ -14,6 +14,7 @@
 // every digit run leaves the SM as one contiguous, coalesced store.
 #include "gbin_device.cuh"
 #include "gbin_internal.h"
+#include "lookback.cuh"
 #include "prefix_scan.cuh"
 
 namespace gbin {
@@ -501,6 +502,105 @@ int radix_partition_skr_by_owner(const void *in, void *out, uint64_t n, int skr_
 int radix_exchange_skr_by_owner(const void *in, uint64_t n, int skr_words, void *scratch, const XchgPlan &xp, cudaStream_t st) {
     // n == 0 still takes part in the count exchange and the completion barrier (one empty tile)
     return one_pass_any(skr_words / 2, in, nullptr, n, DigitSel{0, 32, xp.world}, static_cast<uint32_t *>(scratch), nullptr, st, &xp);
+}
+
+// ------------------------------------------------------------------ one owner part (the table in parts, one part per call)
+// Stable select of the records with owner_of_mmer(m-mer, n_parts) == part, written in input order to out[0..): one launch that
+// reads every record once and writes only the selected ones, at their final place.  Tiles are handed out by a ticket, so a tile's
+// predecessor is always running, and a tile's output offset comes from the decoupled look-back (lookback.cuh).  Inside a tile,
+// record j = tile * SEL_TILE + i * SEL_THREADS + tid; the (round i, warp) counts are scanned in that order, which is input order.
+// SKR: super-k-mer records (m-mer in word 1, windows in the low byte of word 2); else instance records (m-mer in the low half of
+// the last 64-bit word, one window each).  counters[0] += records selected, counters[1] += their k-mer instances.
+constexpr int SEL_THREADS = 256, SEL_ITEMS = 4, SEL_TILE = SEL_THREADS * SEL_ITEMS;
+static_assert(SEL_ITEMS * RS_WARPS == 32, "one lane per (round, warp) count");
+
+template <int NU64, bool SKR>
+__global__ void __launch_bounds__(SEL_THREADS)
+    select_part_kernel(const Blob<NU64> *__restrict__ in, uint64_t n, uint32_t part, uint32_t n_parts, Blob<NU64> *__restrict__ out,
+                       unsigned long long *__restrict__ tile_state, uint32_t *__restrict__ ticket, unsigned long long *__restrict__ counters) {
+    __shared__ uint32_t s_tile;
+    __shared__ uint32_t s_off[SEL_ITEMS * RS_WARPS];
+    __shared__ unsigned long long s_inst[RS_WARPS];
+    __shared__ unsigned long long s_base;
+    const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    if (tid == 0) s_tile = atomicAdd(ticket, 1u);
+    __syncthreads();
+    const uint32_t tile = s_tile;
+    const uint64_t base = (uint64_t)tile * SEL_TILE;
+    Blob<NU64> items[SEL_ITEMS];
+    bool sel[SEL_ITEMS];
+    unsigned long long inst = 0;
+#pragma unroll
+    for (int i = 0; i < SEL_ITEMS; i++) {
+        const uint64_t j = base + (uint64_t)i * SEL_THREADS + tid;
+        sel[i] = false;
+        if (j < n) {
+            items[i] = load_blob<NU64>(in + j);
+            const uint32_t mmer = SKR ? (uint32_t)(items[i].w[0] >> 32) : (uint32_t)items[i].w[NU64 - 1];
+            sel[i] = owner_of_mmer(mmer, n_parts) == part;
+            if (sel[i]) inst += SKR ? (items[i].w[1] & 0xffull) : 1ull;
+        }
+    }
+#pragma unroll
+    for (int i = 0; i < SEL_ITEMS; i++) {
+        const unsigned b = __ballot_sync(0xffffffffu, sel[i]);
+        if (lane == 0) s_off[i * RS_WARPS + warp] = __popc(b);
+    }
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) inst += __shfl_xor_sync(0xffffffffu, inst, d);
+    if (lane == 0) s_inst[warp] = inst;
+    __syncthreads();
+    if (warp == 0) {
+        const uint32_t c = s_off[lane];
+        uint32_t incl = c;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const uint32_t v = __shfl_up_sync(0xffffffffu, incl, d);
+            if (lane >= (uint32_t)d) incl += v;
+        }
+        const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
+        s_off[lane] = incl - c;
+        if (lane == 0) lkb_publish_aggregate(tile_state, tile, total);
+        const unsigned long long prefix = lkb_resolve_warp<1>(tile_state, tile, total, lane);
+        if (lane == 0) {
+            s_base = prefix;
+            unsigned long long ti = 0;
+            for (int w = 0; w < RS_WARPS; w++) ti += s_inst[w];
+            if (total) atomicAdd(&counters[0], (unsigned long long)total);
+            if (ti) atomicAdd(&counters[1], ti);
+        }
+    }
+    __syncthreads();
+    const unsigned long long b0 = s_base;
+    const uint32_t lt_mask = (1u << lane) - 1;
+#pragma unroll
+    for (int i = 0; i < SEL_ITEMS; i++) {
+        const unsigned b = __ballot_sync(0xffffffffu, sel[i]);
+        if (sel[i]) store_blob<NU64>(out + b0 + s_off[i * RS_WARPS + warp] + __popc(b & lt_mask), items[i]);
+    }
+}
+
+size_t select_part_state_bytes(uint64_t n) { return (n / SEL_TILE + 1) * sizeof(unsigned long long); }
+
+int select_part(const void *in, uint64_t n, int rec_words, bool skr, uint32_t part, uint32_t n_parts, void *out, unsigned long long *tile_state,
+                uint32_t *ticket, unsigned long long *counters, cudaStream_t st) {
+    if (n == 0) return 0;
+    const uint64_t tiles = (n + SEL_TILE - 1) / SEL_TILE;
+    cudaMemsetAsync(tile_state, 0, tiles * sizeof(unsigned long long), st);
+    cudaMemsetAsync(ticket, 0, sizeof(uint32_t), st);
+    const unsigned grid = (unsigned)tiles;
+#define GBIN_SELECT(NU64, SKR)                                                                                                            \
+    select_part_kernel<NU64, SKR><<<grid, SEL_THREADS, 0, st>>>(static_cast<const Blob<NU64> *>(in), n, part, n_parts, static_cast<Blob<NU64> *>(out), \
+                                                                 tile_state, ticket, counters)
+    if (skr) {
+        if (rec_words == 8) GBIN_SELECT(4, true);
+        else GBIN_SELECT(6, true);
+    } else {
+        if (rec_words == 4) GBIN_SELECT(2, false);
+        else GBIN_SELECT(3, false);
+    }
+#undef GBIN_SELECT
+    return 1;
 }
 
 }  // namespace gbin

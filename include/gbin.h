@@ -179,7 +179,8 @@ int gbin_set_pipeline(gbin_ctx *ctx, int pipeline);
  *   "v3_h"   0..           with v3_nc = 2: bases next to the signature that extend the level-1 key (clamped to what K, M allow)
  *   "v3_pass_max" >= 1000  k-mer instances per pass of pipeline 3 (default 2 * 10^9; small values exercise the multi-pass path)
  *   "xchg_timeout_ms" >= 100  how long the multi-GPU exchange kernels wait for a peer before they give up (default 120000)
- *   "host_chunks" 1..16    pieces in which gbin_bin_reads_host streams reads in / the table out */
+ *   "host_chunks" 1..16    pieces in which gbin_bin_reads_host streams reads in / the table out
+ *   "part_chunk_kb" >= 1   byte span of the read chunks of gbin_bin_reads_*_part, in KiB (default 1048576 = 1 GiB) */
 int gbin_set_tuning(gbin_ctx *ctx, const char *name, int value);
 /* Lends `bytes` of device memory (16-byte aligned, caller-owned) to the NEXT grouping call on the context (gbin_group_skr_device,
  * gbin_bin_reads_device): pipeline 3 puts the two buffers of its entry sort there when they fit, instead of allocating them.  The
@@ -274,6 +275,23 @@ int gbin_multi_devices(const gbin_multi *m);
 gbin_ctx *gbin_multi_context(gbin_multi *m, int i);
 const char *gbin_multi_last_error(const gbin_multi *m);
 int gbin_multi_bin_reads_host(gbin_multi *m, const gbin_reads *reads, gbin_table *tables_out);
+
+/* ---- read sets larger than one device: the table in P owner parts, one part per call ----
+ * Part p of P is the table restricted to the m-mer buckets with gbin_owner_of(mmer_code, P) == p: the same table GPU p owns in a
+ * P-GPU run; n_instances / n_distinct count that part only.  Digests of the P parts add up to the digest of the whole table.
+ * Every call streams ALL reads through the device in chunks (gbin_set_tuning "part_chunk_kb"), keeps the super-k-mer records of
+ * part p and groups them, so device memory holds two read chunks + about 1/P of the records and of the table, whatever n_reads is.
+ * Arrival index = read index over the whole `reads` (ids as in gbin_bin_reads_host: read_ids[i] or id_base + i); n_reads < 2^32.
+ * The host form writes into the context's pinned arena (ctx_owned = 1, valid until the next call), as gbin_bin_reads_host does:
+ * digest, dump or gbin_table_clone each part before asking for the next.  n_parts must be 1..65536 and part < n_parts
+ * (else GBIN_E_INVALID_ARG).  A part that overflows pipeline 2's units, reads too long for the super-k-mer scan, or a context set
+ * to pipeline 1 make the part go through instance records (pipeline 1); gbin_get_pipeline_info reports what made this part. */
+int gbin_bin_reads_host_part(gbin_ctx *ctx, const gbin_reads *reads, uint32_t part, uint32_t n_parts, gbin_table *out);
+/* Same with reads in DEVICE memory (e.g. from gbin_split_reads_device); the table stays on the device (ctx_owned, on_device = 1). */
+int gbin_bin_reads_device_part(gbin_ctx *ctx, const gbin_reads *reads, uint32_t part, uint32_t n_parts, void *stream, gbin_table *out);
+/* Smallest P for which one part of a batch of n_instances k-mer instances fits the device's free memory now (model and measured
+ * constants: DESIGN.md §5).  GBIN_E_NOMEM when not even 65536 parts fit. */
+int gbin_plan_parts(gbin_ctx *ctx, uint64_t n_instances, uint32_t *n_parts_out);
 
 /* ---- main's read loop on the device (binning.c:1154-1166; SURVEY.md 8 row f2) ----
  * Splits a file image in DEVICE memory into reads exactly as `while (fgets(read, read_length_define, file)) { read[--len] = 0; ... }`
