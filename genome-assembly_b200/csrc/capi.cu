@@ -91,6 +91,13 @@ struct HostBuf {  // page-locked; freed when destroyed
     }
 };
 
+// A range of host reads copied to the device (stage_host_reads): its bytes, its starts (rebased to the first copied byte) followed by
+// its lens, and the pinned host array the starts are rebased in.  Slot 0 also holds gbin_bin_file_host's file image and its split.
+struct ReadStage {
+    DevBuf data, meta;
+    HostBuf rebased;
+};
+
 // Small device-resident scalars (ctx->misc) and their pinned host mirror (ctx->h_misc).  Values the host needs at the same
 // point are grouped into one member, so that read_back() fetches them in one copy.
 struct Misc {
@@ -165,8 +172,9 @@ struct gbin_ctx {
     char err[512];
     gbin_timings tm;
     cudaEvent_t ev[EV_COUNT];
-    // inputs staged by the host path
-    DevBuf d_reads, d_starts, d_lens, d_ids;
+    // inputs staged by the host path: [0] a whole batch or shard, or a chunk of the parts path, which alternates with [1]
+    ReadStage stage[2];
+    DevBuf d_ids;
     // pipeline workspace
     DevBuf rec_a, rec_b, radix_scratch, win_counts, rec_off, scan_scratch;
     DevBuf group_of, run_start, surv_index, id_offset, surv_group, bucket_of;
@@ -208,8 +216,8 @@ struct gbin_ctx {
     // pinned host arena for results of the host path + small readbacks
     HostBuf h_misc, h_result, h_kmer_codes, h_kmer_id_off, h_read_ids, h_file;
     DevBuf split_nl, split_tiles_buf, split_base;  // device-side fgets splitting
-    // one owner part per call: two read chunks (bytes; rebased starts + lens) of the host form, the part's records, the select's tiles
-    DevBuf part_data[2], part_meta[2], part_rec, part_state;
+    // one owner part per call: the part's records, the select's tiles
+    DevBuf part_rec, part_state;
     uint64_t part_chunk_bytes = 1ull << 30;  // gbin_set_tuning "part_chunk_kb"
     cudaEvent_t ev_part_h2d[4];              // [2 * slot + 0 | 1]: around the copy of a chunk into slot 0 | 1 (timed)
     KernelProf prof;
@@ -363,6 +371,87 @@ int partition_by_owner(gbin_ctx *ctx, uint64_t n, uint32_t n_parts, void *stream
     return GBIN_OK;
 }
 
+// The checks of a reads descriptor, made before anything is copied or launched.  Reads in host memory must lie inside data_bytes and,
+// when max_read_len is given, be no longer than it; ragged reads in device memory are not looked at.  *max_len (when given) receives
+// the longest ragged host read.
+int check_reads(gbin_ctx *ctx, const gbin_reads *rd, bool on_host, uint32_t *max_len = nullptr) {
+    const uint64_t n = rd->n_reads, bytes = rd->data_bytes;
+    if (n == 0) return GBIN_OK;
+    if (!rd->data) return fail(ctx, GBIN_E_INVALID_ARG, "reads->data is NULL");
+    if (n >= (1ull << 32)) return fail(ctx, GBIN_E_TOO_LARGE, "more than 2^32-1 reads in one batch");
+    if (on_host && bytes == 0) return fail(ctx, GBIN_E_INVALID_ARG, "host reads need data_bytes");
+    if (!rd->starts) {
+        if (rd->stride < rd->read_len) return fail(ctx, GBIN_E_INVALID_ARG, "stride < read_len");
+        if (bytes && (rd->read_len > bytes || (n > 1 && rd->stride > (bytes - rd->read_len) / (n - 1))))
+            return fail(ctx, GBIN_E_INVALID_ARG, "fixed-stride reads exceed data_bytes");
+        return GBIN_OK;
+    }
+    if (!rd->lens) return fail(ctx, GBIN_E_INVALID_ARG, "ragged reads need lens");
+    uint32_t mx = 0;
+    for (uint64_t i = 0; on_host && i < n; i++) {
+        const uint64_t s = rd->starts[i], len = rd->lens[i];
+        if (s > bytes || len > bytes - s) return fail(ctx, GBIN_E_INVALID_ARG, "read %llu exceeds data_bytes", (unsigned long long)i);
+        if (rd->max_read_len && len > rd->max_read_len) return fail(ctx, GBIN_E_INVALID_ARG, "read %llu is longer than max_read_len", (unsigned long long)i);
+        if (len > mx) mx = (uint32_t)len;
+    }
+    if (max_len) *max_len = mx;
+    return GBIN_OK;
+}
+
+ReadsView reads_view(const gbin_reads *rd) {
+    return ReadsView{reinterpret_cast<const uint8_t *>(rd->data), rd->data_bytes, rd->n_reads, rd->stride, rd->read_len, rd->starts, rd->lens};
+}
+
+// Reads [r0, r1) of a batch, which span bytes [b0, b1) of its data.
+struct ReadRange {
+    uint64_t r0, r1, b0, b1;
+    uint32_t max_len;  // 0: not known on the host (plan_reads finds it)
+};
+
+// The range [r0, r1) (r0 < r1) of a checked descriptor, with its byte span and longest read: one pass over it for ragged reads.
+ReadRange read_range(const gbin_reads *rd, uint64_t r0, uint64_t r1) {
+    if (!rd->starts) return {r0, r1, r0 * rd->stride, (r1 - 1) * rd->stride + rd->read_len, rd->read_len};
+    uint64_t b0 = ~0ull, b1 = 0;
+    uint32_t ml = 0;
+    for (uint64_t i = r0; i < r1; i++) {
+        const uint64_t s = rd->starts[i], e = s + rd->lens[i];
+        if (s < b0) b0 = s;
+        if (e > b1) b1 = e;
+        if (rd->lens[i] > ml) ml = rd->lens[i];
+    }
+    return {r0, r1, b0, b1, ml ? ml : 1};
+}
+
+// Enqueues on `st` the copy of the host reads of `r` into staging slot `slot` and makes *view the device batch of those reads (its
+// read 0 is read r.r0; no ids).  Ragged starts are rebased to r.b0 in the slot's pinned array, or copied as they are when r.b0 == 0.
+// The slot must be free: whatever read it before has finished.  The caller records its own events around the copy.
+int stage_host_reads(gbin_ctx *ctx, const gbin_reads *rd, const ReadRange &r, int slot, cudaStream_t st, gbin_reads *view) {
+    ReadStage &s = ctx->stage[slot];
+    const uint64_t m = r.r1 - r.r0, bytes = r.b1 - r.b0;
+    *view = *rd;
+    view->n_reads = m;
+    view->read_ids = nullptr;
+    view->max_read_len = r.max_len;
+    CU(s.data.ensure(bytes + 64));
+    if (bytes) CU(cudaMemcpyAsync(s.data.p, rd->data + r.b0, bytes, cudaMemcpyHostToDevice, st));
+    view->data = s.data.as<char>();
+    view->data_bytes = bytes;
+    if (!rd->starts) return GBIN_OK;
+    const uint64_t *starts = rd->starts + r.r0;
+    if (r.b0) {
+        CU(s.rebased.ensure(m * sizeof(uint64_t)));
+        uint64_t *rebased = static_cast<uint64_t *>(s.rebased.p);
+        for (uint64_t i = 0; i < m; i++) rebased[i] = starts[i] - r.b0;
+        starts = rebased;
+    }
+    CU(s.meta.ensure(m * (sizeof(uint64_t) + sizeof(uint32_t)) + 16));
+    CU(cudaMemcpyAsync(s.meta.p, starts, m * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(s.meta.as<char>() + m * sizeof(uint64_t), rd->lens + r.r0, m * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    view->starts = s.meta.as<uint64_t>();
+    view->lens = reinterpret_cast<const uint32_t *>(s.meta.as<char>() + m * sizeof(uint64_t));
+    return GBIN_OK;
+}
+
 __global__ void max_len_kernel(const uint32_t *__restrict__ lens, uint64_t n, unsigned int *__restrict__ out) {
     const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     unsigned int v = i < n ? lens[i] : 0u;
@@ -375,53 +464,45 @@ struct WinCountIn {
     __device__ __forceinline__ uint64_t operator()(uint64_t j) const { return c[j]; }
 };
 
-// Validates the reads descriptor (device pointers), finds max length and instance count.
+// Finds the instance count and the longest read of a descriptor in device memory that check_reads passed or the library built, and
+// refuses reads longer than gbin_max_read_len().
 // On return: *n_inst, *max_len, and for the ragged form ctx->rec_off holds per-read record offsets.
 int plan_reads(gbin_ctx *ctx, const gbin_reads *rd, cudaStream_t st, uint64_t *n_inst, uint32_t *max_len, int *launches) {
     const int K = ctx->cfg.kmer_size;
     Misc *dm = ctx->misc.as<Misc>();
     Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
-    if (rd->n_reads == 0) {
-        *n_inst = 0;
-        *max_len = 0;
-        return GBIN_OK;
-    }
-    if (!rd->data) return fail(ctx, GBIN_E_INVALID_ARG, "reads->data is NULL");
-    if (rd->n_reads >= (1ull << 32)) return fail(ctx, GBIN_E_TOO_LARGE, "more than 2^32-1 reads in one batch");
+    *n_inst = 0;
+    *max_len = 0;
+    if (rd->n_reads == 0) return GBIN_OK;
     if (!rd->starts) {
-        if (rd->stride < rd->read_len) return fail(ctx, GBIN_E_INVALID_ARG, "stride < read_len");
-        if (rd->data_bytes && (rd->n_reads - 1) * rd->stride + rd->read_len > rd->data_bytes)
-            return fail(ctx, GBIN_E_INVALID_ARG, "fixed-stride reads exceed data_bytes");
         *max_len = rd->read_len;
         *n_inst = rd->read_len >= (uint32_t)K ? rd->n_reads * (uint64_t)(rd->read_len - K + 1) : 0;
-        return GBIN_OK;
+    } else {
+        CU(ctx->win_counts.ensure(rd->n_reads * sizeof(uint32_t)));
+        CU(ctx->rec_off.ensure((rd->n_reads + 1) * sizeof(uint64_t)));
+        CU(ctx->scan_scratch.ensure(group_scan_scratch_bytes(rd->n_reads)));
+        CU(cudaMemsetAsync(&dm->reads.max_len, 0, sizeof(unsigned int), st));
+        if (rd->max_read_len == 0) {
+            max_len_kernel<<<(unsigned)((rd->n_reads + 255) / 256), 256, 0, st>>>(rd->lens, rd->n_reads, &dm->reads.max_len);
+            (*launches)++;
+        }
+        *launches += launch_count_windows(reads_view(rd), K, ctx->win_counts.as<uint32_t>(), st);
+        *launches += exclusive_scan<uint64_t, WinCountIn>(WinCountIn{ctx->win_counts.as<uint32_t>()}, ctx->rec_off.as<uint64_t>(), rd->n_reads,
+                                                          ctx->scan_scratch.as<uint64_t>(),
+                                                          reinterpret_cast<uint64_t *>(&dm->reads.total_windows), st);
+        CU(read_back(ctx, &Misc::reads, st));
+        *n_inst = hm->reads.total_windows;
+        *max_len = rd->max_read_len ? rd->max_read_len : hm->reads.max_len;
     }
-    if (!rd->lens) return fail(ctx, GBIN_E_INVALID_ARG, "ragged reads need lens");
-    ReadsView rv{reinterpret_cast<const uint8_t *>(rd->data), rd->data_bytes, rd->n_reads, rd->stride, rd->read_len, rd->starts, rd->lens};
-    CU(ctx->win_counts.ensure(rd->n_reads * sizeof(uint32_t)));
-    CU(ctx->rec_off.ensure((rd->n_reads + 1) * sizeof(uint64_t)));
-    CU(ctx->scan_scratch.ensure(group_scan_scratch_bytes(rd->n_reads)));
-    CU(cudaMemsetAsync(&dm->reads.max_len, 0, sizeof(unsigned int), st));
-    if (rd->max_read_len == 0) {
-        max_len_kernel<<<(unsigned)((rd->n_reads + 255) / 256), 256, 0, st>>>(rd->lens, rd->n_reads, &dm->reads.max_len);
-        (*launches)++;
-    }
-    *launches += launch_count_windows(rv, K, ctx->win_counts.as<uint32_t>(), st);
-    *launches += exclusive_scan<uint64_t, WinCountIn>(WinCountIn{ctx->win_counts.as<uint32_t>()}, ctx->rec_off.as<uint64_t>(), rd->n_reads,
-                                                      ctx->scan_scratch.as<uint64_t>(),
-                                                      reinterpret_cast<uint64_t *>(&dm->reads.total_windows), st);
-    CU(read_back(ctx, &Misc::reads, st));
-    *n_inst = hm->reads.total_windows;
-    *max_len = rd->max_read_len ? rd->max_read_len : hm->reads.max_len;
+    if (*max_len > gbin_max_read_len()) return fail(ctx, GBIN_E_TOO_LARGE, "read length %u exceeds the limit of %u bases", *max_len, gbin_max_read_len());
     return GBIN_OK;
 }
 
 int run_scan(gbin_ctx *ctx, const gbin_reads *rd, uint32_t arrival_base, void *d_records, uint32_t max_len, cudaStream_t st, int *launches) {
     Misc *dm = ctx->misc.as<Misc>();
-    ReadsView rv{reinterpret_cast<const uint8_t *>(rd->data), rd->data_bytes, rd->n_reads, rd->stride, rd->read_len, rd->starts, rd->lens};
     CU(cudaMemsetAsync(&dm->grp.bad_bases, 0, sizeof(unsigned long long), st));
     const bool on = ctx->prof.begin(KK_SCAN, st);
-    const int ls = launch_scan_reads(rv, rd->starts ? ctx->rec_off.as<uint64_t>() : nullptr, ctx->cfg.kmer_size, ctx->cfg.mmer_size, ctx->KW,
+    const int ls = launch_scan_reads(reads_view(rd), rd->starts ? ctx->rec_off.as<uint64_t>() : nullptr, ctx->cfg.kmer_size, ctx->cfg.mmer_size, ctx->KW,
                                      arrival_base, max_len ? max_len : 1, d_records, &dm->grp.bad_bases, ctx->sm_count, st);
     ctx->prof.end(on, ls < 0 ? 0 : ls, st);
     if (ls < 0) return fail(ctx, GBIN_E_TOO_LARGE, "a read of %u bases does not fit the scan kernel's shared memory (limit %u bases)", max_len, gbin_max_read_len());
@@ -519,7 +600,6 @@ int run_skr_scan(gbin_ctx *ctx, const gbin_reads *rd, uint64_t n, uint32_t max_l
     const int NW = K <= 32 ? 8 : 12;
     Misc *dm = ctx->misc.as<Misc>();
     Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
-    ReadsView rv{reinterpret_cast<const uint8_t *>(rd->data), rd->data_bytes, rd->n_reads, rd->stride, rd->read_len, rd->starts, rd->lens};
     uint64_t cap = ext ? ext_cap : n / 4 + rd->n_reads + 1024;
     if (!ext && cap > n) cap = n;
     uint64_t n_skr = 0;
@@ -539,7 +619,7 @@ int run_skr_scan(gbin_ctx *ctx, const gbin_reads *rd, uint64_t n, uint32_t max_l
                 CU(cudaStreamWaitEvent(st, ctx->ev_feed[c], 0));
                 if (c + 1 == chunks) CU(cudaEventRecord(ctx->ev[EV_READS_ON_DEVICE], st));  // every byte of the reads is on the device
             }
-            const int l1 = launch_skr_scan(rv, r0, r1, K, M, arrival_base, max_len, ext ? ext : ctx->skr_a.p, cap, ctx->tile_state.as<unsigned long long>(),
+            const int l1 = launch_skr_scan(reads_view(rd), r0, r1, K, M, arrival_base, max_len, ext ? ext : ctx->skr_a.p, cap, ctx->tile_state.as<unsigned long long>(),
                                            &dm->skr_ticket, dm->skr_counters, ctx->sm_count, st);
             if (l1 < 0) {  // reads too long for the shared memory of this kernel: the caller uses the instance-record scan
                 if (feed && attempt == 0) CU(cudaStreamSynchronize(ctx->st_h2d));
@@ -1017,7 +1097,6 @@ int bin_device_impl(gbin_ctx *ctx, const gbin_reads *rd, cudaStream_t st, gbin_t
     uint32_t max_len = 0;
     int rc = plan_reads(ctx, rd, st, &n, &max_len, launches);
     if (rc) return rc;
-    if (max_len > gbin_max_read_len()) return fail(ctx, GBIN_E_TOO_LARGE, "read length %u exceeds the limit of %u bases", max_len, gbin_max_read_len());
     if (ctx->pipeline < 3 && n >= (1ull << 32) - 8192)
         return fail(ctx, GBIN_E_TOO_LARGE, "%llu k-mer instances in one batch (pipelines 1 and 2 hold 2^32; pipeline 3 works in passes)", (unsigned long long)n);
     const bool v2 = ctx->pipeline >= 2 && n != 0 && (ctx->pipeline >= 3 || n < (1ull << 31));
@@ -1301,12 +1380,14 @@ const char *gbin_kernel_kind_name(int kind) {
 
 int gbin_bin_reads_device(gbin_ctx *ctx, const gbin_reads *reads, void *stream, gbin_table *out) {
     if (!ctx || !reads || !out) return GBIN_E_INVALID_ARG;
+    int rc = check_reads(ctx, reads, false);
+    if (rc) return rc;
     cudaStream_t st;
     CU(begin_call(ctx, stream, &st));
     int launches = 0;
     CU(cudaEventRecord(ctx->ev[EV_START], st));
     CU(cudaEventRecord(ctx->ev[EV_READS_ON_DEVICE], st));
-    int rc = bin_device_impl(ctx, reads, st, out, &launches);
+    rc = bin_device_impl(ctx, reads, st, out, &launches);
     if (rc) return rc;
     CU(cudaStreamSynchronize(st));
     finish_timings(ctx, launches, false);
@@ -1350,62 +1431,15 @@ static int table_to_pinned(gbin_ctx *ctx, const gbin_table &dev, HostSink *sink,
     return GBIN_OK;
 }
 
-int gbin_bin_reads_host(gbin_ctx *ctx, const gbin_reads *reads, gbin_table *out) {
-    if (!ctx || !reads || !out) return GBIN_E_INVALID_ARG;
-    cudaStream_t st;
-    CU(begin_call(ctx, nullptr, &st));
-    int launches = 0;
-    gbin_reads d = *reads;
-    HostFeed feed{};
-    bool use_feed = false;
-    CU(cudaEventRecord(ctx->ev[EV_START], st));
-    if (reads->n_reads) {
-        if (!reads->data || reads->data_bytes == 0) return fail(ctx, GBIN_E_INVALID_ARG, "host reads need data and data_bytes");
-        CU(ctx->d_reads.ensure(reads->data_bytes + 64));
-        d.data = ctx->d_reads.as<char>();
-        if (!reads->starts && reads->stride >= reads->read_len && (reads->n_reads - 1) * reads->stride + reads->read_len <= reads->data_bytes) {
-            // fixed stride: read ranges are byte ranges, so the copy is left to the scan stage, which overlaps it with the scan
-            feed = HostFeed{reads->data, ctx->d_reads.as<char>(), reads->data_bytes, ctx->host_chunks};
-            if (reads->n_reads < 4096u * (uint64_t)feed.chunks) feed.chunks = 1;
-            use_feed = true;
-            CU(cudaStreamWaitEvent(ctx->st_h2d, ctx->ev[EV_START], 0));
-        } else {
-            CU(cudaMemcpyAsync(ctx->d_reads.p, reads->data, reads->data_bytes, cudaMemcpyHostToDevice, st));
-        }
-        if (reads->starts) {
-            if (!reads->lens) return fail(ctx, GBIN_E_INVALID_ARG, "ragged reads need lens");
-            CU(ctx->d_starts.ensure(reads->n_reads * sizeof(uint64_t)));
-            CU(ctx->d_lens.ensure(reads->n_reads * sizeof(uint32_t)));
-            CU(cudaMemcpyAsync(ctx->d_starts.p, reads->starts, reads->n_reads * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-            CU(cudaMemcpyAsync(ctx->d_lens.p, reads->lens, reads->n_reads * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
-            d.starts = ctx->d_starts.as<uint64_t>();
-            d.lens = ctx->d_lens.as<uint32_t>();
-            if (d.max_read_len == 0) {  // known on the host: spare the device reduction
-                uint32_t mx = 0;
-                for (uint64_t i = 0; i < reads->n_reads; i++) {
-                    if (reads->lens[i] > mx) mx = reads->lens[i];
-                    if (reads->data_bytes && reads->starts[i] + reads->lens[i] > reads->data_bytes)
-                        return fail(ctx, GBIN_E_INVALID_ARG, "read %llu exceeds data_bytes", (unsigned long long)i);
-                }
-                d.max_read_len = mx ? mx : 1;
-            }
-        }
-        if (reads->read_ids) {
-            CU(ctx->d_ids.ensure(reads->n_reads * sizeof(int32_t)));
-            CU(cudaMemcpyAsync(ctx->d_ids.p, reads->read_ids, reads->n_reads * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-            d.read_ids = ctx->d_ids.as<int32_t>();
-        }
-    }
-    if (!use_feed) CU(cudaEventRecord(ctx->ev[EV_READS_ON_DEVICE], st));
-    HostSink sink = host_sink(ctx);
-    gbin_table dev;
-    int rc = bin_device_impl(ctx, &d, st, &dev, &launches, use_feed ? &feed : nullptr, &sink);
+// The end of a host call, after `rc` from its device stage: on success the table goes to the pinned arenas and the call's timings are
+// taken; on failure the copy streams are drained, so that no copy into or out of the context's buffers outlives the call.
+static int finish_host_call(gbin_ctx *ctx, int rc, const gbin_table &dev, HostSink *sink, cudaStream_t st, int launches, gbin_table *out) {
     if (rc) {
         cudaStreamSynchronize(ctx->st_h2d);
         cudaStreamSynchronize(ctx->st_d2h);
         return rc;
     }
-    rc = table_to_pinned(ctx, dev, &sink, st, out);
+    rc = table_to_pinned(ctx, dev, sink, st, out);
     if (rc) return rc;
     CU(cudaEventRecord(ctx->ev[EV_TABLE_ON_HOST], st));
     CU(cudaStreamSynchronize(st));
@@ -1414,36 +1448,63 @@ int gbin_bin_reads_host(gbin_ctx *ctx, const gbin_reads *reads, gbin_table *out)
     return GBIN_OK;
 }
 
+int gbin_bin_reads_host(gbin_ctx *ctx, const gbin_reads *reads, gbin_table *out) {
+    if (!ctx || !reads || !out) return GBIN_E_INVALID_ARG;
+    uint32_t max_len = 0;
+    int rc = check_reads(ctx, reads, true, &max_len);
+    if (rc) return rc;
+    cudaStream_t st;
+    CU(begin_call(ctx, nullptr, &st));
+    int launches = 0;
+    const uint64_t n = reads->n_reads;
+    gbin_reads d = *reads;
+    HostFeed feed{};
+    const bool use_feed = n && !reads->starts;
+    CU(cudaEventRecord(ctx->ev[EV_START], st));
+    if (use_feed) {
+        // fixed stride: read ranges are byte ranges, so the copy is left to the scan stage, which overlaps it with the scan
+        CU(ctx->stage[0].data.ensure(reads->data_bytes + 64));
+        d.data = ctx->stage[0].data.as<char>();
+        feed = HostFeed{reads->data, ctx->stage[0].data.as<char>(), reads->data_bytes, ctx->host_chunks};
+        if (n < 4096u * (uint64_t)feed.chunks) feed.chunks = 1;
+        CU(cudaStreamWaitEvent(ctx->st_h2d, ctx->ev[EV_START], 0));
+    } else if (n) {  // ragged: the whole buffer, and the longest read known on the host spares the device reduction
+        const ReadRange all{0, n, 0, reads->data_bytes, reads->max_read_len ? reads->max_read_len : (max_len ? max_len : 1)};
+        if ((rc = stage_host_reads(ctx, reads, all, 0, st, &d))) return rc;
+    }
+    if (n && reads->read_ids) {
+        CU(ctx->d_ids.ensure(n * sizeof(int32_t)));
+        CU(cudaMemcpyAsync(ctx->d_ids.p, reads->read_ids, n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+        d.read_ids = ctx->d_ids.as<int32_t>();
+    }
+    if (!use_feed) CU(cudaEventRecord(ctx->ev[EV_READS_ON_DEVICE], st));
+    HostSink sink = host_sink(ctx);
+    gbin_table dev;
+    rc = bin_device_impl(ctx, &d, st, &dev, &launches, use_feed ? &feed : nullptr, &sink);
+    return finish_host_call(ctx, rc, dev, &sink, st, launches, out);
+}
+
 // ---------------------------------------------------------------- the table in owner parts, one part per call
 
 namespace {
-// A chunk of a part call: reads [r0, r1), which span bytes [b0, b1) of reads->data.
-struct PartChunk {
-    uint64_t r0, r1, b0, b1;
-    uint32_t max_len;  // 0: not known on the host (plan_reads finds it)
-};
-
 // Cuts the reads into chunks of whole reads whose byte span is at most ctx->part_chunk_bytes, with at least one read each.
 // Fixed-stride reads: contiguous byte ranges.  Ragged reads in host memory: the span [min start, max end) of the chunk's reads, which
 // is copied whole and exceeds the budget only for a single read longer than it (the chunk buffer then grows to fit).  Reads laid out
 // out of order make more, shorter chunks.
 // Ragged reads in device memory are scanned where they are, so they are cut by read count, at the mean bytes per read.
-int plan_part_chunks(gbin_ctx *ctx, const gbin_reads *rd, bool on_host, std::vector<PartChunk> *out) {
+std::vector<ReadRange> plan_part_chunks(const gbin_ctx *ctx, const gbin_reads *rd, bool on_host) {
     const uint64_t n = rd->n_reads, budget = ctx->part_chunk_bytes;
-    out->clear();
-    if (n == 0) return GBIN_OK;
+    std::vector<ReadRange> out;
+    if (n == 0) return out;
     if (!rd->starts || !on_host) {
         const uint64_t per_read = rd->starts ? rd->data_bytes / n + 1 : rd->stride;
         const uint64_t per = per_read == 0 ? n : (budget / per_read ? budget / per_read : 1);
         for (uint64_t r0 = 0; r0 < n; r0 += per) {
             const uint64_t r1 = n - r0 > per ? r0 + per : n;
-            if (rd->starts) out->push_back({r0, r1, 0, rd->data_bytes, rd->max_read_len});
-            else out->push_back({r0, r1, r0 * rd->stride, (r1 - 1) * rd->stride + rd->read_len, rd->read_len});
+            out.push_back(rd->starts ? ReadRange{r0, r1, 0, rd->data_bytes, rd->max_read_len} : read_range(rd, r0, r1));
         }
-        return GBIN_OK;
+        return out;
     }
-    for (uint64_t i = 0; i < n; i++)
-        if (rd->starts[i] + rd->lens[i] > rd->data_bytes) return fail(ctx, GBIN_E_INVALID_ARG, "read %llu exceeds data_bytes", (unsigned long long)i);
     for (uint64_t r0 = 0, r1; r0 < n; r0 = r1) {
         uint64_t lo = rd->starts[r0], hi = lo + rd->lens[r0];
         uint32_t ml = rd->lens[r0];
@@ -1455,16 +1516,16 @@ int plan_part_chunks(gbin_ctx *ctx, const gbin_reads *rd, bool on_host, std::vec
             hi = nhi;
             if (rd->lens[r1] > ml) ml = rd->lens[r1];
         }
-        out->push_back({r0, r1, lo, hi, ml ? ml : 1});
+        out.push_back({r0, r1, lo, hi, ml ? ml : 1});
     }
-    return GBIN_OK;
+    return out;
 }
 
 // Streams every chunk through the device and keeps the records of part `part` in ctx->part_rec, in arrival order: super-k-mer
 // records, or instance records when `inst`.  Host form: chunk c is copied into slot c & 1 on the copy stream while chunk c - 1 is
 // scanned; the slot's previous chunk has been scanned and selected by then (the host waited for both).  *too_long: the
 // super-k-mer scan cannot hold these reads, nothing was selected.  *scan_ms / *h2d_ms: scan + select / copy time summed over chunks.
-int scan_select_part(gbin_ctx *ctx, const gbin_reads *rd, bool on_host, const std::vector<PartChunk> &chunks, uint32_t part, uint32_t n_parts,
+int scan_select_part(gbin_ctx *ctx, const gbin_reads *rd, bool on_host, const std::vector<ReadRange> &chunks, uint32_t part, uint32_t n_parts,
                      bool inst, cudaStream_t st, int *launches, uint64_t *n_sel, uint64_t *n_sel_inst, bool *too_long, float *scan_ms, float *h2d_ms) {
     const int words = inst ? 2 * ctx->KW + 2 : (ctx->cfg.kmer_size <= 32 ? 8 : 12);
     const size_t rb = 4u * (size_t)words;
@@ -1473,21 +1534,11 @@ int scan_select_part(gbin_ctx *ctx, const gbin_reads *rd, bool on_host, const st
     *n_sel = *n_sel_inst = 0;
     *too_long = false;
     CU(cudaMemsetAsync(dm->part_sel, 0, sizeof dm->part_sel, st));
-    std::vector<uint64_t> rebased[2];  // host staging of a slot's starts, relative to its chunk's first byte
+    gbin_reads staged[2];  // the chunks in the two staging slots
     auto copy_in = [&](size_t c) -> int {
-        const PartChunk &k = chunks[c];
         const int s = (int)(c & 1);
-        CU(ctx->part_data[s].ensure(k.b1 - k.b0 + 64));
         CU(cudaEventRecord(ctx->ev_part_h2d[2 * s], ctx->st_h2d));
-        if (k.b1 > k.b0) CU(cudaMemcpyAsync(ctx->part_data[s].p, rd->data + k.b0, k.b1 - k.b0, cudaMemcpyHostToDevice, ctx->st_h2d));
-        if (rd->starts) {
-            const uint64_t m = k.r1 - k.r0;
-            CU(ctx->part_meta[s].ensure(m * (sizeof(uint64_t) + sizeof(uint32_t)) + 16));
-            rebased[s].resize(m);
-            for (uint64_t i = 0; i < m; i++) rebased[s][i] = rd->starts[k.r0 + i] - k.b0;
-            CU(cudaMemcpyAsync(ctx->part_meta[s].p, rebased[s].data(), m * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->st_h2d));
-            CU(cudaMemcpyAsync(ctx->part_meta[s].as<char>() + m * sizeof(uint64_t), rd->lens + k.r0, m * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->st_h2d));
-        }
+        if (const int rc = stage_host_reads(ctx, rd, chunks[c], s, ctx->st_h2d, &staged[s])) return rc;
         CU(cudaEventRecord(ctx->ev_part_h2d[2 * s + 1], ctx->st_h2d));
         return GBIN_OK;
     };
@@ -1498,7 +1549,7 @@ int scan_select_part(gbin_ctx *ctx, const gbin_reads *rd, bool on_host, const st
     };
     int rc = (on_host && !chunks.empty()) ? copy_in(0) : GBIN_OK;
     for (size_t c = 0; !rc && c < chunks.size(); c++) {
-        const PartChunk &k = chunks[c];
+        const ReadRange &k = chunks[c];
         const int s = (int)(c & 1);
         if (on_host && c + 1 < chunks.size() && (rc = copy_in(c + 1))) return rc;
         gbin_reads v = *rd;  // the chunk as a batch of its own, scanned with arrival_base = its first read
@@ -1506,12 +1557,7 @@ int scan_select_part(gbin_ctx *ctx, const gbin_reads *rd, bool on_host, const st
         v.read_ids = nullptr;
         v.max_read_len = k.max_len;
         if (on_host) {
-            v.data = ctx->part_data[s].as<char>();
-            v.data_bytes = k.b1 - k.b0;
-            if (rd->starts) {
-                v.starts = ctx->part_meta[s].as<uint64_t>();
-                v.lens = reinterpret_cast<const uint32_t *>(ctx->part_meta[s].as<char>() + v.n_reads * sizeof(uint64_t));
-            }
+            v = staged[s];
             CU(cudaStreamWaitEvent(st, ctx->ev_part_h2d[2 * s + 1], 0));
         } else if (rd->starts) {
             v.starts = rd->starts + k.r0;
@@ -1524,7 +1570,6 @@ int scan_select_part(gbin_ctx *ctx, const gbin_reads *rd, bool on_host, const st
         uint64_t n_c = 0, n_src = 0;
         uint32_t max_len = 0;
         if ((rc = plan_reads(ctx, &v, st, &n_c, &max_len, launches))) return rc;
-        if (max_len > gbin_max_read_len()) return fail(ctx, GBIN_E_TOO_LARGE, "read length %u exceeds the limit of %u bases", max_len, gbin_max_read_len());
         const void *src = nullptr;
         if (n_c && inst) {
             CU(ctx->rec_b.ensure((n_c + 1) * rb));
@@ -1577,17 +1622,7 @@ int bin_part_impl(gbin_ctx *ctx, const gbin_reads *rd, bool on_host, uint32_t pa
                   int *launches, float *scan_ms, float *h2d_ms) {
     if (n_parts == 0 || n_parts > 65536 || part >= n_parts) return fail(ctx, GBIN_E_INVALID_ARG, "part %u of %u parts (need part < n_parts <= 65536)", part, n_parts);
     const uint64_t n = rd->n_reads;
-    if (n >= (1ull << 32)) return fail(ctx, GBIN_E_TOO_LARGE, "more than 2^32-1 reads in one batch");
-    if (n) {
-        if (!rd->data || (on_host && rd->data_bytes == 0)) return fail(ctx, GBIN_E_INVALID_ARG, "reads need data and data_bytes");
-        if (rd->starts && !rd->lens) return fail(ctx, GBIN_E_INVALID_ARG, "ragged reads need lens");
-        if (!rd->starts && rd->stride < rd->read_len) return fail(ctx, GBIN_E_INVALID_ARG, "stride < read_len");
-        if (!rd->starts && rd->data_bytes && (n - 1) * rd->stride + rd->read_len > rd->data_bytes)
-            return fail(ctx, GBIN_E_INVALID_ARG, "fixed-stride reads exceed data_bytes");
-    }
-    std::vector<PartChunk> chunks;
-    int rc = plan_part_chunks(ctx, rd, on_host, &chunks);
-    if (rc) return rc;
+    const std::vector<ReadRange> chunks = plan_part_chunks(ctx, rd, on_host);
     const int32_t *d_ids = rd->read_ids;  // looked up by arrival = index over all the reads
     if (on_host && rd->read_ids && n) {
         CU(ctx->d_ids.ensure(n * sizeof(int32_t)));
@@ -1598,7 +1633,7 @@ int bin_part_impl(gbin_ctx *ctx, const gbin_reads *rd, bool on_host, uint32_t pa
     for (;;) {
         uint64_t n_sel = 0, n_sel_inst = 0;
         bool too_long = false;
-        rc = scan_select_part(ctx, rd, on_host, chunks, part, n_parts, inst, st, launches, &n_sel, &n_sel_inst, &too_long, scan_ms, h2d_ms);
+        int rc = scan_select_part(ctx, rd, on_host, chunks, part, n_parts, inst, st, launches, &n_sel, &n_sel_inst, &too_long, scan_ms, h2d_ms);
         CU(cudaStreamSynchronize(ctx->st_h2d));  // a copy into a chunk buffer may still be in flight when the loop ended early
         if (rc) return rc;
         if (too_long) {
@@ -1652,6 +1687,8 @@ constexpr double PART_BYTES_PER_INSTANCE = 58.0, PART_SKEW = 1.05, PART_BYTES_PE
 
 int gbin_bin_reads_host_part(gbin_ctx *ctx, const gbin_reads *reads, uint32_t part, uint32_t n_parts, gbin_table *out) {
     if (!ctx || !reads || !out) return GBIN_E_INVALID_ARG;
+    int rc = check_reads(ctx, reads, true);
+    if (rc) return rc;
     cudaStream_t st;
     CU(begin_call(ctx, nullptr, &st));
     int launches = 0;
@@ -1659,18 +1696,8 @@ int gbin_bin_reads_host_part(gbin_ctx *ctx, const gbin_reads *reads, uint32_t pa
     CU(cudaEventRecord(ctx->ev[EV_START], st));
     HostSink sink = host_sink(ctx);
     gbin_table dev;
-    int rc = bin_part_impl(ctx, reads, true, part, n_parts, st, &sink, &dev, &launches, &scan_ms, &h2d_ms);
-    if (rc) {
-        cudaStreamSynchronize(ctx->st_h2d);
-        cudaStreamSynchronize(ctx->st_d2h);
-        return rc;
-    }
-    rc = table_to_pinned(ctx, dev, &sink, st, out);
-    if (rc) return rc;
-    CU(cudaEventRecord(ctx->ev[EV_TABLE_ON_HOST], st));
-    CU(cudaStreamSynchronize(st));
-    CU(cudaStreamSynchronize(ctx->st_d2h));
-    finish_timings(ctx, launches, true);
+    rc = bin_part_impl(ctx, reads, true, part, n_parts, st, &sink, &dev, &launches, &scan_ms, &h2d_ms);
+    if ((rc = finish_host_call(ctx, rc, dev, &sink, st, launches, out))) return rc;
     ctx->tm.h2d_ms = h2d_ms;
     ctx->tm.scan_ms = scan_ms;
     return GBIN_OK;
@@ -1678,12 +1705,14 @@ int gbin_bin_reads_host_part(gbin_ctx *ctx, const gbin_reads *reads, uint32_t pa
 
 int gbin_bin_reads_device_part(gbin_ctx *ctx, const gbin_reads *reads, uint32_t part, uint32_t n_parts, void *stream, gbin_table *out) {
     if (!ctx || !reads || !out) return GBIN_E_INVALID_ARG;
+    int rc = check_reads(ctx, reads, false);
+    if (rc) return rc;
     cudaStream_t st;
     CU(begin_call(ctx, stream, &st));
     int launches = 0;
     float scan_ms = 0.f, h2d_ms = 0.f;
     CU(cudaEventRecord(ctx->ev[EV_START], st));
-    int rc = bin_part_impl(ctx, reads, false, part, n_parts, st, nullptr, out, &launches, &scan_ms, &h2d_ms);
+    rc = bin_part_impl(ctx, reads, false, part, n_parts, st, nullptr, out, &launches, &scan_ms, &h2d_ms);
     if (rc) return rc;
     CU(cudaStreamSynchronize(st));
     finish_timings(ctx, launches, false);
@@ -1754,14 +1783,14 @@ int split_reads_impl(gbin_ctx *ctx, const char *d_data, uint64_t size, int read_
     CU(cudaGetLastError());
     CU(read_back(ctx, &Misc::split_n_reads, st));
     const uint64_t n_reads = hm->split_n_reads;
-    CU(ctx->d_starts.ensure((n_reads + 1) * sizeof(uint64_t)));
-    CU(ctx->d_lens.ensure((n_reads + 1) * sizeof(uint32_t)));
-    *launches += split_emit_reads(ctx->split_nl.as<uint64_t>(), n_nl, size, cap, n_lines, ctx->split_base.as<uint32_t>(), ctx->d_starts.as<uint64_t>(),
-                                  ctx->d_lens.as<uint32_t>(), st);
+    CU(ctx->stage[0].meta.ensure((n_reads + 1) * (sizeof(uint64_t) + sizeof(uint32_t))));
+    uint64_t *starts = ctx->stage[0].meta.as<uint64_t>();
+    uint32_t *lens = reinterpret_cast<uint32_t *>(starts + n_reads + 1);
+    *launches += split_emit_reads(ctx->split_nl.as<uint64_t>(), n_nl, size, cap, n_lines, ctx->split_base.as<uint32_t>(), starts, lens, st);
     CU(cudaGetLastError());
     out->n_reads = n_reads;
-    out->starts = ctx->d_starts.as<uint64_t>();
-    out->lens = ctx->d_lens.as<uint32_t>();
+    out->starts = starts;
+    out->lens = lens;
     out->max_read_len = 0;  // the reads are at most cap - 1 bases long, usually far shorter: the binning call finds the real maximum on the device
     return GBIN_OK;
 }
@@ -1805,7 +1834,7 @@ int gbin_bin_file_host(gbin_ctx *ctx, const char *path, int read_length_define, 
     }
     const uint64_t size = (uint64_t)fsize;
     cudaError_t e = ctx->h_file.ensure(size + 64);
-    if (e == cudaSuccess) e = ctx->d_reads.ensure(size + 64);
+    if (e == cudaSuccess) e = ctx->stage[0].data.ensure(size + 64);
     if (e != cudaSuccess) {
         fclose(f);
         (void)cudaGetLastError();
@@ -1816,20 +1845,13 @@ int gbin_bin_file_host(gbin_ctx *ctx, const char *path, int read_length_define, 
     if (got != size) return fail(ctx, GBIN_E_IO, "short read on %s", path);
     int launches = 0;
     CU(cudaEventRecord(ctx->ev[EV_START], st));
-    if (size) CU(cudaMemcpyAsync(ctx->d_reads.p, ctx->h_file.p, size, cudaMemcpyHostToDevice, st));
+    if (size) CU(cudaMemcpyAsync(ctx->stage[0].data.p, ctx->h_file.p, size, cudaMemcpyHostToDevice, st));
     CU(cudaEventRecord(ctx->ev[EV_READS_ON_DEVICE], st));
     gbin_reads rd;
-    int rc = split_reads_impl(ctx, ctx->d_reads.as<char>(), size, read_length_define, st, &rd, &launches);
-    if (rc) return rc;
     gbin_table dev;
-    rc = bin_device_impl(ctx, &rd, st, &dev, &launches);
-    if (rc) return rc;
-    rc = table_to_pinned(ctx, dev, nullptr, st, out);
-    if (rc) return rc;
-    CU(cudaEventRecord(ctx->ev[EV_TABLE_ON_HOST], st));
-    CU(cudaStreamSynchronize(st));
-    finish_timings(ctx, launches, true);
-    return GBIN_OK;
+    int rc = split_reads_impl(ctx, ctx->stage[0].data.as<char>(), size, read_length_define, st, &rd, &launches);
+    if (!rc) rc = bin_device_impl(ctx, &rd, st, &dev, &launches);
+    return finish_host_call(ctx, rc, dev, nullptr, st, launches, out);
 }
 
 int gbin_table_digest(gbin_ctx *ctx, const gbin_table *t, void *stream, uint64_t *digest_out) {
@@ -1922,6 +1944,8 @@ int gbin_table_to_host(gbin_ctx *ctx, const gbin_table *dev, gbin_table *host) {
 
 int gbin_count_instances_device(gbin_ctx *ctx, const gbin_reads *reads, void *stream, uint64_t *n_out) {
     if (!ctx || !reads || !n_out) return GBIN_E_INVALID_ARG;
+    const int rc = check_reads(ctx, reads, false);
+    if (rc) return rc;
     cudaStream_t st;
     CU(begin_call(ctx, stream, &st));
     uint32_t max_len = 0;
@@ -1932,14 +1956,14 @@ int gbin_count_instances_device(gbin_ctx *ctx, const gbin_reads *reads, void *st
 int gbin_scan_reads_device(gbin_ctx *ctx, const gbin_reads *reads, uint32_t arrival_base, void *d_records, uint64_t capacity,
                            void *stream, uint64_t *n_out) {
     if (!ctx || !reads || !n_out) return GBIN_E_INVALID_ARG;
+    int rc = check_reads(ctx, reads, false);
+    if (rc) return rc;
     cudaStream_t st;
     CU(begin_call(ctx, stream, &st));
     uint64_t n = 0;
     uint32_t max_len = 0;
     int launches = 0;
-    int rc = plan_reads(ctx, reads, st, &n, &max_len, &launches);
-    if (rc) return rc;
-    if (max_len > GBIN_MAX_READ_LEN) return fail(ctx, GBIN_E_TOO_LARGE, "read length %u exceeds GBIN_MAX_READ_LEN", max_len);
+    if ((rc = plan_reads(ctx, reads, st, &n, &max_len, &launches))) return rc;
     if (n > capacity) return fail(ctx, GBIN_E_INVALID_ARG, "record buffer too small: need %llu", (unsigned long long)n);
     if (n && !d_records) return GBIN_E_INVALID_ARG;
     rc = run_scan(ctx, reads, arrival_base, d_records, max_len, st, &launches);
@@ -2105,14 +2129,14 @@ uint32_t gbin_skr_record_bytes(const gbin_ctx *ctx) { return ctx ? (ctx->cfg.kme
 int gbin_scan_skr_device(gbin_ctx *ctx, const gbin_reads *reads, uint32_t arrival_base, void *d_skr, uint64_t capacity, void *stream,
                          uint64_t *n_skr_out, uint64_t *n_instances_out) {
     if (!ctx || !reads || !n_skr_out) return GBIN_E_INVALID_ARG;
+    int rc = check_reads(ctx, reads, false);
+    if (rc) return rc;
     cudaStream_t st;
     CU(begin_call(ctx, stream, &st));
     uint64_t n = 0, n_skr = 0;
     uint32_t max_len = 0;
     int launches = 0;
-    int rc = plan_reads(ctx, reads, st, &n, &max_len, &launches);
-    if (rc) return rc;
-    if (max_len > GBIN_MAX_READ_LEN) return fail(ctx, GBIN_E_TOO_LARGE, "read length %u exceeds GBIN_MAX_READ_LEN", max_len);
+    if ((rc = plan_reads(ctx, reads, st, &n, &max_len, &launches))) return rc;
     if (n && !d_skr) return GBIN_E_INVALID_ARG;
     if (n) {
         rc = run_skr_scan(ctx, reads, n, max_len, arrival_base, d_skr, capacity, st, &n_skr, &launches);
@@ -2294,15 +2318,17 @@ gbin_ctx *gbin_multi_context(gbin_multi *m, int i) { return (m && i >= 0 && i < 
 // g's part of the table (its own m-mer buckets) in that context's pinned arena (ctx-owned, valid until the next call).
 int gbin_multi_bin_reads_host(gbin_multi *m, const gbin_reads *reads, gbin_table *tables_out) {
     if (!m || !reads || !tables_out) return GBIN_E_INVALID_ARG;
+    m->err[0] = 0;
+    if (const int rc = check_reads(m->ctx[0], reads, true)) {
+        snprintf(m->err, sizeof m->err, "%s", gbin_last_error(m->ctx[0]));
+        return rc;
+    }
     const int G = m->n;
     const uint64_t n = reads->n_reads;
-    if (n && !reads->data) return GBIN_E_INVALID_ARG;
-    if (reads->starts && !reads->lens) return GBIN_E_INVALID_ARG;
     std::vector<int> rcs(G, GBIN_OK);
     std::vector<uint64_t> n_skr(G, 0);
     std::vector<uint64_t> part_counts((size_t)G * G, 0);  // [g * G + o]: instance records GPU g holds for owner o (overflow redo)
     std::vector<std::string> errs(G);
-    m->err[0] = 0;
     auto work = [&](int g) {
         gbin_ctx *ctx = m->ctx[g];
         int &rc = rcs[g];
@@ -2314,55 +2340,26 @@ int gbin_multi_bin_reads_host(gbin_multi *m, const gbin_reads *reads, gbin_table
         cudaStream_t st = ctx->stream;
         const uint64_t lo = n * g / G, hi = n * (g + 1) / G, cnt = hi - lo;
         // ---- this GPU's shard to the device
-        gbin_reads d = *reads;
-        d.n_reads = cnt;
-        d.read_ids = nullptr;
+        gbin_reads d{};  // no reads when the shard is empty
+        const int r0 = cnt ? stage_host_reads(ctx, reads, read_range(reads, lo, hi), 0, st, &d) : GBIN_OK;
+        if (r0) failed(r0, "copying the shard to the device");
         cudaError_t e = cudaSuccess;
-        if (cnt) {
-            if (!reads->starts) {
-                const uint64_t b0 = lo * reads->stride, b1 = (hi - 1) * reads->stride + reads->read_len;
-                e = ctx->d_reads.ensure(b1 - b0 + 64);
-                if (e == cudaSuccess) e = cudaMemcpyAsync(ctx->d_reads.p, reads->data + b0, b1 - b0, cudaMemcpyHostToDevice, st);
-                d.data = ctx->d_reads.as<char>();
-                d.data_bytes = b1 - b0;
-            } else {
-                uint64_t b0 = ~0ull, b1 = 0;
-                for (uint64_t i = lo; i < hi; i++) {
-                    if (reads->starts[i] < b0) b0 = reads->starts[i];
-                    if (reads->starts[i] + reads->lens[i] > b1) b1 = reads->starts[i] + reads->lens[i];
-                }
-                if (b1 < b0) b0 = b1 = 0;
-                std::vector<uint64_t> st_rel(cnt);
-                for (uint64_t i = 0; i < cnt; i++) st_rel[i] = reads->starts[lo + i] - b0;
-                e = ctx->d_reads.ensure(b1 - b0 + 64);
-                if (e == cudaSuccess) e = ctx->d_starts.ensure(cnt * sizeof(uint64_t));
-                if (e == cudaSuccess) e = ctx->d_lens.ensure(cnt * sizeof(uint32_t));
-                if (e == cudaSuccess && b1 > b0) e = cudaMemcpyAsync(ctx->d_reads.p, reads->data + b0, b1 - b0, cudaMemcpyHostToDevice, st);
-                if (e == cudaSuccess) e = cudaMemcpyAsync(ctx->d_starts.p, st_rel.data(), cnt * sizeof(uint64_t), cudaMemcpyHostToDevice, st);
-                if (e == cudaSuccess) e = cudaMemcpyAsync(ctx->d_lens.p, reads->lens + lo, cnt * sizeof(uint32_t), cudaMemcpyHostToDevice, st);
-                if (e == cudaSuccess) e = cudaStreamSynchronize(st);  // st_rel goes out of scope
-                d.data = ctx->d_reads.as<char>();
-                d.data_bytes = b1 - b0;
-                d.starts = ctx->d_starts.as<uint64_t>();
-                d.lens = ctx->d_lens.as<uint32_t>();
-                d.max_read_len = 0;
-            }
-        }
         const int32_t *d_ids = nullptr;
-        if (e == cudaSuccess && reads->read_ids && n) {  // ids are looked up by global arrival index: every GPU holds the whole array
+        if (!rc && reads->read_ids && n) {  // ids are looked up by global arrival index: every GPU holds the whole array
             e = ctx->d_ids.ensure(n * sizeof(int32_t));
             if (e == cudaSuccess) e = cudaMemcpyAsync(ctx->d_ids.p, reads->read_ids, n * sizeof(int32_t), cudaMemcpyHostToDevice, st);
             d_ids = ctx->d_ids.as<int32_t>();
         }
         if (e != cudaSuccess) {
             (void)cudaGetLastError();
-            failed(e == cudaErrorMemoryAllocation ? GBIN_E_NOMEM : GBIN_E_CUDA, "copying the shard to the device");
+            failed(e == cudaErrorMemoryAllocation ? GBIN_E_NOMEM : GBIN_E_CUDA, "copying the read ids to the device");
         }
         // ---- scan into this context's record buffer (sized by an estimate, regrown to the exact need when short)
         uint64_t ninst = 0, cap = 0;
         if (!rc && cnt) {
             uint64_t est = 0;
-            rc = gbin_count_instances_device(ctx, &d, st, &est);
+            const int r1 = gbin_count_instances_device(ctx, &d, st, &est);
+            if (r1) failed(r1, "counting the instances");
             cap = est / 6 + cnt + 1024;
             const size_t rb = gbin_skr_record_bytes(ctx);
             for (int attempt = 0; !rc && attempt < 2; attempt++) {

@@ -87,7 +87,11 @@ typedef struct gbin_table {
 /* Reads are given either fixed-stride (starts == NULL: read i is reads[i*stride .. i*stride+read_len))
  * or ragged (read i is reads[starts[i] .. starts[i]+lens[i])).  Reads shorter than K yield nothing
  * but still own their arrival index / id, as in main (binning.c:1165).  read_ids == NULL means
- * id = id_base + i. Arrival order == index order. */
+ * id = id_base + i. Arrival order == index order.
+ * Every entry point that takes reads checks the descriptor before it copies or launches anything: data != NULL, n_reads < 2^32
+ * (else GBIN_E_TOO_LARGE), stride >= read_len and fixed-stride reads inside a non-zero data_bytes, lens given for ragged reads.
+ * The host entry points also need data_bytes != 0 and check every ragged read against it, and enforce a non-zero max_read_len as an
+ * upper bound on every lens[i]; ragged reads in device memory are trusted.  Any of these fails with GBIN_E_INVALID_ARG unless noted. */
 typedef struct gbin_reads {
     const char *data;       /* ASCII bases; host or device memory depending on the entry point */
     uint64_t data_bytes;    /* bytes addressable from data */
@@ -98,7 +102,7 @@ typedef struct gbin_reads {
     const uint64_t *starts; /* ragged form (NULL for fixed stride) */
     const uint32_t *lens;
     const int32_t *read_ids; /* optional explicit ids (what process_read's read_id argument carries) */
-    uint32_t max_read_len;  /* ragged form: upper bound on lens[] (0 = let the library find it) */
+    uint32_t max_read_len;  /* ragged form: upper bound on lens[] (0 = let the library find it; host entry points refuse a longer read) */
     uint32_t reserved;
 } gbin_reads;
 
@@ -267,7 +271,8 @@ void gbin_xchg_destroy(gbin_ctx *ctx);
  * part of the table GPU g owns: disjoint m-mer buckets, together the table of a single-GPU run (their digests add up to its digest).
  * When a shared-memory unit overflows on any GPU (one k-mer with more instances than a unit holds, e.g. homopolymer-rich reads), every
  * GPU redoes its shard in instance-record form (gbin_scan_reads_device, gbin_partition_records_device, a gather of every GPU's part
- * by its owner, gbin_group_records_device): same result. */
+ * by its owner, gbin_group_records_device): same result.  It refuses every descriptor gbin_bin_reads_host refuses, with the same
+ * codes, before any GPU starts. */
 typedef struct gbin_multi gbin_multi;
 int gbin_multi_create(const gbin_config *cfg, const int *devices, int n_devices, gbin_multi **out);
 void gbin_multi_destroy(gbin_multi *m);
