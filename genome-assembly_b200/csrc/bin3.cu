@@ -16,10 +16,12 @@
 //      of the flat table ONCE, at its final place.
 //   5. span_reorder_kernel: atoms that were split into d-rounds come out round by round; their (few) surviving k-mers
 //      are sorted and their id lists moved from the staging arrays to the final place.
-//   6. skr_emit_buckets (skr_group.cu): bucket directory; buckets that lost all k-mers vanish (binning.c:1136-1142).
+//   6. emit_bucket_directory (skr_group.cu): bucket directory; buckets that lost all k-mers vanish (binning.c:1136-1142).
+#include <vector>
+
 #include "bin3.cuh"
+#include "gbin_ctx.h"
 #include "gbin_device.cuh"
-#include "gbin_internal.h"
 #include "prefix_scan.cuh"
 
 namespace gbin {
@@ -81,7 +83,7 @@ __global__ void __launch_bounds__(256)
     if (threadIdx.x == 0 && s_real) atomicAdd(n_real, (unsigned long long)s_real);
 }
 
-int v3_make_entries(const void *skr, uint64_t n_rec, const KeyLayout &kl, uint64_t *ent, uint16_t *piece_info, unsigned long long *n_real_dev,
+static int v3_make_entries(const void *skr, uint64_t n_rec, const KeyLayout &kl, uint64_t *ent, uint16_t *piece_info, unsigned long long *n_real_dev,
                     cudaStream_t st) {
     cudaMemsetAsync(n_real_dev, 0, sizeof(unsigned long long), st);
     if (n_rec == 0) return 0;
@@ -121,7 +123,7 @@ __global__ void v3_run_totals_kernel(const uint64_t *__restrict__ total, uint64_
     *n_runs_out = (uint32_t)(t >> 32);
 }
 
-int v3_plan_runs(const uint64_t *ent, const uint16_t *sorted_info, uint64_t n_ent, uint32_t *inst_prefix, uint64_t *both64, uint32_t *run_start,
+static int v3_plan_runs(const uint64_t *ent, const uint16_t *sorted_info, uint64_t n_ent, uint32_t *inst_prefix, uint64_t *both64, uint32_t *run_start,
                  uint64_t *scratch64, uint32_t *n_inst_dev, uint32_t *n_runs_dev, cudaStream_t st) {
     if (n_ent == 0) {
         cudaMemsetAsync(n_inst_dev, 0, 4, st);
@@ -247,15 +249,6 @@ __global__ void __launch_bounds__(128)
         r = q;
     }
 }
-
-struct G3Counters {
-    unsigned long long distinct;
-    unsigned long long total_kmers, total_ids;
-    unsigned int overflow;
-    unsigned int n_units, n_spans;
-    unsigned int pad;
-    unsigned long long lsd_kmers, lsd_ids;  // surviving k-mers / ids of the spans that are put in order by the global sort
-};
 
 __global__ void v3_head_runs_kernel(const uint64_t *__restrict__ nunits, const uint64_t *__restrict__ base, uint64_t n_runs, uint32_t *__restrict__ head_run) {
     const uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -1293,13 +1286,11 @@ static Plan3 v3_plan_params(const KeyLayout &kl, int cap_i) {
     return pp;
 }
 
-uint64_t v3_max_units(uint64_t n_inst, uint64_t n_runs, int cap) {
+static uint64_t v3_max_units(uint64_t n_inst, uint64_t n_runs, int cap) {
     const uint64_t c = cap == 512 ? 512 : 1024;
     // a packed unit holds at least one atom; an atom in rounds holds more than cap instances and gets at most 2 * ceil(instances / cap) + 1 units
     return n_runs + 5 * (n_inst / c) + 16;
 }
-size_t v3_unit_bytes() { return sizeof(Unit3); }
-size_t v3_unit_out_bytes() { return sizeof(UnitOut3); }
 
 struct PtrIn64 {
     const uint64_t *p;
@@ -1307,7 +1298,7 @@ struct PtrIn64 {
 };
 
 // Units over the n_runs atoms.  nunits64 / base64: [n_runs + 1] u64 scratch each; atom3: [3 * n_runs] u32 scratch; spanlen: [n_runs] u32; head_run: [max_units].
-int v3_plan_units(const uint16_t *sorted_info, const uint64_t *ent, const KeyLayout &kl, int cap, const uint32_t *inst_prefix, const uint32_t *run_start, uint64_t n_runs,
+static int v3_plan_units(const uint16_t *sorted_info, const uint64_t *ent, const KeyLayout &kl, int cap, const uint32_t *inst_prefix, const uint32_t *run_start, uint64_t n_runs,
                   uint64_t *nunits64, uint64_t *base64, uint32_t *atom3, uint32_t *spanlen, uint32_t *head_run, void *scratch, void *units, uint64_t max_units,
                   void *gc_dev, uint32_t n_chunks, uint32_t *chunk_bounds, cudaStream_t st) {
     RunView3 rv{run_start, inst_prefix};
@@ -1334,26 +1325,39 @@ int v3_plan_units(const uint16_t *sorted_info, const uint64_t *ent, const KeyLay
 static int v3_group_units(int cap) { return cap == 512 ? G3_WARPS : G3_PAIRS; }
 static int v3_group_threads(int cap) { return v3_group_units(cap) * (cap == 512 ? UnitLayout<512, 1>::W : UnitLayout<1024, 1>::W) * 32; }
 
-size_t v3_group_smem_bytes(int KW, int cap) {
+static size_t v3_group_smem_bytes(int KW, int cap) {
     const size_t per_unit = cap == 512 ? (KW == 1 ? UnitLayout<512, 1>::BYTES : UnitLayout<512, 2>::BYTES)
                                        : (KW == 1 ? UnitLayout<1024, 1>::BYTES : UnitLayout<1024, 2>::BYTES);
     return per_unit * v3_group_units(cap);
 }
 
-int v3_group_launch(const void *skr, const uint64_t *ent, const void *units, const KeyLayout &kl, int cap, int cutoff, const int32_t *ids_by_arrival, int32_t id_base,
-                    const V3Out &o, uint64_t max_units, uint64_t *unit_excl, uint64_t *lsd_excl, void *scan_scratch, void *gc_dev, const V3Chunks &ch, const V3Lsd &lsd,
-                    bool finalize_only, int sm_count, KernelProf *prof, cudaStream_t st) {
-    const int KW = kl.K <= 32 ? 1 : 2;
+// The arrays of the global sort that puts long spans in order (rec_a and v3_lsd_aux), for `cap` k-mers; excl: the scan over long-span units.
+static G3Lsd v3_lsd_view(gbin_ctx *ctx, const uint64_t *excl, uint64_t cap) {
+    if (cap == 0) return G3Lsd{excl, nullptr, nullptr, nullptr, nullptr, nullptr, 0};
+    uint32_t *aux = ctx->v3_lsd_aux.as<uint32_t>();
+    return G3Lsd{excl, ctx->rec_a.p, aux, aux + (cap + 1), aux + 2 * (cap + 1), aux + 3 * (cap + 1), cap};
+}
+
+// The grouping of one pass as n_chunks launches over consecutive ranges of the unit list (chunk_bounds, from v3_plan_units), each
+// followed by its finalize.  After every chunk the totals {k-mers << 32 | ids} emitted up to its end are published (chunk_totals,
+// and lsd_totals for the k-mers handed to the global sort); with to_host they are copied to the pinned mirror and ev_chunk[c] is
+// recorded, so that the host can stream finished parts of the table.  In the hybrid layout the two grouping launches of a chunk run
+// side by side on the context's second stream.  lsd_cap: k-mers the arrays of the global sort for long spans hold (0: none).
+static int v3_group_launch(gbin_ctx *ctx, const void *skr, const uint64_t *ent, const KeyLayout &kl, int cutoff, const int32_t *ids_by_arrival, int32_t id_base,
+                           const G3Stage &stg, const G3Final &fin, uint64_t lsd_cap, uint64_t max_units, uint32_t n_chunks, bool to_host, bool finalize_only,
+                           cudaStream_t st) {
+    Misc *dm = ctx->misc.as<Misc>();
+    Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
+    const int KW = kl.K <= 32 ? 1 : 2, cap = ctx->v3_cap_eff, sm_count = ctx->sm_count;
     const size_t smem = v3_group_smem_bytes(KW, cap);
     const int threads = v3_group_threads(cap), threads_s = v3_group_threads(512);
-    cudaMemsetAsync(ch.tickets, 0, sizeof(uint32_t) * 2 * ch.n, st);
-    const uint32_t kdiv = cutoff >= 0 ? (uint32_t)cutoff + 1u : 1u;
-    G3Stage stg{o.stg_codes, o.stg_mmer, o.stg_loff, o.stg_ids, static_cast<UnitOut3 *>(o.unit_out), o.kmer_cap, o.id_cap, kdiv};
-    G3Final fin{o.kmer_codes, o.kmer_mmer, o.kmer_id_off, o.read_ids, o.id_off_base};
-    G3Lsd ls{lsd_excl, lsd.rec, lsd.src_off, lsd.cnt, lsd.fidx, lsd.nadj, lsd.cap};
-    G3Counters *gc = static_cast<G3Counters *>(gc_dev);
+    uint32_t *tickets = dm->v3_tickets, *bounds = dm->chunk_bounds;
+    cudaMemsetAsync(tickets, 0, sizeof(uint32_t) * 2 * n_chunks, st);
+    uint64_t *unit_excl = ctx->v3_unit_excl.as<uint64_t>(), *lsd_excl = unit_excl + max_units + 1;
+    const G3Lsd ls = v3_lsd_view(ctx, lsd_excl, lsd_cap);
+    G3Counters *gc = &dm->gc3;
     const uint32_t *sk = static_cast<const uint32_t *>(skr);
-    const Unit3 *un = static_cast<const Unit3 *>(units);
+    const Unit3 *un = ctx->units.as<Unit3>();
     const int per_sm = g3_ctas_per_sm(smem);
     const bool hybrid = v3_hybrid(kl, cap);
     const size_t smem_s = v3_group_smem_bytes(KW, 512);
@@ -1362,39 +1366,40 @@ int v3_group_launch(const void *skr, const uint64_t *ent, const void *units, con
     auto launch = [&](auto kern, auto kern_small, auto fin_kern) {
         cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (hybrid) cudaFuncSetAttribute(kern_small, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_s);
-        for (uint32_t c = 0; c < ch.n; c++) {
+        for (uint32_t c = 0; c < n_chunks; c++) {
             if (!finalize_only) {
-                bool on = prof && prof->begin(KK_SKR_GROUP, st);
+                bool on = ctx->prof.begin(KK_SKR_GROUP, st);
                 if (!hybrid) {
-                    kern<<<sm_count * per_sm, threads, smem, st>>>(sk, ent, un, kl, cutoff, ids_by_arrival, id_base, stg, gc, ch.bounds, c, ch.tickets, 0u);
+                    kern<<<sm_count * per_sm, threads, smem, st>>>(sk, ent, un, kl, cutoff, ids_by_arrival, id_base, stg, gc, bounds, c, tickets, 0u);
                 } else {
                     // side by side: the large-unit kernel goes first with as many CTAs as its shared memory lets an SM hold, the
                     // small-unit kernel's CTAs take what is left of every SM and, being persistent, the room the other kernel leaves when
                     // it runs out of units (its tail is covered)
-                    cudaEventRecord(ch.ev_fork, st);
-                    cudaStreamWaitEvent(ch.aux, ch.ev_fork, 0);
-                    kern<<<sm_count * per_sm, threads, smem, st>>>(sk, ent, un, kl, cutoff, ids_by_arrival, id_base, stg, gc, ch.bounds, c, ch.tickets, 2u);
-                    kern_small<<<sm_count * per_sm_s, threads_s, smem_s, ch.aux>>>(sk, ent, un, kl, cutoff, ids_by_arrival, id_base, stg, gc, ch.bounds, c, ch.tickets + ch.n, 1u);
-                    cudaEventRecord(ch.ev_join, ch.aux);
-                    cudaStreamWaitEvent(st, ch.ev_join, 0);
+                    cudaEventRecord(ctx->ev_fork, st);
+                    cudaStreamWaitEvent(ctx->st_aux, ctx->ev_fork, 0);
+                    kern<<<sm_count * per_sm, threads, smem, st>>>(sk, ent, un, kl, cutoff, ids_by_arrival, id_base, stg, gc, bounds, c, tickets, 2u);
+                    kern_small<<<sm_count * per_sm_s, threads_s, smem_s, ctx->st_aux>>>(sk, ent, un, kl, cutoff, ids_by_arrival, id_base, stg, gc, bounds, c, tickets + n_chunks, 1u);
+                    cudaEventRecord(ctx->ev_join, ctx->st_aux);
+                    cudaStreamWaitEvent(st, ctx->ev_join, 0);
                 }
-                if (prof) prof->end(on, hybrid ? 2 : 1, st);
+                ctx->prof.end(on, hybrid ? 2 : 1, st);
                 launches += hybrid ? 2 : 1;
             }
-            bool on = prof && prof->begin(KK_V3_SPAN, st);
-            int l = exclusive_scan<uint64_t, UnitSN>(UnitSN{stg.unit_out, ch.bounds, c}, unit_excl, max_units, static_cast<uint64_t *>(scan_scratch), ch.chunk_sum, st);
-            v3_chunk_total_kernel<<<1, 1, 0, st>>>(ch.chunk_sum, c, ch.totals_dev, gc, ch.n, 0);
-            l += exclusive_scan<uint64_t, UnitSNLong>(UnitSNLong{stg.unit_out, un, ch.bounds, c}, lsd_excl, max_units, static_cast<uint64_t *>(scan_scratch), ch.chunk_sum, st);
-            v3_chunk_total_kernel<<<1, 1, 0, st>>>(ch.chunk_sum, c, ch.lsd_totals_dev, gc, ch.n, 1);
+            bool on = ctx->prof.begin(KK_V3_SPAN, st);
+            uint64_t *scan_scratch = ctx->scan_scratch.as<uint64_t>(), *chunk_sum = &dm->v3_chunk_sum;
+            int l = exclusive_scan<uint64_t, UnitSN>(UnitSN{stg.unit_out, bounds, c}, unit_excl, max_units, scan_scratch, chunk_sum, st);
+            v3_chunk_total_kernel<<<1, 1, 0, st>>>(chunk_sum, c, dm->chunk_totals, gc, n_chunks, 0);
+            l += exclusive_scan<uint64_t, UnitSNLong>(UnitSNLong{stg.unit_out, un, bounds, c}, lsd_excl, max_units, scan_scratch, chunk_sum, st);
+            v3_chunk_total_kernel<<<1, 1, 0, st>>>(chunk_sum, c, dm->lsd_totals, gc, n_chunks, 1);
             // a second run (after the arrays of the global sort were allocated) only handles the long spans: the short-span merge is not idempotent
-            fin_kern<<<sm_count * 12, 128, 0, st>>>(un, unit_excl, ch.totals_dev, ch.lsd_totals_dev, stg, fin, ls, gc, ch.bounds, c, finalize_only);
-            if (prof) prof->end(on, l + 3, st);
+            fin_kern<<<sm_count * 12, 128, 0, st>>>(un, unit_excl, dm->chunk_totals, dm->lsd_totals, stg, fin, ls, gc, bounds, c, finalize_only);
+            ctx->prof.end(on, l + 3, st);
             launches += l + 3;
-            if (ch.totals_host) {
-                cudaMemcpyAsync(ch.totals_host + c, ch.totals_dev + c, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st);
-                cudaMemcpyAsync(ch.lsd_totals_host + c, ch.lsd_totals_dev + c, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st);
+            if (to_host) {
+                cudaMemcpyAsync(hm->chunk_totals + c, dm->chunk_totals + c, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st);
+                cudaMemcpyAsync(hm->lsd_totals + c, dm->lsd_totals + c, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st);
+                cudaEventRecord(ctx->ev_chunk[c], st);
             }
-            if (ch.done) cudaEventRecord(ch.done[c], st);
         }
     };
     // instances per lane in flight: 4 at capacity 1024, 2 at 512 (more warps per SM there: less need for instruction-level parallelism, smaller code)
@@ -1704,45 +1709,51 @@ static int v3_span_sort(void *rec_v, void *rec2_v, uint64_t n, uint32_t *work32,
     return l + 4;
 }
 
-// The long spans' k-mers (n records, appended by finalize3_kernel) are sorted by (m-mer, k-mer) — a permutation inside every span —
-// and then written, with their id lists, to the table.  rec_a / rec_b: Rec<KW> [n] each; dnew: [n + 1] u64.
-int v3_lsd_finish(const KeyLayout &kl, uint64_t n, void *rec_a, void *rec_b, void *radix_scratch, uint64_t *dnew, void *scan_scratch, const V3Out &o, const V3Lsd &lsd,
-                  int sm_count, KernelProf *prof, cudaStream_t st) {
-    if (n == 0) return 0;
-    const int KW = kl.K <= 32 ? 1 : 2;
+// The long spans' k-mers (n records, appended by finalize3_kernel to rec_a) are sorted by (m-mer, k-mer) — a permutation inside every
+// span — and then written, with their id lists, to the table.
+static int v3_lsd_finish(gbin_ctx *ctx, const KeyLayout &kl, uint64_t n, const G3Stage &stg, const G3Final &fin, uint64_t lsd_cap, cudaStream_t st,
+                         int *launches) {
+    if (n == 0) return GBIN_OK;
+    CU(ctx->radix_scratch.ensure(radix_scratch_bytes(n)));
+    CU(ctx->run_excl.ensure((n + 2) * 8));
+    CU(ctx->scan_scratch.ensure(group_scan_scratch_bytes(n + 1024)));
+    void *rec_a = ctx->rec_a.p, *rec_b = ctx->rec_b.p, *scan_scratch = ctx->scan_scratch.p;
+    uint64_t *dnew = ctx->run_excl.as<uint64_t>();  // [n + 1]
+    const int KW = kl.K <= 32 ? 1 : 2, sm_count = ctx->sm_count;
+    KernelProf *prof = &ctx->prof;
     bool in_b = false;
     int passes = 0;
     int l = 0;
     bool need_global = true;
     if (n < (1ull << 31)) {
         uint32_t *work32 = reinterpret_cast<uint32_t *>(dnew);  // [n + 2] u64 = [2 n + 4] u32; free until the list-length scan below
-        bool on = prof && prof->begin(KK_V3_SPAN, st);
+        bool on = prof->begin(KK_V3_SPAN, st);
         const int ls_ = KW == 1 ? v3_span_sort<1>(rec_a, rec_b, n, work32, scan_scratch, sm_count, st) : v3_span_sort<2>(rec_a, rec_b, n, work32, scan_scratch, sm_count, st);
-        if (prof) prof->end(on, ls_, st);
+        prof->end(on, ls_, st);
         l += ls_;
         uint32_t flag = 1;
         cudaMemcpyAsync(&flag, work32 + 2 * n + 3, sizeof flag, cudaMemcpyDeviceToHost, st);
         if (cudaStreamSynchronize(st) == cudaSuccess) need_global = flag != 0;
     }
-    if (need_global) l += radix_sort_records(rec_a, rec_b, n, KW, kl.K, kl.M, radix_scratch, &in_b, &passes, prof, st);
+    if (need_global) l += radix_sort_records(rec_a, rec_b, n, KW, kl.K, kl.M, ctx->radix_scratch.p, &in_b, &passes, prof, st);
     const void *sorted = in_b ? rec_b : rec_a;
-    G3Final fin{o.kmer_codes, o.kmer_mmer, o.kmer_id_off, o.read_ids, o.id_off_base};
-    G3Lsd ls{nullptr, nullptr, lsd.src_off, lsd.cnt, lsd.fidx, lsd.nadj, lsd.cap};
-    bool on = prof && prof->begin(KK_V3_SPAN, st);
+    const G3Lsd ls = v3_lsd_view(ctx, nullptr, lsd_cap);
+    bool on = prof->begin(KK_V3_SPAN, st);
     int l2 = 0;
     if (KW == 1) {
         const Rec<1> *r = static_cast<const Rec<1> *>(sorted);
-        l2 += exclusive_scan<uint64_t, LsdCnt<1>>(LsdCnt<1>{r, lsd.cnt}, dnew, n, static_cast<uint64_t *>(scan_scratch), nullptr, st);
+        l2 += exclusive_scan<uint64_t, LsdCnt<1>>(LsdCnt<1>{r, ls.cnt}, dnew, n, static_cast<uint64_t *>(scan_scratch), nullptr, st);
         lsd_place_kernel<1><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(r, n, dnew, ls, fin);
-        lsd_lists_kernel<1><<<(unsigned)((n * 8 + 255) / 256), 256, 0, st>>>(r, n, dnew, ls, o.stg_ids, fin);
+        lsd_lists_kernel<1><<<(unsigned)((n * 8 + 255) / 256), 256, 0, st>>>(r, n, dnew, ls, stg.ids, fin);
     } else {
         const Rec<2> *r = static_cast<const Rec<2> *>(sorted);
-        l2 += exclusive_scan<uint64_t, LsdCnt<2>>(LsdCnt<2>{r, lsd.cnt}, dnew, n, static_cast<uint64_t *>(scan_scratch), nullptr, st);
+        l2 += exclusive_scan<uint64_t, LsdCnt<2>>(LsdCnt<2>{r, ls.cnt}, dnew, n, static_cast<uint64_t *>(scan_scratch), nullptr, st);
         lsd_place_kernel<2><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(r, n, dnew, ls, fin);
-        lsd_lists_kernel<2><<<(unsigned)((n * 8 + 255) / 256), 256, 0, st>>>(r, n, dnew, ls, o.stg_ids, fin);
+        lsd_lists_kernel<2><<<(unsigned)((n * 8 + 255) / 256), 256, 0, st>>>(r, n, dnew, ls, stg.ids, fin);
     }
-    if (prof) prof->end(on, l2 + 2, st);
-    return l + l2 + 2;
+    prof->end(on, l2 + 2, st);
+    *launches += l + l2 + 2;
+    return GBIN_OK;
 }
 
 // ---- passes: a batch with more k-mer instances than 32-bit coordinates hold is grouped in several passes over consecutive
@@ -1773,18 +1784,6 @@ __global__ void pass_bounds_kernel(const uint64_t *__restrict__ ent, uint64_t n_
     while (b < n_ent && ((uint32_t)(ent[b] >> 32) >> mshift) == mm) b++;
     bounds[i] = b;
 }
-uint32_t v3_pass_tiles(uint64_t n_ent) { return (uint32_t)((n_ent + PASS_TILE - 1) / PASS_TILE); }
-uint32_t v3_pass_tile_entries() { return PASS_TILE; }
-int v3_pass_tile_sums(const uint16_t *sorted_info, uint64_t n_ent, unsigned long long *sums_dev, cudaStream_t st) {
-    if (n_ent == 0) return 0;
-    pass_tile_sums_kernel<<<v3_pass_tiles(n_ent), 256, 0, st>>>(sorted_info, n_ent, sums_dev);
-    return 1;
-}
-int v3_pass_bounds(const uint64_t *ent, uint64_t n_ent, int mshift, unsigned long long *bounds_dev, uint32_t n_bounds, cudaStream_t st) {
-    if (n_bounds == 0) return 0;
-    pass_bounds_kernel<<<(n_bounds + 63) / 64, 64, 0, st>>>(ent, n_ent, mshift, bounds_dev, n_bounds);
-    return 1;
-}
 
 // ---- how many different m-mer codes do the records hold?  (bitmap over the code space; decides the key layout)
 __global__ void mmer_bitmap_kernel(const uint32_t *__restrict__ skr, int skr_words, uint64_t n_rec, uint32_t *__restrict__ bitmap) {
@@ -1801,15 +1800,299 @@ __global__ void bitmap_count_kernel(const uint32_t *__restrict__ bitmap, uint64_
     for (int d = 16; d > 0; d >>= 1) c += __shfl_xor_sync(0xffffffffu, c, d);
     if ((threadIdx.x & 31) == 0 && c) atomicAdd(count, (unsigned long long)c);
 }
-size_t v3_mmer_bitmap_bytes(int M) { return ((size_t)1 << (2 * M)) / 8 + 64; }
-int v3_count_mmers(const void *skr, int skr_words, uint64_t n_rec, int M, uint32_t *bitmap, unsigned long long *count_dev, cudaStream_t st) {
+
+
+// ------------------------------------------------------------------ the pipeline
+
+// Key layout for this batch: explicit (gbin_set_tuning v3_nc = 1 | 2) or chosen from the mean m-mer bucket size (v3_nc = 0):
+// buckets that fit a unit need nothing but the m-mer code; larger ones are broken up by extending the key (bin3.cuh).
+static int v3_choose_layout(gbin_ctx *ctx, const void *skr, uint64_t n_skr, cudaStream_t st, KeyLayout *out, int *launches) {
+    const int K = ctx->cfg.kmer_size, M = ctx->cfg.mmer_size;
+    // Unit capacity: 1024 instances when whole m-mer buckets are units (fewer buckets straddle units), 512 when the key is
+    // extended or the k-mers are two words wide (twice the warps per SM: the grouping kernel is latency-bound; measured
+    // 17.1 -> 11.3 ms on a config-3 shaped batch, 13.4 -> 7.9 ms on a config-5 shaped one).
+    auto set_cap = [&](const KeyLayout &kl) { ctx->v3_cap_eff = ctx->v3_cap ? ctx->v3_cap : ((ctx->KW == 2 || kl.nc == 2) ? 512 : 1024); };
+    if (ctx->v3_nc != 0) {
+        *out = make_key_layout(K, M, ctx->v3_h, ctx->v3_nc);
+        set_cap(*out);
+        return GBIN_OK;
+    }
+    if (2 * M + 2 > 31 || M > 13 || n_skr == 0) {  // no room for a longer key / code space too large for the bitmap: plain m-mer keys
+        *out = make_key_layout(K, M, 0, 1);
+        set_cap(*out);
+        return GBIN_OK;
+    }
+    // the decision is kept for batches of similar size on this context
+    if (ctx->v3_auto_n && n_skr >= ctx->v3_auto_n / 2 && n_skr <= ctx->v3_auto_n * 2) {
+        *out = make_key_layout(K, M, ctx->v3_auto_h, ctx->v3_auto_nc);
+        set_cap(*out);
+        return GBIN_OK;
+    }
+    Misc *dm = ctx->misc.as<Misc>();
+    Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
+    // how many different m-mer codes do the records hold: a bitmap over the code space
     const uint64_t words = ((uint64_t)1 << (2 * M)) / 32;
+    CU(ctx->v3_bitmap.ensure(((size_t)1 << (2 * M)) / 8 + 64));
+    uint32_t *bitmap = ctx->v3_bitmap.as<uint32_t>();
     cudaMemsetAsync(bitmap, 0, words * 4, st);
-    cudaMemsetAsync(count_dev, 0, sizeof(unsigned long long), st);
-    if (n_rec == 0) return 0;
-    mmer_bitmap_kernel<<<(unsigned)((n_rec + 255) / 256), 256, 0, st>>>(static_cast<const uint32_t *>(skr), skr_words, n_rec, bitmap);
-    bitmap_count_kernel<<<592, 256, 0, st>>>(bitmap, words, count_dev);
-    return 2;
+    cudaMemsetAsync(&dm->n_mmers, 0, sizeof(unsigned long long), st);
+    mmer_bitmap_kernel<<<(unsigned)((n_skr + 255) / 256), 256, 0, st>>>(static_cast<const uint32_t *>(skr), K <= 32 ? 8 : 12, n_skr, bitmap);
+    bitmap_count_kernel<<<592, 256, 0, st>>>(bitmap, words, &dm->n_mmers);
+    *launches += 2;
+    CU(cudaGetLastError());
+    CU(read_back(ctx, &Misc::n_mmers, st));
+    const double buckets = hm->n_mmers ? (double)hm->n_mmers : 1.0;
+    const double mean_inst = (double)n_skr / buckets * ((K - M + 2) / 2.0);  // a record holds about (K-M+2)/2 windows
+    int nc = 1, h = 0;
+    const int cap1 = ctx->v3_cap ? ctx->v3_cap : 1024, cap2 = ctx->v3_cap ? ctx->v3_cap : 512;
+    if (mean_inst > cap1 / 2.5) {
+        nc = 2;
+        double per = mean_inst / 2.0;
+        while (per > cap2 / 8.0 && h < 15) {
+            per /= 4.0;
+            h++;
+        }
+    }
+    *out = make_key_layout(K, M, h, nc);
+    set_cap(*out);
+    ctx->v3_auto_n = n_skr;
+    ctx->v3_auto_h = out->h;
+    ctx->v3_auto_nc = out->nc;
+    return GBIN_OK;
+}
+
+// One pass of pipeline 3 over the sorted entries [ent, ent + n_ent): plan, group, finalize; the pass's k-mers / ids are appended to
+// the table behind the S_off k-mers / N_off ids of the passes before it.  *ok = false: the pass does not fit (see run_v3_group).
+static int run_v3_pass(gbin_ctx *ctx, const void *skr, const uint64_t *ent, const uint16_t *sorted_info, uint64_t n_ent, const KeyLayout &kl, const int32_t *d_ids,
+                       int32_t id_base, cudaStream_t st, uint64_t S_off, uint64_t N_off, bool single_pass, HostSink *sink, int *launches, bool *ok, uint64_t *n_inst,
+                       uint64_t *distinct, uint64_t *S_out, uint64_t *N_out) {
+    *ok = false;
+    const int cutoff = ctx->cfg.abundance_cutoff, KW = ctx->KW;
+    Misc *dm = ctx->misc.as<Misc>();
+    Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
+    // ---- plan: instance prefix, atoms, units
+    CU(ctx->inst_prefix.ensure((n_ent + 2) * 4));
+    CU(ctx->run_excl.ensure((n_ent + 2) * 8));
+    CU(ctx->skr_run_start.ensure((n_ent + 2) * 4));
+    CU(ctx->scan_scratch.ensure(group_scan_scratch_bytes(n_ent)));
+    bool on = ctx->prof.begin(KK_SKR_PLAN, st);
+    int lp = v3_plan_runs(ent, sorted_info, n_ent, ctx->inst_prefix.as<uint32_t>(), ctx->run_excl.as<uint64_t>(), ctx->skr_run_start.as<uint32_t>(),
+                          ctx->scan_scratch.as<uint64_t>(), &dm->plan.n_inst, &dm->plan.n_runs, st);
+    ctx->prof.end(on, lp, st);
+    *launches += lp;
+    CU(cudaGetLastError());
+    CU(read_back(ctx, &Misc::plan, st));
+    const uint64_t n_runs = hm->plan.n_runs, n = hm->plan.n_inst;
+    *n_inst = n;
+    ctx->rs.n_mmer_runs += n_runs;
+    const uint64_t max_units = v3_max_units(n, n_runs, ctx->v3_cap_eff);
+    CU(ctx->small_prefix.ensure((n_runs + 2) * 8));
+    CU(ctx->v3_base64.ensure((n_runs + 2) * 8));
+    CU(ctx->v3_atoms.ensure((4 * n_runs + 8) * 4));
+    CU(ctx->v3_head_run.ensure((max_units + 1) * 4));
+    CU(ctx->units.ensure(max_units * sizeof(Unit3)));
+    CU(ctx->v3_unit_out.ensure(max_units * sizeof(UnitOut3)));
+    CU(ctx->v3_unit_excl.ensure((2 * max_units + 2) * 8));
+    CU(ctx->scan_scratch.ensure(group_scan_scratch_bytes(n_runs + max_units + 1024)));
+    const bool to_host = single_pass && sink && sink->chunks > 1;  // stream finished chunks of the table to the host
+    const uint32_t n_chunks = to_host ? (uint32_t)sink->chunks : 1u;
+    on = ctx->prof.begin(KK_SKR_PLAN, st);
+    lp = v3_plan_units(sorted_info, ent, kl, ctx->v3_cap_eff, ctx->inst_prefix.as<uint32_t>(), ctx->skr_run_start.as<uint32_t>(), n_runs, ctx->small_prefix.as<uint64_t>(),
+                       ctx->v3_base64.as<uint64_t>(), ctx->v3_atoms.as<uint32_t>(), ctx->v3_atoms.as<uint32_t>() + 3 * n_runs, ctx->v3_head_run.as<uint32_t>(),
+                       ctx->scan_scratch.p, ctx->units.p, max_units, &dm->gc3, n_chunks, dm->chunk_bounds, st);
+    ctx->prof.end(on, lp, st);
+    *launches += lp;
+    CU(cudaGetLastError());
+
+    // ---- level 2 + prune + emit.  Output bounds: a surviving k-mer has more than `cutoff` instances.
+    const uint64_t kmer_cap = cutoff >= 0 ? n / ((uint64_t)cutoff + 1) + 1 : n + 1;
+    CU(ctx->o_kmer_codes.ensure_keep(((S_off + kmer_cap) * KW + 1) * sizeof(uint64_t), S_off * KW * sizeof(uint64_t), st));
+    CU(ctx->o_kmer_mmer.ensure_keep((S_off + kmer_cap + 1) * sizeof(uint32_t), S_off * sizeof(uint32_t), st));
+    CU(ctx->o_kmer_id_off.ensure_keep((S_off + kmer_cap + 2) * sizeof(uint64_t), S_off * sizeof(uint64_t), st));
+    CU(ctx->o_read_ids.ensure_keep((N_off + n + 1) * sizeof(int32_t), N_off * sizeof(int32_t), st));
+    CU(ctx->stg_ids.ensure((n + 1) * sizeof(int32_t)));
+    CU(ctx->stg_codes.ensure((kmer_cap * KW + 1) * sizeof(uint64_t)));
+    CU(ctx->stg_mmer.ensure((kmer_cap + 1) * sizeof(uint32_t)));
+    CU(ctx->stg_off.ensure((kmer_cap + 1) * sizeof(uint32_t)));
+    const uint32_t kdiv = cutoff >= 0 ? (uint32_t)cutoff + 1u : 1u;
+    const G3Stage stg{ctx->stg_codes.as<uint64_t>(), ctx->stg_mmer.as<uint32_t>(), ctx->stg_off.as<uint32_t>(), ctx->stg_ids.as<int32_t>(),
+                      ctx->v3_unit_out.as<UnitOut3>(), kmer_cap, n, kdiv};
+    const G3Final fin{ctx->o_kmer_codes.as<uint64_t>() + S_off * KW, ctx->o_kmer_mmer.as<uint32_t>() + S_off, ctx->o_kmer_id_off.as<uint64_t>() + S_off,
+                      ctx->o_read_ids.as<int32_t>() + N_off, N_off};
+    const size_t rb = sizeof(uint64_t) * KW + 8;
+    auto lsd_arrays = [&](uint64_t cap) -> int {  // arrays of the global sort for long spans, for `cap` k-mers
+        if (cap == 0) return GBIN_OK;
+        CU(ctx->rec_a.ensure((cap + 1) * rb));
+        CU(ctx->rec_b.ensure((cap + 1) * rb));
+        CU(ctx->v3_lsd_aux.ensure((cap + 1) * 16));
+        return GBIN_OK;
+    };
+    // long spans appear when buckets are large enough for extended keys; their k-mers are a fraction of the bound (grown on demand)
+    uint64_t lsd_cap = (kl.nc == 2 || ctx->v3_lsd_seen) ? (kmer_cap < (1u << 22) ? kmer_cap : kmer_cap / 4) : 0;
+    if (lsd_cap && lsd_cap < ctx->v3_lsd_cap_seen && ctx->v3_lsd_cap_seen <= kmer_cap) lsd_cap = ctx->v3_lsd_cap_seen;
+    int rc = lsd_arrays(lsd_cap);
+    if (rc) return rc;
+    lp = v3_group_launch(ctx, skr, ent, kl, cutoff, d_ids, id_base, stg, fin, lsd_cap, max_units, n_chunks, to_host, false, st);
+    *launches += lp;
+    CU(cudaGetLastError());
+    if (to_host) {  // the grouping kernels pack each chunk's totals as {k-mers << 32 | ids}
+        rc = stream_finished_chunks(ctx, sink, n_chunks, hm->chunk_totals, 32, hm->lsd_totals);
+        if (rc) return rc;
+    }
+    CU(read_back(ctx, &Misc::gc3, st));
+    if (hm->gc3.overflow == 6u && hm->gc3.lsd_kmers > lsd_cap) {
+        // long spans met no (or too small) sort arrays: allocate them and redo their placement (the staged results are still there)
+        ctx->v3_lsd_seen = true;
+        lsd_cap = hm->gc3.lsd_kmers + hm->gc3.lsd_kmers / 16 + 1024;
+        if (lsd_cap > kmer_cap) lsd_cap = kmer_cap;
+        ctx->v3_lsd_cap_seen = lsd_cap;
+        rc = lsd_arrays(lsd_cap);
+        if (rc) return rc;
+        CU(cudaMemsetAsync(&dm->gc3.overflow, 0, sizeof(unsigned int), st));
+        lp = v3_group_launch(ctx, skr, ent, kl, cutoff, d_ids, id_base, stg, fin, lsd_cap, max_units, n_chunks, false, true, st);
+        *launches += lp;
+        CU(cudaGetLastError());
+        CU(read_back(ctx, &Misc::gc3, st));
+    }
+    ctx->rs.n_units += hm->gc3.n_units;
+    ctx->rs.n_lsd_kmers += hm->gc3.lsd_kmers;
+    if (hm->gc3.overflow) {  // not done: the caller falls back
+        snprintf(ctx->err, sizeof ctx->err, "pipeline 3 gave the batch up (code %u: a (bucket, d) class larger than a unit)", hm->gc3.overflow);
+        return GBIN_OK;
+    }
+    if (hm->gc3.lsd_kmers) {
+        if ((rc = v3_lsd_finish(ctx, kl, hm->gc3.lsd_kmers, stg, fin, lsd_cap, st, launches))) return rc;
+        CU(cudaGetLastError());
+    }
+    *distinct = hm->gc3.distinct;
+    *S_out = hm->gc3.total_kmers;
+    *N_out = hm->gc3.total_ids;
+    *ok = true;
+    return GBIN_OK;
+}
+
+// *done = false when the batch does not fit (a (bucket, d) class larger than a unit); it then goes through pipeline 2, which sorts
+// the records themselves.
+int run_v3_group(gbin_ctx *ctx, const void *skr, uint64_t n_skr, const int32_t *d_ids, int32_t id_base, cudaStream_t st, gbin_table *out, int *launches,
+                 bool *done, uint64_t *n_inst_out, HostSink *sink) {
+    *done = false;
+    const int K = ctx->cfg.kmer_size, M = ctx->cfg.mmer_size;
+    Misc *dm = ctx->misc.as<Misc>();
+    Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
+    KeyLayout kl;
+    int rc = v3_choose_layout(ctx, skr, n_skr, st, &kl, launches);
+    if (rc) return rc;
+    if (n_skr >= (1ull << (32 - kl.cshift))) return GBIN_OK;  // slots are 32-bit
+    memset(&ctx->rs, 0, sizeof ctx->rs);
+    ctx->rs.n_super_kmers = n_skr;
+    ctx->rs.key_nc = (uint32_t)kl.nc;
+    ctx->rs.key_h = (uint32_t)kl.h;
+
+    // ---- entries + level 1: stable sort of the entries by key
+    const uint64_t n_slots = n_skr << kl.cshift;
+    // the two entry buffers of the sort: in donated memory when the caller gave enough of it (the multi-GPU path hands over the
+    // scan's record buffer, dead after the exchange — one allocation of that size less per step), else the context's own
+    const uint64_t ent_bytes = ((n_slots + 2) * 8 + 255) & ~255ull;
+    uint64_t *ent_a_p, *ent_b_p;
+    if (ctx->donated && ctx->donated_bytes >= 2 * ent_bytes && (reinterpret_cast<uintptr_t>(ctx->donated) & 15u) == 0) {
+        ent_a_p = static_cast<uint64_t *>(ctx->donated);
+        ent_b_p = ent_a_p + ent_bytes / 8;
+        if (ctx->ent_a.cap + ctx->ent_b.cap > (1ull << 30)) {  // a large batch on donated memory: the own buffers of an earlier one would only crowd the HBM
+            ctx->ent_a.release();
+            ctx->ent_b.release();
+        }
+    } else {
+        CU(ctx->ent_a.ensure(ent_bytes));
+        CU(ctx->ent_b.ensure(ent_bytes));
+        ent_a_p = ctx->ent_a.as<uint64_t>();
+        ent_b_p = ctx->ent_b.as<uint64_t>();
+    }
+    ctx->donated = nullptr;  // one call only
+    ctx->donated_bytes = 0;
+    CU(ctx->piece_n.ensure((n_slots + 16) * 2));
+    CU(ctx->sorted_info.ensure((n_slots + 16) * 2));
+    bool on = ctx->prof.begin(KK_V3_ENTRIES, st);
+    int lp = v3_make_entries(skr, n_skr, kl, ent_a_p, ctx->piece_n.as<uint16_t>(), &dm->n_real_entries, st);
+    ctx->prof.end(on, lp, st);
+    *launches += lp;
+    CU(cudaGetLastError());
+    CU(ctx->radix_scratch.ensure(radix_scratch_bytes(n_slots)));
+    bool in_b = false;
+    int passes = 0;
+    *launches += radix_sort_entries(ent_a_p, ent_b_p, n_slots, kl.key_bits, ctx->radix_scratch.p, &in_b, &passes, ctx->piece_n.as<uint16_t>(),
+                                    ctx->sorted_info.as<uint16_t>(), &ctx->prof, st, kl.nc == 2 ? &dm->n_real_entries : nullptr);
+    CU(cudaGetLastError());
+    ctx->tm.sort_passes = (uint32_t)passes;
+    const uint64_t *ent = in_b ? ent_b_p : ent_a_p;
+    CU(cudaEventRecord(ctx->ev[EV_SORTED], st));
+    uint64_t n_ent = n_slots;
+    if (kl.nc == 2) {  // empty pieces carry the all-ones key and sort behind everything: plan over the real ones only
+        CU(read_back(ctx, &Misc::n_real_entries, st));
+        n_ent = hm->n_real_entries;
+    }
+
+    // ---- passes: ranges of the sorted entries with at most pass_max k-mer instances each, cut between m-mer buckets
+    std::vector<uint64_t> bounds{0, n_ent};
+    const uint64_t pass_max = ctx->v3_pass_max;
+    if (n_skr * (uint64_t)(K - M + 1) > pass_max) {  // more than one pass is possible: look at the instance counts
+        const uint32_t nt = (uint32_t)((n_ent + PASS_TILE - 1) / PASS_TILE);
+        CU(ctx->scan_scratch.ensure((size_t)nt * 8 + 64));
+        unsigned long long *sums_dev = ctx->scan_scratch.as<unsigned long long>();
+        if (n_ent) {
+            pass_tile_sums_kernel<<<nt, 256, 0, st>>>(ctx->sorted_info.as<uint16_t>(), n_ent, sums_dev);
+            (*launches)++;
+        }
+        std::vector<unsigned long long> sums(nt);
+        CU(cudaMemcpyAsync(sums.data(), sums_dev, (size_t)nt * 8, cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        std::vector<unsigned long long> cuts;
+        unsigned long long acc = 0, all = 0;
+        for (uint32_t t = 0; t < nt; t++) all += sums[t];
+        // a batch of several passes is a batch that crowds the HBM: the workspace of a pass (staging, bounds of the table's growth) scales
+        // with the pass, so such a batch is cut into passes of half the size
+        const uint64_t pass_max = all > 2 * ctx->v3_pass_max ? ctx->v3_pass_max / 2 : ctx->v3_pass_max;
+        for (uint32_t t = 0; t < nt; t++) {
+            if (acc && acc + sums[t] > pass_max) {
+                cuts.push_back((unsigned long long)t * PASS_TILE);
+                acc = 0;
+            }
+            acc += sums[t];
+        }
+        if (!cuts.empty()) {
+            CU(cudaMemcpyAsync(sums_dev, cuts.data(), cuts.size() * 8, cudaMemcpyHostToDevice, st));
+            pass_bounds_kernel<<<((uint32_t)cuts.size() + 63) / 64, 64, 0, st>>>(ent, n_ent, kl.mshift, sums_dev, (uint32_t)cuts.size());
+            (*launches)++;
+            CU(cudaMemcpyAsync(cuts.data(), sums_dev, cuts.size() * 8, cudaMemcpyDeviceToHost, st));
+            CU(cudaStreamSynchronize(st));
+            bounds.assign(1, 0);
+            for (unsigned long long c : cuts)
+                if (c > bounds.back() && c < n_ent) bounds.push_back(c);
+            bounds.push_back(n_ent);
+        }
+    }
+    const bool single = bounds.size() == 2;
+    uint64_t S_off = 0, N_off = 0, n_total = 0, distinct = 0;
+    for (size_t p = 0; p + 1 < bounds.size(); p++) {
+        bool ok = false;
+        uint64_t n_p = 0, d_p = 0, S_p = 0, N_p = 0;
+        rc = run_v3_pass(ctx, skr, ent + bounds[p], ctx->sorted_info.as<uint16_t>() + bounds[p], bounds[p + 1] - bounds[p], kl, d_ids, id_base, st, S_off, N_off, single, sink, launches, &ok, &n_p, &d_p, &S_p, &N_p);
+        if (rc) return rc;
+        if (!ok) return GBIN_OK;  // not done: the caller falls back
+        S_off += S_p;
+        N_off += N_p;
+        n_total += n_p;
+        distinct += d_p;
+    }
+    *n_inst_out = n_total;
+    ctx->rs.n_passes = (uint32_t)(bounds.size() - 1);
+    const uint64_t S = S_off, NS = N_off;
+    if (S >= (1ull << 32)) return fail(ctx, GBIN_E_TOO_LARGE, "%llu surviving k-mers in one batch (limit 2^32)", (unsigned long long)S);
+    uint64_t B = 0;
+    rc = emit_bucket_directory(ctx, S, NS, st, launches, &B);
+    if (rc) return rc;
+    *out = device_table(ctx, n_total, distinct, S, NS, B);
+    *done = true;
+    return GBIN_OK;
 }
 
 }  // namespace gbin

@@ -93,4 +93,14 @@ struct __align__(16) Unit3 {
     uint32_t span_len;       // 0: the unit holds whole buckets; L: first of the L units of a bucket that does not fit one unit; ~0: another unit of such a bucket
 };
 
+// Device scalars of pipeline 3 (the host reads them through Misc::gc3).
+struct G3Counters {
+    unsigned long long distinct;
+    unsigned long long total_kmers, total_ids;
+    unsigned int overflow;
+    unsigned int n_units, n_spans;
+    unsigned int pad;
+    unsigned long long lsd_kmers, lsd_ids;  // surviving k-mers / ids of the spans that are put in order by the global sort
+};
+
 }  // namespace gbin

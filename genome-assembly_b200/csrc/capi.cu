@@ -1,8 +1,9 @@
-// capi.cu — the extern "C" layer of libgbin.so: context, HBM workspace and the pipeline
-//   scan (process_read, binning.c:918-1040) -> sort (zhash grouping, :1044-1069) -> run-length + prune (:1085-1144).
+// capi.cu — the extern "C" layer of libgbin.so: the context, read checks and staging, the scan stage and the fallback ladder
+// (pipeline 3 -> 2 -> 1), the host calls, the owner parts path, the owner exchange and the multi-GPU call.
+// The grouping pipelines keep their host orchestration next to their kernels: run_v3_group (bin3.cu), run_v2_group
+// (skr_group.cu), run_group (group_prune.cu).
 // There is no CPU fallback anywhere in this file: every entry point either runs the CUDA kernels or
 // returns an error code.
-#include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -13,237 +14,21 @@
 #include <thread>
 #include <vector>
 
-#include "../../include/gbin.h"
-#include "gbin_internal.h"
+#include "gbin_ctx.h"
 #include "prefix_scan.cuh"
 
 using namespace gbin;
 
 namespace {
 
-struct DevBuf {  // frees its memory when destroyed (with the context that holds it)
-    void *p = nullptr;
-    size_t cap = 0;
-    DevBuf() = default;
-    DevBuf(const DevBuf &) = delete;
-    DevBuf &operator=(const DevBuf &) = delete;
-    ~DevBuf() { release(); }
-    cudaError_t ensure(size_t bytes) {
-        if (bytes <= cap) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-        size_t want = bytes + bytes / 16 + 256;  // a little slack so near-equal batches do not reallocate
-        cudaError_t e = cudaMalloc(&p, want);
-        if (e != cudaSuccess) {
-            (void)cudaGetLastError();
-            e = cudaMalloc(&p, bytes);
-            want = bytes;
-        }
-        if (e == cudaSuccess) cap = want;
-        return e;
-    }
-    // grows like ensure() but keeps the first `keep` bytes (the parts of a table that earlier passes of a batch have written)
-    cudaError_t ensure_keep(size_t bytes, size_t keep, cudaStream_t st) {
-        if (bytes <= cap) return cudaSuccess;
-        if (!p || keep == 0) return ensure(bytes);
-        void *q = nullptr;
-        const size_t want = bytes + bytes / 16 + 256;
-        cudaError_t e = cudaMalloc(&q, want);
-        if (e != cudaSuccess) return e;
-        e = cudaMemcpyAsync(q, p, keep, cudaMemcpyDeviceToDevice, st);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-        cudaFree(p);
-        p = q;
-        cap = want;
-        return e;
-    }
-    void release() {
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-    }
-    template <typename T>
-    T *as() const { return static_cast<T *>(p); }
-};
-
-struct HostBuf {  // page-locked; freed when destroyed
-    void *p = nullptr;
-    size_t cap = 0;
-    HostBuf() = default;
-    HostBuf(const HostBuf &) = delete;
-    HostBuf &operator=(const HostBuf &) = delete;
-    ~HostBuf() { release(); }
-    cudaError_t ensure(size_t bytes) {
-        if (bytes <= cap) return cudaSuccess;
-        if (p) cudaFreeHost(p);
-        p = nullptr;
-        cap = 0;
-        const size_t want = bytes + bytes / 8 + 4096;
-        cudaError_t e = cudaMallocHost(&p, want);
-        if (e == cudaSuccess) cap = want;
-        return e;
-    }
-    void release() {
-        if (p) cudaFreeHost(p);
-        p = nullptr;
-        cap = 0;
-    }
-};
-
-// A range of host reads copied to the device (stage_host_reads): its bytes, its starts (rebased to the first copied byte) followed by
-// its lens, and the pinned host array the starts are rebased in.  Slot 0 also holds gbin_bin_file_host's file image and its split.
-struct ReadStage {
-    DevBuf data, meta;
-    HostBuf rebased;
-};
-
-// Small device-resident scalars (ctx->misc) and their pinned host mirror (ctx->h_misc).  Values the host needs at the same
-// point are grouped into one member, so that read_back() fetches them in one copy.
-struct Misc {
-    struct {
-        GroupCounts counts;
-        unsigned long long bad_bases;  // of pipeline 1's scan
-    } grp;
-    struct {
-        unsigned long long total_windows;
-        unsigned int max_len;
-    } reads;
-    uint64_t part_counts[256];
-    // super-k-mer pipelines (2 and 3)
-    unsigned long long skr_counters[4];  // [0] bad bases, [1] records, [2] instances
-    uint32_t skr_ticket, n_buckets_dev;
-    struct {
-        uint32_t n_inst, n_runs;
-    } plan;
-    unsigned long long chunk_totals[SKR_MAX_CHUNKS];
-    // pipeline 2
-    SkrGroupCounters gc;
-    uint32_t chunk_tickets[SKR_MAX_CHUNKS];
-    // pipeline 3
-    V3Counters gc3;
-    unsigned long long n_mmers;         // distinct m-mer codes of a batch (automatic key layout)
-    unsigned long long n_real_entries;  // entries of the sort that are not empty pieces
-    uint32_t chunk_bounds[SKR_MAX_CHUNKS + 1];
-    uint32_t v3_tickets[2 * SKR_MAX_CHUNKS];
-    unsigned long long lsd_totals[SKR_MAX_CHUNKS];
-    uint64_t v3_chunk_sum;
-    // file path and table digest
-    uint32_t split_n_nl, split_n_reads;
-    char last_byte;                     // of the file image
-    unsigned long long digest;
-    // one owner part per call: records and k-mer instances selected so far, and the select kernel's ticket
-    unsigned long long part_sel[2];
-    uint32_t part_ticket;
-};
-
-// Host path only.  HostFeed: the reads are still in host memory; the scan stage copies them chunk by chunk on the copy
-// stream and scans every chunk as soon as it has landed.  HostSink: pinned destinations for the big arrays of the
-// table; finished chunks of the grouping are copied out on the second copy stream while later chunks are still running.
+// Host path only: the reads are still in host memory; the scan stage copies them chunk by chunk on the copy stream and
+// scans every chunk as soon as it has landed.
 struct HostFeed {
     const char *src;     // host
     char *dst;           // device
     uint64_t bytes;
     int chunks;
 };
-struct HostSink {
-    uint64_t *kmer_codes, *kmer_id_off;  // pinned; capacities in k-mers
-    int32_t *read_ids;                   // pinned; capacity in ids
-    uint64_t kmer_cap, id_cap;
-    uint64_t kmers_done, ids_done;       // what has been enqueued for copy so far
-    int chunks;
-};
-
-// Timing events of one call, in the order they are recorded.
-enum : int { EV_START, EV_READS_ON_DEVICE, EV_SCANNED, EV_SORTED, EV_GROUPED, EV_TABLE_ON_HOST, EV_COUNT };
-
-}  // namespace
-
-struct gbin_ctx {
-    gbin_config cfg;
-    int KW;
-    int sm_count;
-    cudaStream_t stream;
-    cudaStream_t st_h2d, st_d2h;  // copy streams of the host path (H2D of later read chunks / D2H of finished table chunks overlap the kernels)
-    cudaEvent_t ev_feed[SKR_MAX_CHUNKS], ev_chunk[SKR_MAX_CHUNKS], ev_copy;
-    cudaStream_t st_aux;          // second compute stream of pipeline 3's grouping stage
-    cudaEvent_t ev_fork, ev_join;
-    int host_chunks;              // GBIN_HOST_CHUNKS (default 8; 1 = no overlap)
-    char err[512];
-    gbin_timings tm;
-    cudaEvent_t ev[EV_COUNT];
-    // inputs staged by the host path: [0] a whole batch or shard, or a chunk of the parts path, which alternates with [1]
-    ReadStage stage[2];
-    DevBuf d_ids;
-    // pipeline workspace
-    DevBuf rec_a, rec_b, radix_scratch, win_counts, rec_off, scan_scratch;
-    DevBuf group_of, run_start, surv_index, id_offset, surv_group, bucket_of;
-    DevBuf misc;
-    // workspace of the super-k-mer pipelines (2 and 3)
-    DevBuf skr_a, skr_b, tile_state, inst_prefix, run_excl, skr_run_start, small_prefix, unit_base, units, unit_state, o_kmer_mmer, bucket_excl, big_list, big_k0, big_k1, big_arr, stg_ids, stg_codes, stg_mmer, stg_off, skr_side;
-    // pipeline 3 workspace
-    DevBuf ent_a, ent_b, piece_n, sorted_info, v3_base64, v3_head_run, v3_unit_out, v3_unit_excl, v3_atoms, v3_lsd_aux, v3_bitmap;
-    DevBuf x_list_off, x_ids;         // gbin_expand_read_ids_device's result
-    void *donated = nullptr;          // gbin_donate_scratch: caller-owned device memory the next grouping call may use for its sort buffers
-    uint64_t donated_bytes = 0;
-    bool v3_lsd_seen = false;         // a batch on this context had long spans: keep the arrays of their global sort
-    uint64_t v3_lsd_cap_seen = 0;     // and how many k-mers they were sized for
-    uint64_t v3_pass_max = 2000000000ull;  // k-mer instances per pass of pipeline 3 (gbin_set_tuning "v3_pass_max")
-    uint64_t v3_auto_n = 0;           // record count for which the key layout below was chosen (v3_nc == 0: automatic)
-    int v3_auto_h = 0, v3_auto_nc = 1;
-    int v3_h, v3_nc, v3_cap;  // key layout and unit capacity of pipeline 3 (gbin_set_tuning; GBIN_V3_H / GBIN_V3_NC / GBIN_V3_CAP); v3_cap 0 = by layout
-    int v3_cap_eff;           // the capacity of the current batch
-    int xchg_timeout_ms = 120000;  // gbin_set_tuning "xchg_timeout_ms" / GBIN_XCHG_TIMEOUT_MS
-    int pipeline;        // 3: sort by reference + warp units, falling back to 2, then 1 (default); 2: super-k-mer path with v1 as fallback; 1: v1 only
-    int last_pipeline;   // which one produced the last table
-    uint32_t fallbacks;  // fallbacks to the next pipeline (3 -> 2 -> 1) since creation
-    gbin_run_stats rs;   // sizes seen by the last pipeline-2 or pipeline-3 run
-    // owner exchange over peer memory (multi-GPU, one process per GPU)
-    struct {
-        bool created = false, attached = false;
-        uint32_t rank = 0, world = 0, epoch = 0;
-        uint64_t cap = 0;
-        void *recv = nullptr;
-        XchgShared *sh = nullptr;
-        char **dst_tab = nullptr;
-        XchgResult *result = nullptr;
-        XchgPlan plan;
-        void *opened[2 * XCHG_MAX_WORLD];
-        int n_opened = 0;
-    } xg;
-    // device-resident result
-    DevBuf o_mmer_codes, o_mmer_kmer_off, o_kmer_codes, o_kmer_id_off, o_read_ids;
-    // pinned host arena for results of the host path + small readbacks
-    HostBuf h_misc, h_result, h_kmer_codes, h_kmer_id_off, h_read_ids, h_file;
-    DevBuf split_nl, split_tiles_buf, split_base;  // device-side fgets splitting
-    // one owner part per call: the part's records, the select's tiles
-    DevBuf part_rec, part_state;
-    uint64_t part_chunk_bytes = 1ull << 30;  // gbin_set_tuning "part_chunk_kb"
-    cudaEvent_t ev_part_h2d[4];              // [2 * slot + 0 | 1]: around the copy of a chunk into slot 0 | 1 (timed)
-    KernelProf prof;
-};
-
-namespace {
-
-int fail(gbin_ctx *ctx, int code, const char *fmt, ...) {
-    if (ctx) {
-        va_list ap;
-        va_start(ap, fmt);
-        vsnprintf(ctx->err, sizeof ctx->err, fmt, ap);
-        va_end(ap);
-    }
-    return code;
-}
-
-#define CU(call)                                                                                              \
-    do {                                                                                                      \
-        cudaError_t e__ = (call);                                                                             \
-        if (e__ != cudaSuccess) {                                                                             \
-            (void)cudaGetLastError();                                                                         \
-            return fail(ctx, e__ == cudaErrorMemoryAllocation ? GBIN_E_NOMEM : GBIN_E_CUDA, "%s: %s (%s:%d)", \
-                        #call, cudaGetErrorString(e__), __FILE__, __LINE__);                                  \
-        }                                                                                                     \
-    } while (0)
 
 int check_config(const gbin_config *c) {
     if (!c) return GBIN_E_INVALID_ARG;
@@ -259,62 +44,10 @@ cudaError_t begin_call(gbin_ctx *ctx, void *stream, cudaStream_t *st) {
     return cudaSetDevice(ctx->cfg.device);
 }
 
-// Copies one member of the device scalars into the pinned mirror and waits for it: one host round trip.
-template <typename T>
-cudaError_t read_back(gbin_ctx *ctx, T Misc::*field, cudaStream_t st) {
-    Misc *dm = ctx->misc.as<Misc>();
-    Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
-    const cudaError_t e = cudaMemcpyAsync(&(hm->*field), &(dm->*field), sizeof(T), cudaMemcpyDeviceToHost, st);
-    return e == cudaSuccess ? cudaStreamSynchronize(st) : e;
-}
+}  // namespace
 
-// The device table over the context's output arrays.
-gbin_table device_table(const gbin_ctx *ctx, uint64_t n_instances, uint64_t n_distinct, uint64_t S, uint64_t NS, uint64_t B) {
-    gbin_table t;
-    memset(&t, 0, sizeof t);
-    t.kmer_size = ctx->cfg.kmer_size;
-    t.mmer_size = ctx->cfg.mmer_size;
-    t.abundance_cutoff = ctx->cfg.abundance_cutoff;
-    t.kmer_words = ctx->KW;
-    t.on_device = 1;
-    t.ctx_owned = 1;
-    t.n_instances = n_instances;
-    t.n_distinct = n_distinct;
-    t.n_kmers = S;
-    t.n_ids = NS;
-    t.n_buckets = B;
-    t.mmer_codes = ctx->o_mmer_codes.as<uint32_t>();
-    t.mmer_kmer_off = ctx->o_mmer_kmer_off.as<uint64_t>();
-    t.kmer_codes = ctx->o_kmer_codes.as<uint64_t>();
-    t.kmer_id_off = ctx->o_kmer_id_off.as<uint64_t>();
-    t.read_ids = ctx->o_read_ids.as<int32_t>();
-    return t;
-}
+namespace gbin {
 
-// Bucket directory of the super-k-mer pipelines over the S surviving k-mers in ctx->o_kmer_mmer; *B receives the bucket count.
-int emit_bucket_directory(gbin_ctx *ctx, uint64_t S, uint64_t NS, cudaStream_t st, int *launches, uint64_t *B) {
-    Misc *dm = ctx->misc.as<Misc>();
-    Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
-    CU(ctx->bucket_excl.ensure((S + 1) * 4));
-    CU(ctx->o_mmer_codes.ensure((S + 1) * sizeof(uint32_t)));
-    CU(ctx->o_mmer_kmer_off.ensure((S + 2) * sizeof(uint64_t)));
-    CU(ctx->scan_scratch.ensure(group_scan_scratch_bytes(S + 1024)));
-    const bool on = ctx->prof.begin(KK_EMIT, st);
-    const int lp = skr_emit_buckets(ctx->o_kmer_mmer.as<uint32_t>(), S, NS, ctx->bucket_excl.as<uint32_t>(), ctx->scan_scratch.as<uint32_t>(),
-                                    ctx->o_mmer_codes.as<uint32_t>(), ctx->o_mmer_kmer_off.as<uint64_t>(), ctx->o_kmer_id_off.as<uint64_t>(),
-                                    &dm->n_buckets_dev, st);
-    ctx->prof.end(on, lp, st);
-    *launches += lp;
-    CU(cudaGetLastError());
-    CU(read_back(ctx, &Misc::n_buckets_dev, st));
-    *B = hm->n_buckets_dev;
-    return GBIN_OK;
-}
-
-// Host path: streams the finished part of the table to the host while later chunks are grouped.  The table is written in
-// unit order, and what the units of chunk c wrote is final once ctx->ev_chunk[c] has fired; totals_host[c] then holds
-// {k-mers << shift | ids} written up to the end of chunk c.  A chunk with k-mers left to pipeline 3's global sort for long spans
-// (lsd_totals_host[c] != 0) ends the streaming, as does an arena too small: the rest is copied at the end.
 int stream_finished_chunks(gbin_ctx *ctx, HostSink *sink, uint32_t n, const unsigned long long *totals_host, int shift,
                            const unsigned long long *lsd_totals_host) {
     const int KW = ctx->KW;
@@ -335,6 +68,10 @@ int stream_finished_chunks(gbin_ctx *ctx, HostSink *sink, uint32_t n, const unsi
     }
     return GBIN_OK;
 }
+
+}  // namespace gbin
+
+namespace {
 
 // What was streamed into the sink belongs to an abandoned attempt: wait until nothing is in flight into the arenas, then start over.
 int abandon_sink(gbin_ctx *ctx, HostSink *sink) {
@@ -511,84 +248,6 @@ int run_scan(gbin_ctx *ctx, const gbin_reads *rd, uint32_t arrival_base, void *d
     return GBIN_OK;
 }
 
-// Sort + run-length + prune + emit of n records living in `recs` (scratch twin `twin`).
-int run_group(gbin_ctx *ctx, void *recs, void *twin, uint64_t n, const int32_t *d_ids, int32_t id_base, cudaStream_t st,
-              gbin_table *out, int *launches, cudaEvent_t ev_sorted) {
-    const int KW = ctx->KW, K = ctx->cfg.kmer_size, M = ctx->cfg.mmer_size, cutoff = ctx->cfg.abundance_cutoff;
-    Misc *dm = ctx->misc.as<Misc>();
-    Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
-    CU(ctx->radix_scratch.ensure(radix_scratch_bytes(n)));
-    bool in_b = false;
-    int passes = 0;
-    *launches += radix_sort_records(recs, twin, n, KW, K, M, ctx->radix_scratch.p, &in_b, &passes, &ctx->prof, st);
-    CU(cudaGetLastError());
-    ctx->tm.sort_passes = (uint32_t)passes;
-    const void *sorted = in_b ? twin : recs;
-    if (ev_sorted) CU(cudaEventRecord(ev_sorted, st));
-
-    GroupWorkspace ws{};
-    CU(ctx->group_of.ensure((n + 1) * sizeof(uint32_t)));
-    CU(ctx->run_start.ensure((n + 2) * sizeof(uint32_t)));
-    CU(ctx->scan_scratch.ensure(group_scan_scratch_bytes(n)));
-    ws.group_of = ctx->group_of.as<uint32_t>();
-    ws.run_start = ctx->run_start.as<uint32_t>();
-    ws.scan_scratch = ctx->scan_scratch.p;
-    ws.counts = &dm->grp.counts;
-    ws.cutoff = cutoff;
-
-    bool on = ctx->prof.begin(KK_RUNS, st);
-    int lg = group_find_runs(sorted, n, KW, ws, st);
-    ctx->prof.end(on, lg, st);
-    *launches += lg;
-    CU(cudaGetLastError());
-    CU(read_back(ctx, &Misc::grp, st));
-    if (hm->grp.bad_bases) return fail(ctx, GBIN_E_NON_ACGT, "%llu bases other than A/C/G/T in the batch", hm->grp.bad_bases);
-    const uint64_t G = hm->grp.counts.n_distinct;
-
-    uint64_t S = 0, NS = 0, B = 0;
-    if (G) {
-        CU(ctx->surv_index.ensure((G + 1) * sizeof(uint32_t)));
-        CU(ctx->id_offset.ensure((G + 1) * sizeof(uint64_t)));
-        ws.surv_index = ctx->surv_index.as<uint32_t>();
-        ws.id_offset = ctx->id_offset.as<uint64_t>();
-        on = ctx->prof.begin(KK_PRUNE, st);
-        lg = group_prune_offsets(n, G, cutoff, ws, st);
-        ctx->prof.end(on, lg, st);
-        *launches += lg;
-        CU(cudaGetLastError());
-        CU(read_back(ctx, &Misc::grp, st));
-        S = hm->grp.counts.n_kmers;
-        NS = hm->grp.counts.n_ids;
-    }
-    if (S) {
-        CU(ctx->surv_group.ensure(S * sizeof(uint32_t)));
-        CU(ctx->bucket_of.ensure(S * sizeof(uint32_t)));
-        ws.surv_group = ctx->surv_group.as<uint32_t>();
-        ws.bucket_of = ctx->bucket_of.as<uint32_t>();
-        on = ctx->prof.begin(KK_PRUNE, st);
-        lg = group_mark_buckets(sorted, KW, G, S, ws, st);
-        ctx->prof.end(on, lg, st);
-        *launches += lg;
-        CU(cudaGetLastError());
-        CU(read_back(ctx, &Misc::grp, st));
-        B = hm->grp.counts.n_buckets;
-    }
-    CU(ctx->o_mmer_codes.ensure((B + 1) * sizeof(uint32_t)));
-    CU(ctx->o_mmer_kmer_off.ensure((B + 1) * sizeof(uint64_t)));
-    CU(ctx->o_kmer_codes.ensure((S * KW + 1) * sizeof(uint64_t)));
-    CU(ctx->o_kmer_id_off.ensure((S + 1) * sizeof(uint64_t)));
-    CU(ctx->o_read_ids.ensure((NS + 1) * sizeof(int32_t)));
-    TableOut to{ctx->o_mmer_codes.as<uint32_t>(), ctx->o_mmer_kmer_off.as<uint64_t>(), ctx->o_kmer_codes.as<uint64_t>(),
-                ctx->o_kmer_id_off.as<uint64_t>(), ctx->o_read_ids.as<int32_t>()};
-    on = ctx->prof.begin(KK_EMIT, st);
-    lg = group_emit(sorted, n, KW, G, S, NS, B, d_ids, id_base, ws, to, st);
-    ctx->prof.end(on, lg, st);
-    *launches += lg;
-    CU(cudaGetLastError());
-    *out = device_table(ctx, n, G, S, NS, B);
-    return GBIN_OK;
-}
-
 // ---- super-k-mer pipelines.  Pipeline 2: super-k-mer records -> stable sort by m-mer -> grouping in shared memory.
 
 // Scan stage of pipelines 2 and 3: one record per signature segment, in arrival order, into ctx->skr_a (own == true) or into the
@@ -640,408 +299,6 @@ int run_skr_scan(gbin_ctx *ctx, const gbin_reads *rd, uint64_t n, uint32_t max_l
         cap = n_skr;  // more segments than estimated: the kernel only counted; run it again with room for all
     }
     *n_skr_out = n_skr;
-    return GBIN_OK;
-}
-
-// Sort + plan + group + emit over n_skr records in `skr` (clobbered; `twin` is the sort's second buffer).
-// *done = false when a unit overflowed and the batch must go through pipeline v1.
-int run_v2_group(gbin_ctx *ctx, void *skr, void *twin, uint64_t n_skr, const int32_t *d_ids, int32_t id_base, cudaStream_t st, gbin_table *out,
-                 int *launches, bool *done, uint64_t *n_inst_out, HostSink *sink = nullptr) {
-    *done = false;
-    const int K = ctx->cfg.kmer_size, M = ctx->cfg.mmer_size, cutoff = ctx->cfg.abundance_cutoff, KW = ctx->KW;
-    const int NW = K <= 32 ? 8 : 12;
-    Misc *dm = ctx->misc.as<Misc>();
-    Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
-
-    // ---- level 1: stable sort of the records by m-mer code
-    CU(ctx->radix_scratch.ensure(radix_scratch_bytes(n_skr)));
-    bool in_b = false;
-    int passes = 0;
-    CU(ctx->skr_side.ensure((n_skr + 2) * 8));
-    *launches += radix_sort_skr_by_mmer(skr, twin, n_skr, NW, M, ctx->radix_scratch.p, &in_b, &passes, ctx->skr_side.as<uint64_t>(), &ctx->prof, st);
-    CU(cudaGetLastError());
-    ctx->tm.sort_passes = (uint32_t)passes;
-    const void *sorted = in_b ? twin : skr;
-    CU(cudaEventRecord(ctx->ev[EV_SORTED], st));
-
-    // ---- plan: instance prefix, m-mer runs, units
-    CU(ctx->inst_prefix.ensure((n_skr + 2) * 4));
-    CU(ctx->run_excl.ensure((n_skr + 2) * 8));
-    CU(ctx->skr_run_start.ensure((n_skr + 2) * 4));
-    CU(ctx->scan_scratch.ensure(group_scan_scratch_bytes(n_skr)));
-    bool on = ctx->prof.begin(KK_SKR_PLAN, st);
-    int lp = skr_plan_runs(ctx->skr_side.as<uint64_t>(), n_skr, ctx->inst_prefix.as<uint32_t>(), ctx->run_excl.as<uint64_t>(), ctx->skr_run_start.as<uint32_t>(),
-                           ctx->scan_scratch.as<uint64_t>(), &dm->plan.n_inst, &dm->plan.n_runs, st);
-    ctx->prof.end(on, lp, st);
-    *launches += lp;
-    CU(cudaGetLastError());
-    CU(read_back(ctx, &Misc::plan, st));
-    const uint64_t n_runs = hm->plan.n_runs, n = hm->plan.n_inst;
-    *n_inst_out = n;
-    ctx->rs.n_super_kmers = n_skr;
-    ctx->rs.n_mmer_runs = n_runs;
-    const uint64_t max_units = skr_max_units(n, n_runs);
-    CU(ctx->small_prefix.ensure((n_runs + 1) * 4));
-    CU(ctx->unit_base.ensure((n_runs + 1) * 4));
-    CU(ctx->units.ensure(max_units * skr_unit_bytes()));
-    CU(ctx->unit_state.ensure(max_units * 8));
-    CU(ctx->big_list.ensure(skr_max_big_runs(n) * 8));
-    CU(ctx->big_k0.ensure((n + 1) * 8));
-    if (KW == 2) CU(ctx->big_k1.ensure((n + 1) * 8));
-    CU(ctx->big_arr.ensure((n + 1) * 4));
-    CU(ctx->scan_scratch.ensure(group_scan_scratch_bytes(n / 2 + n_runs + 1024)));
-    on = ctx->prof.begin(KK_SKR_PLAN, st);
-    lp = skr_plan_units(sorted, K, ctx->inst_prefix.as<uint32_t>(), ctx->skr_run_start.as<uint32_t>(), n_runs, ctx->small_prefix.as<uint32_t>(),
-                        ctx->unit_base.as<uint32_t>(), ctx->scan_scratch.as<uint32_t>(), ctx->units.p, max_units, &dm->gc, ctx->big_list.as<uint32_t>(),
-                        ctx->big_k0.as<uint64_t>(), ctx->big_k1.as<uint64_t>(), ctx->big_arr.as<uint32_t>(), ctx->sm_count, st);
-    ctx->prof.end(on, lp, st);
-    *launches += lp;
-    CU(cudaGetLastError());
-
-    // ---- level 2 + prune + emit. Output bounds: a surviving k-mer has more than `cutoff` instances.
-    const uint64_t kmer_cap = cutoff >= 0 ? n / ((uint64_t)cutoff + 1) + 1 : n + 1;
-    CU(ctx->o_kmer_codes.ensure((kmer_cap * KW + 1) * sizeof(uint64_t)));
-    CU(ctx->o_kmer_mmer.ensure((kmer_cap + 1) * sizeof(uint32_t)));
-    CU(ctx->o_kmer_id_off.ensure((kmer_cap + 2) * sizeof(uint64_t)));
-    CU(ctx->o_read_ids.ensure((n + 1) * sizeof(int32_t)));
-    CU(ctx->stg_ids.ensure((n + 1) * sizeof(int32_t)));
-    CU(ctx->stg_codes.ensure((kmer_cap * KW + 1) * sizeof(uint64_t)));
-    CU(ctx->stg_mmer.ensure((kmer_cap + 1) * sizeof(uint32_t)));
-    CU(ctx->stg_off.ensure((kmer_cap + 1) * sizeof(uint32_t)));
-    on = ctx->prof.begin(KK_SKR_GROUP, st);
-    SkrGroupChunks ch{1u, dm->chunk_tickets, nullptr, nullptr, nullptr};
-    if (sink && sink->chunks > 1) {
-        ch.n = (uint32_t)sink->chunks;
-        ch.totals_dev = dm->chunk_totals;
-        ch.totals_host = hm->chunk_totals;
-        ch.done = ctx->ev_chunk;
-    }
-    lp = skr_group_launch(sorted, K, cutoff, ctx->inst_prefix.as<uint32_t>(), ctx->units.p, ctx->unit_state.as<unsigned long long>(), max_units, ch,
-                          &dm->gc, ctx->big_k0.as<uint64_t>(), ctx->big_k1.as<uint64_t>(), ctx->big_arr.as<uint32_t>(), d_ids, id_base, ctx->o_kmer_codes.as<uint64_t>(), ctx->o_kmer_mmer.as<uint32_t>(),
-                          ctx->o_kmer_id_off.as<uint64_t>(), ctx->o_read_ids.as<int32_t>(), kmer_cap, n, ctx->stg_ids.as<int32_t>(), ctx->stg_codes.as<uint64_t>(),
-                          ctx->stg_mmer.as<uint32_t>(), ctx->stg_off.as<uint32_t>(), ctx->sm_count, st);
-    ctx->prof.end(on, lp, st);
-    *launches += lp;
-    CU(cudaGetLastError());
-    if (ch.done) {  // the grouping kernels pack each chunk's totals as {k-mers << 31 | ids}
-        const int rc = stream_finished_chunks(ctx, sink, ch.n, hm->chunk_totals, 31, nullptr);
-        if (rc) return rc;
-    }
-    CU(read_back(ctx, &Misc::gc, st));
-    ctx->rs.n_units = hm->gc.n_units;
-    if (hm->gc.overflow) {  // a unit did not fit shared memory: this batch goes through pipeline v1
-        ctx->fallbacks++;
-        return GBIN_OK;
-    }
-    const uint64_t S = hm->gc.total_kmers, NS = hm->gc.total_ids;
-    uint64_t B = 0;
-    const int rc = emit_bucket_directory(ctx, S, NS, st, launches, &B);
-    if (rc) return rc;
-    *out = device_table(ctx, n, hm->gc.distinct, S, NS, B);
-    *done = true;
-    return GBIN_OK;
-}
-
-// ---- pipeline 3: entries sorted by reference, one warp (512-instance units) or one pair of warps (1024-instance units) per unit,
-// staging + finalize (bin3.cu)
-// The records in `skr` are read, not moved.  *done = false when the batch does not fit (a (bucket, d) class larger than a unit);
-// it then goes through pipeline 2, which sorts the records themselves.
-
-// Key layout for this batch: explicit (gbin_set_tuning v3_nc = 1 | 2) or chosen from the mean m-mer bucket size (v3_nc = 0):
-// buckets that fit a unit need nothing but the m-mer code; larger ones are broken up by extending the key (bin3.cuh).
-int v3_choose_layout(gbin_ctx *ctx, const void *skr, uint64_t n_skr, cudaStream_t st, KeyLayout *out, int *launches) {
-    const int K = ctx->cfg.kmer_size, M = ctx->cfg.mmer_size;
-    // Unit capacity: 1024 instances when whole m-mer buckets are units (fewer buckets straddle units), 512 when the key is
-    // extended or the k-mers are two words wide (twice the warps per SM: the grouping kernel is latency-bound; measured
-    // 17.1 -> 11.3 ms on a config-3 shaped batch, 13.4 -> 7.9 ms on a config-5 shaped one).
-    auto set_cap = [&](const KeyLayout &kl) { ctx->v3_cap_eff = ctx->v3_cap ? ctx->v3_cap : ((ctx->KW == 2 || kl.nc == 2) ? 512 : 1024); };
-    if (ctx->v3_nc != 0) {
-        *out = make_key_layout(K, M, ctx->v3_h, ctx->v3_nc);
-        set_cap(*out);
-        return GBIN_OK;
-    }
-    if (2 * M + 2 > 31 || M > 13 || n_skr == 0) {  // no room for a longer key / code space too large for the bitmap: plain m-mer keys
-        *out = make_key_layout(K, M, 0, 1);
-        set_cap(*out);
-        return GBIN_OK;
-    }
-    // the decision is kept for batches of similar size on this context
-    if (ctx->v3_auto_n && n_skr >= ctx->v3_auto_n / 2 && n_skr <= ctx->v3_auto_n * 2) {
-        *out = make_key_layout(K, M, ctx->v3_auto_h, ctx->v3_auto_nc);
-        set_cap(*out);
-        return GBIN_OK;
-    }
-    Misc *dm = ctx->misc.as<Misc>();
-    Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
-    CU(ctx->v3_bitmap.ensure(v3_mmer_bitmap_bytes(M)));
-    *launches += v3_count_mmers(skr, K <= 32 ? 8 : 12, n_skr, M, ctx->v3_bitmap.as<uint32_t>(), &dm->n_mmers, st);
-    CU(cudaGetLastError());
-    CU(read_back(ctx, &Misc::n_mmers, st));
-    const double buckets = hm->n_mmers ? (double)hm->n_mmers : 1.0;
-    const double mean_inst = (double)n_skr / buckets * ((K - M + 2) / 2.0);  // a record holds about (K-M+2)/2 windows
-    int nc = 1, h = 0;
-    const int cap1 = ctx->v3_cap ? ctx->v3_cap : 1024, cap2 = ctx->v3_cap ? ctx->v3_cap : 512;
-    if (mean_inst > cap1 / 2.5) {
-        nc = 2;
-        double per = mean_inst / 2.0;
-        while (per > cap2 / 8.0 && h < 15) {
-            per /= 4.0;
-            h++;
-        }
-    }
-    *out = make_key_layout(K, M, h, nc);
-    set_cap(*out);
-    ctx->v3_auto_n = n_skr;
-    ctx->v3_auto_h = out->h;
-    ctx->v3_auto_nc = out->nc;
-    return GBIN_OK;
-}
-
-// One pass of pipeline 3 over the sorted entries [ent, ent + n_ent): plan, group, finalize; the pass's k-mers / ids are appended to
-// the table behind the S_off k-mers / N_off ids of the passes before it.  *ok = false: the pass does not fit (see run_v3_group).
-int run_v3_pass(gbin_ctx *ctx, const void *skr, const uint64_t *ent, const uint16_t *sorted_info, uint64_t n_ent, const KeyLayout &kl, const int32_t *d_ids, int32_t id_base, cudaStream_t st,
-                uint64_t S_off, uint64_t N_off, bool single_pass, HostSink *sink, int *launches, bool *ok, uint64_t *n_inst, uint64_t *distinct, uint64_t *S_out,
-                uint64_t *N_out) {
-    *ok = false;
-    const int cutoff = ctx->cfg.abundance_cutoff, KW = ctx->KW;
-    Misc *dm = ctx->misc.as<Misc>();
-    Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
-    // ---- plan: instance prefix, atoms, units
-    CU(ctx->inst_prefix.ensure((n_ent + 2) * 4));
-    CU(ctx->run_excl.ensure((n_ent + 2) * 8));
-    CU(ctx->skr_run_start.ensure((n_ent + 2) * 4));
-    CU(ctx->scan_scratch.ensure(group_scan_scratch_bytes(n_ent)));
-    bool on = ctx->prof.begin(KK_SKR_PLAN, st);
-    int lp = v3_plan_runs(ent, sorted_info, n_ent, ctx->inst_prefix.as<uint32_t>(), ctx->run_excl.as<uint64_t>(), ctx->skr_run_start.as<uint32_t>(),
-                          ctx->scan_scratch.as<uint64_t>(), &dm->plan.n_inst, &dm->plan.n_runs, st);
-    ctx->prof.end(on, lp, st);
-    *launches += lp;
-    CU(cudaGetLastError());
-    CU(read_back(ctx, &Misc::plan, st));
-    const uint64_t n_runs = hm->plan.n_runs, n = hm->plan.n_inst;
-    *n_inst = n;
-    ctx->rs.n_mmer_runs += n_runs;
-    const uint64_t max_units = v3_max_units(n, n_runs, ctx->v3_cap_eff);
-    CU(ctx->small_prefix.ensure((n_runs + 2) * 8));
-    CU(ctx->v3_base64.ensure((n_runs + 2) * 8));
-    CU(ctx->v3_atoms.ensure((4 * n_runs + 8) * 4));
-    CU(ctx->v3_head_run.ensure((max_units + 1) * 4));
-    CU(ctx->units.ensure(max_units * v3_unit_bytes()));
-    CU(ctx->v3_unit_out.ensure(max_units * v3_unit_out_bytes()));
-    CU(ctx->v3_unit_excl.ensure((2 * max_units + 2) * 8));
-    CU(ctx->scan_scratch.ensure(group_scan_scratch_bytes(n_runs + max_units + 1024)));
-    V3Chunks ch{1u, dm->v3_tickets, dm->chunk_bounds, &dm->v3_chunk_sum, dm->chunk_totals, dm->lsd_totals, nullptr, nullptr, nullptr,
-                ctx->st_aux, ctx->ev_fork, ctx->ev_join};
-    if (single_pass && sink && sink->chunks > 1) {
-        ch.n = (uint32_t)sink->chunks;
-        ch.totals_host = hm->chunk_totals;
-        ch.lsd_totals_host = hm->lsd_totals;
-        ch.done = ctx->ev_chunk;
-    }
-    on = ctx->prof.begin(KK_SKR_PLAN, st);
-    lp = v3_plan_units(sorted_info, ent, kl, ctx->v3_cap_eff, ctx->inst_prefix.as<uint32_t>(), ctx->skr_run_start.as<uint32_t>(), n_runs, ctx->small_prefix.as<uint64_t>(),
-                       ctx->v3_base64.as<uint64_t>(), ctx->v3_atoms.as<uint32_t>(), ctx->v3_atoms.as<uint32_t>() + 3 * n_runs, ctx->v3_head_run.as<uint32_t>(),
-                       ctx->scan_scratch.p, ctx->units.p, max_units, &dm->gc3, ch.n, dm->chunk_bounds, st);
-    ctx->prof.end(on, lp, st);
-    *launches += lp;
-    CU(cudaGetLastError());
-
-    // ---- level 2 + prune + emit.  Output bounds: a surviving k-mer has more than `cutoff` instances.
-    const uint64_t kmer_cap = cutoff >= 0 ? n / ((uint64_t)cutoff + 1) + 1 : n + 1;
-    CU(ctx->o_kmer_codes.ensure_keep(((S_off + kmer_cap) * KW + 1) * sizeof(uint64_t), S_off * KW * sizeof(uint64_t), st));
-    CU(ctx->o_kmer_mmer.ensure_keep((S_off + kmer_cap + 1) * sizeof(uint32_t), S_off * sizeof(uint32_t), st));
-    CU(ctx->o_kmer_id_off.ensure_keep((S_off + kmer_cap + 2) * sizeof(uint64_t), S_off * sizeof(uint64_t), st));
-    CU(ctx->o_read_ids.ensure_keep((N_off + n + 1) * sizeof(int32_t), N_off * sizeof(int32_t), st));
-    CU(ctx->stg_ids.ensure((n + 1) * sizeof(int32_t)));
-    CU(ctx->stg_codes.ensure((kmer_cap * KW + 1) * sizeof(uint64_t)));
-    CU(ctx->stg_mmer.ensure((kmer_cap + 1) * sizeof(uint32_t)));
-    CU(ctx->stg_off.ensure((kmer_cap + 1) * sizeof(uint32_t)));
-    V3Out vo{ctx->o_kmer_codes.as<uint64_t>() + S_off * KW, ctx->o_kmer_mmer.as<uint32_t>() + S_off, ctx->o_kmer_id_off.as<uint64_t>() + S_off,
-             ctx->o_read_ids.as<int32_t>() + N_off, kmer_cap, n, ctx->stg_codes.as<uint64_t>(), ctx->stg_mmer.as<uint32_t>(), ctx->stg_off.as<uint32_t>(),
-             ctx->stg_ids.as<int32_t>(), ctx->v3_unit_out.p, N_off};
-    const size_t rb = sizeof(uint64_t) * KW + 8;
-    auto lsd_arrays = [&](uint64_t cap) -> int {  // arrays of the global sort for long spans, for `cap` k-mers
-        if (cap == 0) return GBIN_OK;
-        CU(ctx->rec_a.ensure((cap + 1) * rb));
-        CU(ctx->rec_b.ensure((cap + 1) * rb));
-        CU(ctx->v3_lsd_aux.ensure((cap + 1) * 16));
-        return GBIN_OK;
-    };
-    // long spans appear when buckets are large enough for extended keys; their k-mers are a fraction of the bound (grown on demand)
-    uint64_t lsd_cap = (kl.nc == 2 || ctx->v3_lsd_seen) ? (kmer_cap < (1u << 22) ? kmer_cap : kmer_cap / 4) : 0;
-    if (lsd_cap && lsd_cap < ctx->v3_lsd_cap_seen && ctx->v3_lsd_cap_seen <= kmer_cap) lsd_cap = ctx->v3_lsd_cap_seen;
-    int rc = lsd_arrays(lsd_cap);
-    if (rc) return rc;
-    auto lsd_view = [&](uint64_t cap) {
-        uint32_t *aux = ctx->v3_lsd_aux.as<uint32_t>();
-        return cap ? V3Lsd{ctx->rec_a.p, aux, aux + (cap + 1), aux + 2 * (cap + 1), aux + 3 * (cap + 1), cap} : V3Lsd{nullptr, nullptr, nullptr, nullptr, nullptr, 0};
-    };
-    uint64_t *unit_excl = ctx->v3_unit_excl.as<uint64_t>(), *lsd_excl = unit_excl + max_units + 1;
-    lp = v3_group_launch(skr, ent, ctx->units.p, kl, ctx->v3_cap_eff, cutoff, d_ids, id_base, vo, max_units, unit_excl, lsd_excl, ctx->scan_scratch.p, &dm->gc3, ch,
-                         lsd_view(lsd_cap), false, ctx->sm_count, &ctx->prof, st);
-    *launches += lp;
-    CU(cudaGetLastError());
-    if (ch.done) {  // the grouping kernels pack each chunk's totals as {k-mers << 32 | ids}
-        rc = stream_finished_chunks(ctx, sink, ch.n, hm->chunk_totals, 32, hm->lsd_totals);
-        if (rc) return rc;
-    }
-    CU(read_back(ctx, &Misc::gc3, st));
-    if (hm->gc3.overflow == 6u && hm->gc3.lsd_kmers > lsd_cap) {
-        // long spans met no (or too small) sort arrays: allocate them and redo their placement (the staged results are still there)
-        ctx->v3_lsd_seen = true;
-        lsd_cap = hm->gc3.lsd_kmers + hm->gc3.lsd_kmers / 16 + 1024;
-        if (lsd_cap > kmer_cap) lsd_cap = kmer_cap;
-        ctx->v3_lsd_cap_seen = lsd_cap;
-        rc = lsd_arrays(lsd_cap);
-        if (rc) return rc;
-        CU(cudaMemsetAsync(&dm->gc3.overflow, 0, sizeof(unsigned int), st));
-        V3Chunks ch1 = ch;
-        ch1.totals_host = ch1.lsd_totals_host = nullptr;
-        ch1.done = nullptr;
-        lp = v3_group_launch(skr, ent, ctx->units.p, kl, ctx->v3_cap_eff, cutoff, d_ids, id_base, vo, max_units, unit_excl, lsd_excl, ctx->scan_scratch.p, &dm->gc3, ch1,
-                             lsd_view(lsd_cap), true, ctx->sm_count, &ctx->prof, st);
-        *launches += lp;
-        CU(cudaGetLastError());
-        CU(read_back(ctx, &Misc::gc3, st));
-    }
-    ctx->rs.n_units += hm->gc3.n_units;
-    ctx->rs.n_lsd_kmers += hm->gc3.lsd_kmers;
-    if (hm->gc3.overflow) {  // not done: the caller falls back
-        snprintf(ctx->err, sizeof ctx->err, "pipeline 3 gave the batch up (code %u: a (bucket, d) class larger than a unit)", hm->gc3.overflow);
-        return GBIN_OK;
-    }
-    if (hm->gc3.lsd_kmers) {
-        const uint64_t nl = hm->gc3.lsd_kmers;
-        CU(ctx->radix_scratch.ensure(radix_scratch_bytes(nl)));
-        CU(ctx->run_excl.ensure((nl + 2) * 8));
-        CU(ctx->scan_scratch.ensure(group_scan_scratch_bytes(nl + 1024)));
-        lp = v3_lsd_finish(kl, nl, ctx->rec_a.p, ctx->rec_b.p, ctx->radix_scratch.p, ctx->run_excl.as<uint64_t>(), ctx->scan_scratch.p, vo, lsd_view(lsd_cap), ctx->sm_count, &ctx->prof,
-                           st);
-        *launches += lp;
-        CU(cudaGetLastError());
-    }
-    *distinct = hm->gc3.distinct;
-    *S_out = hm->gc3.total_kmers;
-    *N_out = hm->gc3.total_ids;
-    *ok = true;
-    return GBIN_OK;
-}
-
-int run_v3_group(gbin_ctx *ctx, const void *skr, uint64_t n_skr, const int32_t *d_ids, int32_t id_base, cudaStream_t st, gbin_table *out, int *launches,
-                 bool *done, uint64_t *n_inst_out, HostSink *sink = nullptr) {
-    *done = false;
-    const int K = ctx->cfg.kmer_size, M = ctx->cfg.mmer_size;
-    Misc *dm = ctx->misc.as<Misc>();
-    Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
-    KeyLayout kl;
-    int rc = v3_choose_layout(ctx, skr, n_skr, st, &kl, launches);
-    if (rc) return rc;
-    if (n_skr >= (1ull << (32 - kl.cshift))) return GBIN_OK;  // slots are 32-bit
-    memset(&ctx->rs, 0, sizeof ctx->rs);
-    ctx->rs.n_super_kmers = n_skr;
-    ctx->rs.key_nc = (uint32_t)kl.nc;
-    ctx->rs.key_h = (uint32_t)kl.h;
-
-    // ---- entries + level 1: stable sort of the entries by key
-    const uint64_t n_slots = n_skr << kl.cshift;
-    // the two entry buffers of the sort: in donated memory when the caller gave enough of it (the multi-GPU path hands over the
-    // scan's record buffer, dead after the exchange — one allocation of that size less per step), else the context's own
-    const uint64_t ent_bytes = ((n_slots + 2) * 8 + 255) & ~255ull;
-    uint64_t *ent_a_p, *ent_b_p;
-    if (ctx->donated && ctx->donated_bytes >= 2 * ent_bytes && (reinterpret_cast<uintptr_t>(ctx->donated) & 15u) == 0) {
-        ent_a_p = static_cast<uint64_t *>(ctx->donated);
-        ent_b_p = ent_a_p + ent_bytes / 8;
-        if (ctx->ent_a.cap + ctx->ent_b.cap > (1ull << 30)) {  // a large batch on donated memory: the own buffers of an earlier one would only crowd the HBM
-            ctx->ent_a.release();
-            ctx->ent_b.release();
-        }
-    } else {
-        CU(ctx->ent_a.ensure(ent_bytes));
-        CU(ctx->ent_b.ensure(ent_bytes));
-        ent_a_p = ctx->ent_a.as<uint64_t>();
-        ent_b_p = ctx->ent_b.as<uint64_t>();
-    }
-    ctx->donated = nullptr;  // one call only
-    ctx->donated_bytes = 0;
-    CU(ctx->piece_n.ensure((n_slots + 16) * 2));
-    CU(ctx->sorted_info.ensure((n_slots + 16) * 2));
-    bool on = ctx->prof.begin(KK_V3_ENTRIES, st);
-    int lp = v3_make_entries(skr, n_skr, kl, ent_a_p, ctx->piece_n.as<uint16_t>(), &dm->n_real_entries, st);
-    ctx->prof.end(on, lp, st);
-    *launches += lp;
-    CU(cudaGetLastError());
-    CU(ctx->radix_scratch.ensure(radix_scratch_bytes(n_slots)));
-    bool in_b = false;
-    int passes = 0;
-    *launches += radix_sort_entries(ent_a_p, ent_b_p, n_slots, kl.key_bits, ctx->radix_scratch.p, &in_b, &passes, ctx->piece_n.as<uint16_t>(),
-                                    ctx->sorted_info.as<uint16_t>(), &ctx->prof, st, kl.nc == 2 ? &dm->n_real_entries : nullptr);
-    CU(cudaGetLastError());
-    ctx->tm.sort_passes = (uint32_t)passes;
-    const uint64_t *ent = in_b ? ent_b_p : ent_a_p;
-    CU(cudaEventRecord(ctx->ev[EV_SORTED], st));
-    uint64_t n_ent = n_slots;
-    if (kl.nc == 2) {  // empty pieces carry the all-ones key and sort behind everything: plan over the real ones only
-        CU(read_back(ctx, &Misc::n_real_entries, st));
-        n_ent = hm->n_real_entries;
-    }
-
-    // ---- passes: ranges of the sorted entries with at most pass_max k-mer instances each, cut between m-mer buckets
-    std::vector<uint64_t> bounds{0, n_ent};
-    const uint64_t pass_max = ctx->v3_pass_max;
-    if (n_skr * (uint64_t)(K - M + 1) > pass_max) {  // more than one pass is possible: look at the instance counts
-        const uint32_t nt = v3_pass_tiles(n_ent);
-        CU(ctx->scan_scratch.ensure((size_t)nt * 8 + 64));
-        unsigned long long *sums_dev = ctx->scan_scratch.as<unsigned long long>();
-        *launches += v3_pass_tile_sums(ctx->sorted_info.as<uint16_t>(), n_ent, sums_dev, st);
-        std::vector<unsigned long long> sums(nt);
-        CU(cudaMemcpyAsync(sums.data(), sums_dev, (size_t)nt * 8, cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        std::vector<unsigned long long> cuts;
-        unsigned long long acc = 0, all = 0;
-        for (uint32_t t = 0; t < nt; t++) all += sums[t];
-        // a batch of several passes is a batch that crowds the HBM: the workspace of a pass (staging, bounds of the table's growth) scales
-        // with the pass, so such a batch is cut into passes of half the size
-        const uint64_t pass_max = all > 2 * ctx->v3_pass_max ? ctx->v3_pass_max / 2 : ctx->v3_pass_max;
-        for (uint32_t t = 0; t < nt; t++) {
-            if (acc && acc + sums[t] > pass_max) {
-                cuts.push_back((unsigned long long)t * v3_pass_tile_entries());
-                acc = 0;
-            }
-            acc += sums[t];
-        }
-        if (!cuts.empty()) {
-            CU(cudaMemcpyAsync(sums_dev, cuts.data(), cuts.size() * 8, cudaMemcpyHostToDevice, st));
-            *launches += v3_pass_bounds(ent, n_ent, kl.mshift, sums_dev, (uint32_t)cuts.size(), st);
-            CU(cudaMemcpyAsync(cuts.data(), sums_dev, cuts.size() * 8, cudaMemcpyDeviceToHost, st));
-            CU(cudaStreamSynchronize(st));
-            bounds.assign(1, 0);
-            for (unsigned long long c : cuts)
-                if (c > bounds.back() && c < n_ent) bounds.push_back(c);
-            bounds.push_back(n_ent);
-        }
-    }
-    const bool single = bounds.size() == 2;
-    uint64_t S_off = 0, N_off = 0, n_total = 0, distinct = 0;
-    for (size_t p = 0; p + 1 < bounds.size(); p++) {
-        bool ok = false;
-        uint64_t n_p = 0, d_p = 0, S_p = 0, N_p = 0;
-        rc = run_v3_pass(ctx, skr, ent + bounds[p], ctx->sorted_info.as<uint16_t>() + bounds[p], bounds[p + 1] - bounds[p], kl, d_ids, id_base, st, S_off, N_off, single, sink, launches, &ok, &n_p, &d_p, &S_p, &N_p);
-        if (rc) return rc;
-        if (!ok) return GBIN_OK;  // not done: the caller falls back
-        S_off += S_p;
-        N_off += N_p;
-        n_total += n_p;
-        distinct += d_p;
-    }
-    *n_inst_out = n_total;
-    ctx->rs.n_passes = (uint32_t)(bounds.size() - 1);
-    const uint64_t S = S_off, NS = N_off;
-    if (S >= (1ull << 32)) return fail(ctx, GBIN_E_TOO_LARGE, "%llu surviving k-mers in one batch (limit 2^32)", (unsigned long long)S);
-    uint64_t B = 0;
-    rc = emit_bucket_directory(ctx, S, NS, st, launches, &B);
-    if (rc) return rc;
-    *out = device_table(ctx, n_total, distinct, S, NS, B);
-    *done = true;
     return GBIN_OK;
 }
 

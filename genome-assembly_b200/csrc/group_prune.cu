@@ -7,11 +7,30 @@
 //   * keep iff length > ABUNDANCE_CUTOFF             — binning.c:1102
 //   * m-mer buckets that still own a k-mer           — prune_data drops emptied buckets (:1136-1142)
 //   * ids of a group, newest arrival first           — the list walked from its head (:1059-1069)
+#include "gbin_ctx.h"
 #include "gbin_device.cuh"
-#include "gbin_internal.h"
 #include "prefix_scan.cuh"
 
 namespace gbin {
+
+struct GroupWorkspace {  // all device pointers, sized by run_group
+    uint32_t *group_of;     // [n]    group index of every sorted record
+    uint32_t *run_start;    // [n+1]  first record of every group (+ sentinel n)
+    uint32_t *surv_index;   // [n_distinct+1] exclusive count of surviving groups
+    uint64_t *id_offset;    // [n_distinct+1] exclusive sum of surviving run lengths
+    uint32_t *surv_group;   // [n_kmers] group index of surviving k-mer s
+    uint32_t *bucket_of;    // [n_kmers] bucket index of surviving k-mer s
+    void *scan_scratch;     // prefix-scan scratch (u64 elements)
+    GroupCounts *counts;    // device
+    int cutoff;             // ABUNDANCE_CUTOFF (binning.c:12); < 0 keeps everything
+};
+struct TableOut {
+    uint32_t *mmer_codes;
+    uint64_t *mmer_kmer_off;
+    uint64_t *kmer_codes;
+    uint64_t *kmer_id_off;
+    int32_t *read_ids;
+};
 
 template <int KW>
 struct HeadFlag {
@@ -117,7 +136,8 @@ size_t group_scan_scratch_bytes(uint64_t n) { return (scan_scratch_elems(n ? n :
 
 static inline unsigned blocks_for(uint64_t n) { return (unsigned)((n + 255) / 256); }
 
-int group_find_runs(const void *sorted, uint64_t n, int KW, GroupWorkspace &ws, cudaStream_t st) {
+// Phase 1: run-length over sorted records -> group_of, run_start, counts->n_distinct.
+static int group_find_runs(const void *sorted, uint64_t n, int KW, GroupWorkspace &ws, cudaStream_t st) {
     if (n == 0) {
         cudaMemsetAsync(ws.counts, 0, sizeof(GroupCounts), st);
         return 0;
@@ -136,7 +156,8 @@ int group_find_runs(const void *sorted, uint64_t n, int KW, GroupWorkspace &ws, 
     return launches + 1;
 }
 
-int group_prune_offsets(uint64_t n, uint64_t n_distinct, int cutoff, GroupWorkspace &ws, cudaStream_t st) {
+// Phase 2 (needs n_distinct on the host): prune decision + offsets -> counts->n_kmers, n_ids.
+static int group_prune_offsets(uint64_t n, uint64_t n_distinct, int cutoff, GroupWorkspace &ws, cudaStream_t st) {
     (void)n;
     int launches = 0;
     launches += exclusive_scan<uint32_t, SurvFlag>(SurvFlag{ws.run_start, cutoff}, ws.surv_index, n_distinct,
@@ -146,7 +167,8 @@ int group_prune_offsets(uint64_t n, uint64_t n_distinct, int cutoff, GroupWorksp
     return launches;
 }
 
-int group_mark_buckets(const void *sorted, int KW, uint64_t n_distinct, uint64_t n_kmers, GroupWorkspace &ws, cudaStream_t st) {
+// Phase 3 (needs n_kmers on the host): bucket boundaries over surviving k-mers -> counts->n_buckets.
+static int group_mark_buckets(const void *sorted, int KW, uint64_t n_distinct, uint64_t n_kmers, GroupWorkspace &ws, cudaStream_t st) {
     if (n_kmers == 0) {
         cudaMemsetAsync(&ws.counts->n_buckets, 0, sizeof(uint32_t), st);
         return 0;
@@ -164,7 +186,8 @@ int group_mark_buckets(const void *sorted, int KW, uint64_t n_distinct, uint64_t
     return launches;
 }
 
-int group_emit(const void *sorted, uint64_t n, int KW, uint64_t n_distinct, uint64_t n_kmers, uint64_t n_ids, uint64_t n_buckets,
+// Phase 4: emit the flat table.
+static int group_emit(const void *sorted, uint64_t n, int KW, uint64_t n_distinct, uint64_t n_kmers, uint64_t n_ids, uint64_t n_buckets,
                const int32_t *ids_by_arrival, int32_t id_base, GroupWorkspace &ws, const TableOut &out, cudaStream_t st) {
     (void)n_distinct;
     if (n_kmers == 0) {
@@ -185,6 +208,83 @@ int group_emit(const void *sorted, uint64_t n, int KW, uint64_t n_distinct, uint
                                                          out.read_ids);
     }
     return 2;
+}
+
+int run_group(gbin_ctx *ctx, void *recs, void *twin, uint64_t n, const int32_t *d_ids, int32_t id_base, cudaStream_t st,
+              gbin_table *out, int *launches, cudaEvent_t ev_sorted) {
+    const int KW = ctx->KW, K = ctx->cfg.kmer_size, M = ctx->cfg.mmer_size, cutoff = ctx->cfg.abundance_cutoff;
+    Misc *dm = ctx->misc.as<Misc>();
+    Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
+    CU(ctx->radix_scratch.ensure(radix_scratch_bytes(n)));
+    bool in_b = false;
+    int passes = 0;
+    *launches += radix_sort_records(recs, twin, n, KW, K, M, ctx->radix_scratch.p, &in_b, &passes, &ctx->prof, st);
+    CU(cudaGetLastError());
+    ctx->tm.sort_passes = (uint32_t)passes;
+    const void *sorted = in_b ? twin : recs;
+    if (ev_sorted) CU(cudaEventRecord(ev_sorted, st));
+
+    GroupWorkspace ws{};
+    CU(ctx->group_of.ensure((n + 1) * sizeof(uint32_t)));
+    CU(ctx->run_start.ensure((n + 2) * sizeof(uint32_t)));
+    CU(ctx->scan_scratch.ensure(group_scan_scratch_bytes(n)));
+    ws.group_of = ctx->group_of.as<uint32_t>();
+    ws.run_start = ctx->run_start.as<uint32_t>();
+    ws.scan_scratch = ctx->scan_scratch.p;
+    ws.counts = &dm->grp.counts;
+    ws.cutoff = cutoff;
+
+    bool on = ctx->prof.begin(KK_RUNS, st);
+    int lg = group_find_runs(sorted, n, KW, ws, st);
+    ctx->prof.end(on, lg, st);
+    *launches += lg;
+    CU(cudaGetLastError());
+    CU(read_back(ctx, &Misc::grp, st));
+    if (hm->grp.bad_bases) return fail(ctx, GBIN_E_NON_ACGT, "%llu bases other than A/C/G/T in the batch", hm->grp.bad_bases);
+    const uint64_t G = hm->grp.counts.n_distinct;
+
+    uint64_t S = 0, NS = 0, B = 0;
+    if (G) {
+        CU(ctx->surv_index.ensure((G + 1) * sizeof(uint32_t)));
+        CU(ctx->id_offset.ensure((G + 1) * sizeof(uint64_t)));
+        ws.surv_index = ctx->surv_index.as<uint32_t>();
+        ws.id_offset = ctx->id_offset.as<uint64_t>();
+        on = ctx->prof.begin(KK_PRUNE, st);
+        lg = group_prune_offsets(n, G, cutoff, ws, st);
+        ctx->prof.end(on, lg, st);
+        *launches += lg;
+        CU(cudaGetLastError());
+        CU(read_back(ctx, &Misc::grp, st));
+        S = hm->grp.counts.n_kmers;
+        NS = hm->grp.counts.n_ids;
+    }
+    if (S) {
+        CU(ctx->surv_group.ensure(S * sizeof(uint32_t)));
+        CU(ctx->bucket_of.ensure(S * sizeof(uint32_t)));
+        ws.surv_group = ctx->surv_group.as<uint32_t>();
+        ws.bucket_of = ctx->bucket_of.as<uint32_t>();
+        on = ctx->prof.begin(KK_PRUNE, st);
+        lg = group_mark_buckets(sorted, KW, G, S, ws, st);
+        ctx->prof.end(on, lg, st);
+        *launches += lg;
+        CU(cudaGetLastError());
+        CU(read_back(ctx, &Misc::grp, st));
+        B = hm->grp.counts.n_buckets;
+    }
+    CU(ctx->o_mmer_codes.ensure((B + 1) * sizeof(uint32_t)));
+    CU(ctx->o_mmer_kmer_off.ensure((B + 1) * sizeof(uint64_t)));
+    CU(ctx->o_kmer_codes.ensure((S * KW + 1) * sizeof(uint64_t)));
+    CU(ctx->o_kmer_id_off.ensure((S + 1) * sizeof(uint64_t)));
+    CU(ctx->o_read_ids.ensure((NS + 1) * sizeof(int32_t)));
+    TableOut to{ctx->o_mmer_codes.as<uint32_t>(), ctx->o_mmer_kmer_off.as<uint64_t>(), ctx->o_kmer_codes.as<uint64_t>(),
+                ctx->o_kmer_id_off.as<uint64_t>(), ctx->o_read_ids.as<int32_t>()};
+    on = ctx->prof.begin(KK_EMIT, st);
+    lg = group_emit(sorted, n, KW, G, S, NS, B, d_ids, id_base, ws, to, st);
+    ctx->prof.end(on, lg, st);
+    *launches += lg;
+    CU(cudaGetLastError());
+    *out = device_table(ctx, n, G, S, NS, B);
+    return GBIN_OK;
 }
 
 }  // namespace gbin

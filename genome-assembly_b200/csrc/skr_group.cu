@@ -19,8 +19,8 @@
 //      (prune_data drops buckets that lost all their k-mers, binning.c:1136-1142).
 // Anything that does not fit (a single key with more instances than a unit can hold, skewed
 // sub-units) raises an overflow flag; the caller then runs the batch through pipeline v1.
+#include "gbin_ctx.h"
 #include "gbin_device.cuh"
-#include "gbin_internal.h"
 #include "prefix_scan.cuh"
 #include "lookback.cuh"
 #include "skr.cuh"
@@ -114,7 +114,6 @@ struct UnitsOfRun {  // how many units start at run r
     }
 };
 
-struct GroupCounters;
 __device__ __forceinline__ unsigned int *big_counter(GroupCounters *gc);
 __device__ __forceinline__ unsigned int *big_inst_counter(GroupCounters *gc);
 
@@ -414,16 +413,6 @@ struct GroupOut {
     uint64_t *stg_codes;    // [kmer_cap * KW]
     uint32_t *stg_mmer;     // [kmer_cap]
     uint32_t *stg_off;      // [kmer_cap] start of the k-mer's id list inside its unit
-};
-struct GroupCounters {
-    unsigned long long distinct;
-    unsigned long long total_kmers, total_ids;  // written by the last unit
-    unsigned int overflow;
-    unsigned int ticket;
-    unsigned int n_units;
-    unsigned int n_big;     // buckets larger than a unit (work list of partition_big_runs_kernel)
-    unsigned int big_inst;  // k-mer instances in those buckets (allocation cursor of the scratch arrays)
-    unsigned int pad[3];
 };
 
 __device__ __forceinline__ unsigned int *big_counter(GroupCounters *gc) { return &gc->n_big; }
@@ -903,19 +892,16 @@ __global__ void empty_table_kernel2(uint64_t *mmer_kmer_off, uint64_t *kmer_id_o
 
 static PlanParams plan_params() { return PlanParams{G_UNIT_CAP, G_UNIT_CAP / 2, G_UNIT_CAP / 2, G_UNIT_CAP / 2}; }
 
-size_t skr_group_smem_bytes(int KW) {
+static size_t skr_group_smem_bytes(int KW) {
     const size_t cap = G_UNIT_CAP;
     const size_t hs = cap > 2048 ? 8192 : (cap > 1024 ? 4096 : 2048);  // hash slots, as in the kernel
     return KW * cap * 8 + cap * 4 * 2 + hs * 4 + cap * 4 + cap * 2 * 3 + 64;
 }
 
-uint64_t skr_max_units(uint64_t n_inst, uint64_t n_runs) { return n_inst / (G_UNIT_CAP / 4) + 2 * n_runs + 8; }
-size_t skr_unit_bytes() { return sizeof(Unit); }
-uint64_t skr_max_big_runs(uint64_t n_inst) { return n_inst / (uint64_t)G_UNIT_CAP + 2; }
 
 // Phase A (needs n_skr on the host): instance prefix and m-mer run starts in one fused scan.
 // both64: [n_skr + 1] u64 scratch; scratch64: prefix-scan scratch. *n_inst_dev / *n_runs_dev receive the totals.
-int skr_plan_runs(const uint64_t *side, uint64_t n_skr, uint32_t *inst_prefix /*[n+1]*/, uint64_t *both64, uint32_t *run_start /*[n+1]*/,
+static int skr_plan_runs(const uint64_t *side, uint64_t n_skr, uint32_t *inst_prefix /*[n+1]*/, uint64_t *both64, uint32_t *run_start /*[n+1]*/,
                   uint64_t *scratch64, uint32_t *n_inst_dev, uint32_t *n_runs_dev, cudaStream_t st) {
     int l = exclusive_scan<uint64_t, SkrCountAndHead>(SkrCountAndHead{side}, both64, n_skr, scratch64, both64 + n_skr, st);
     skr_run_starts_kernel<<<(unsigned)((n_skr + 255) / 256), 256, 0, st>>>(side, n_skr, both64, both64 + n_skr, inst_prefix, run_start, n_inst_dev,
@@ -924,7 +910,7 @@ int skr_plan_runs(const uint64_t *side, uint64_t n_skr, uint32_t *inst_prefix /*
 }
 
 // Phase B (needs n_runs on the host): units. small_prefix / unit_base are [n_runs] scratch arrays.
-int skr_plan_units(const void *skr_sorted, int K, const uint32_t *inst_prefix, const uint32_t *run_start, uint64_t n_runs,
+static int skr_plan_units(const void *skr_sorted, int K, const uint32_t *inst_prefix, const uint32_t *run_start, uint64_t n_runs,
                    uint32_t *small_prefix, uint32_t *unit_base, uint32_t *scratch, void *units, uint64_t max_units, void *gc_dev,
                    uint32_t *big_list, uint64_t *big_k0, uint64_t *big_k1, uint32_t *big_arr, int sm_count, cudaStream_t st) {
     RunView rv{run_start, inst_prefix};
@@ -959,48 +945,145 @@ __global__ void publish_chunk_total_kernel(const unsigned long long *__restrict_
     chunk_totals[chunk] = end ? (unit_state[end - 1] & LKB_VALUE_MASK) : 0ull;
 }
 
-int skr_group_launch(const void *skr_sorted, int K, int cutoff, const uint32_t *inst_prefix, const void *units, unsigned long long *unit_state,
-                     uint64_t max_units, const SkrGroupChunks &ch, void *gc_dev, uint64_t *big_k0, uint64_t *big_k1, uint32_t *big_arr, const int32_t *ids_by_arrival, int32_t id_base, uint64_t *kmer_codes,
-                     uint32_t *kmer_mmer, uint64_t *kmer_id_off, int32_t *read_ids, uint64_t kmer_cap, uint64_t id_cap, int32_t *stg_ids, uint64_t *stg_codes,
-                     uint32_t *stg_mmer, uint32_t *stg_off, int sm_count, cudaStream_t st) {
-    const int KW = K <= 32 ? 1 : 2;
+int run_v2_group(gbin_ctx *ctx, void *skr, void *twin, uint64_t n_skr, const int32_t *d_ids, int32_t id_base, cudaStream_t st, gbin_table *out,
+                 int *launches, bool *done, uint64_t *n_inst_out, HostSink *sink) {
+    *done = false;
+    const int K = ctx->cfg.kmer_size, M = ctx->cfg.mmer_size, cutoff = ctx->cfg.abundance_cutoff, KW = ctx->KW;
+    const int NW = K <= 32 ? 8 : 12;
+    Misc *dm = ctx->misc.as<Misc>();
+    Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
+
+    // ---- level 1: stable sort of the records by m-mer code
+    CU(ctx->radix_scratch.ensure(radix_scratch_bytes(n_skr)));
+    bool in_b = false;
+    int passes = 0;
+    CU(ctx->skr_side.ensure((n_skr + 2) * 8));
+    *launches += radix_sort_skr_by_mmer(skr, twin, n_skr, NW, M, ctx->radix_scratch.p, &in_b, &passes, ctx->skr_side.as<uint64_t>(), &ctx->prof, st);
+    CU(cudaGetLastError());
+    ctx->tm.sort_passes = (uint32_t)passes;
+    const void *sorted = in_b ? twin : skr;
+    CU(cudaEventRecord(ctx->ev[EV_SORTED], st));
+
+    // ---- plan: instance prefix, m-mer runs, units
+    CU(ctx->inst_prefix.ensure((n_skr + 2) * 4));
+    CU(ctx->run_excl.ensure((n_skr + 2) * 8));
+    CU(ctx->skr_run_start.ensure((n_skr + 2) * 4));
+    CU(ctx->scan_scratch.ensure(group_scan_scratch_bytes(n_skr)));
+    bool on = ctx->prof.begin(KK_SKR_PLAN, st);
+    int lp = skr_plan_runs(ctx->skr_side.as<uint64_t>(), n_skr, ctx->inst_prefix.as<uint32_t>(), ctx->run_excl.as<uint64_t>(), ctx->skr_run_start.as<uint32_t>(),
+                           ctx->scan_scratch.as<uint64_t>(), &dm->plan.n_inst, &dm->plan.n_runs, st);
+    ctx->prof.end(on, lp, st);
+    *launches += lp;
+    CU(cudaGetLastError());
+    CU(read_back(ctx, &Misc::plan, st));
+    const uint64_t n_runs = hm->plan.n_runs, n = hm->plan.n_inst;
+    *n_inst_out = n;
+    ctx->rs.n_super_kmers = n_skr;
+    ctx->rs.n_mmer_runs = n_runs;
+    const uint64_t max_units = n / (G_UNIT_CAP / 4) + 2 * n_runs + 8;
+    CU(ctx->small_prefix.ensure((n_runs + 1) * 4));
+    CU(ctx->unit_base.ensure((n_runs + 1) * 4));
+    CU(ctx->units.ensure(max_units * sizeof(Unit)));
+    CU(ctx->unit_state.ensure(max_units * 8));
+    CU(ctx->big_list.ensure((n / (uint64_t)G_UNIT_CAP + 2) * 8));  // buckets larger than a unit
+    CU(ctx->big_k0.ensure((n + 1) * 8));
+    if (KW == 2) CU(ctx->big_k1.ensure((n + 1) * 8));
+    CU(ctx->big_arr.ensure((n + 1) * 4));
+    CU(ctx->scan_scratch.ensure(group_scan_scratch_bytes(n / 2 + n_runs + 1024)));
+    on = ctx->prof.begin(KK_SKR_PLAN, st);
+    lp = skr_plan_units(sorted, K, ctx->inst_prefix.as<uint32_t>(), ctx->skr_run_start.as<uint32_t>(), n_runs, ctx->small_prefix.as<uint32_t>(),
+                        ctx->unit_base.as<uint32_t>(), ctx->scan_scratch.as<uint32_t>(), ctx->units.p, max_units, &dm->gc, ctx->big_list.as<uint32_t>(),
+                        ctx->big_k0.as<uint64_t>(), ctx->big_k1.as<uint64_t>(), ctx->big_arr.as<uint32_t>(), ctx->sm_count, st);
+    ctx->prof.end(on, lp, st);
+    *launches += lp;
+    CU(cudaGetLastError());
+
+    // ---- level 2 + prune + emit. Output bounds: a surviving k-mer has more than `cutoff` instances.
+    const uint64_t kmer_cap = cutoff >= 0 ? n / ((uint64_t)cutoff + 1) + 1 : n + 1;
+    CU(ctx->o_kmer_codes.ensure((kmer_cap * KW + 1) * sizeof(uint64_t)));
+    CU(ctx->o_kmer_mmer.ensure((kmer_cap + 1) * sizeof(uint32_t)));
+    CU(ctx->o_kmer_id_off.ensure((kmer_cap + 2) * sizeof(uint64_t)));
+    CU(ctx->o_read_ids.ensure((n + 1) * sizeof(int32_t)));
+    CU(ctx->stg_ids.ensure((n + 1) * sizeof(int32_t)));
+    CU(ctx->stg_codes.ensure((kmer_cap * KW + 1) * sizeof(uint64_t)));
+    CU(ctx->stg_mmer.ensure((kmer_cap + 1) * sizeof(uint32_t)));
+    CU(ctx->stg_off.ensure((kmer_cap + 1) * sizeof(uint32_t)));
+    // The grouping runs as n_ch consecutive launches over equal ranges of the unit list, one chained scan across them.  On the host
+    // path the end offsets of every chunk ({k-mers << 31 | ids}) are published after it, so that finished parts of the table stream out.
+    const bool stream = sink && sink->chunks > 1;
+    const uint32_t n_ch = stream ? (uint32_t)sink->chunks : 1u;
     const size_t smem = skr_group_smem_bytes(KW);
+    on = ctx->prof.begin(KK_SKR_GROUP, st);
+    unsigned long long *unit_state = ctx->unit_state.as<unsigned long long>();
     cudaMemsetAsync(unit_state, 0, sizeof(unsigned long long) * max_units, st);
-    cudaMemsetAsync(ch.tickets, 0, sizeof(uint32_t) * ch.n, st);
-    GroupOut out{kmer_codes, kmer_mmer, kmer_id_off, read_ids, kmer_cap, id_cap, stg_ids, stg_codes, stg_mmer, stg_off};
-    GroupCounters *gc = static_cast<GroupCounters *>(gc_dev);
-    const uint32_t *s = static_cast<const uint32_t *>(skr_sorted);
-    const Unit *un = static_cast<const Unit *>(units);
+    cudaMemsetAsync(dm->chunk_tickets, 0, sizeof(uint32_t) * n_ch, st);
+    const GroupOut go{ctx->o_kmer_codes.as<uint64_t>(), ctx->o_kmer_mmer.as<uint32_t>(), ctx->o_kmer_id_off.as<uint64_t>(), ctx->o_read_ids.as<int32_t>(), kmer_cap,
+                      n, ctx->stg_ids.as<int32_t>(), ctx->stg_codes.as<uint64_t>(), ctx->stg_mmer.as<uint32_t>(), ctx->stg_off.as<uint32_t>()};
+    const BigScratch big{ctx->big_k0.as<uint64_t>(), ctx->big_k1.as<uint64_t>(), ctx->big_arr.as<uint32_t>()};
     auto launch = [&](auto kern, int threads, int ctas_per_sm) {
         cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        for (uint32_t c = 0; c < ch.n; c++) {
-            kern<<<sm_count * ctas_per_sm, threads + 32, smem, st>>>(s, inst_prefix, un, BigScratch{big_k0, big_k1, big_arr}, K, cutoff, ids_by_arrival,
-                                                                id_base, out, unit_state, gc, c, ch.n, ch.tickets);
-            if (ch.totals_dev) {
-                publish_chunk_total_kernel<<<1, 1, 0, st>>>(unit_state, gc, c, ch.n, ch.totals_dev);
-                if (ch.totals_host) cudaMemcpyAsync(ch.totals_host + c, ch.totals_dev + c, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st);
-                if (ch.done) cudaEventRecord(ch.done[c], st);
+        for (uint32_t c = 0; c < n_ch; c++) {
+            kern<<<ctx->sm_count * ctas_per_sm, threads + 32, smem, st>>>(static_cast<const uint32_t *>(sorted), ctx->inst_prefix.as<uint32_t>(),
+                                                                          ctx->units.as<Unit>(), big, K, cutoff, d_ids, id_base, go, unit_state, &dm->gc, c,
+                                                                          n_ch, dm->chunk_tickets);
+            if (stream) {
+                publish_chunk_total_kernel<<<1, 1, 0, st>>>(unit_state, &dm->gc, c, n_ch, dm->chunk_totals);
+                cudaMemcpyAsync(hm->chunk_totals + c, dm->chunk_totals + c, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st);
+                cudaEventRecord(ctx->ev_chunk[c], st);
             }
         }
     };
     const int per_sm = (int)((size_t)(227 * 1024) / (smem + 1024));  // CTAs per SM that shared memory allows
     if (KW == 1) launch(skr_group_kernel<2, 1, G_UNIT_CAP, 256>, 256, per_sm < 4 ? per_sm : 4);
     else launch(skr_group_kernel<4, 2, G_UNIT_CAP, 256>, 256, per_sm < 4 ? per_sm : 4);
-    return (int)(ch.totals_dev ? 2 * ch.n : ch.n);
+    lp = (int)(stream ? 2 * n_ch : n_ch);
+    ctx->prof.end(on, lp, st);
+    *launches += lp;
+    CU(cudaGetLastError());
+    if (stream) {
+        const int rc = stream_finished_chunks(ctx, sink, n_ch, hm->chunk_totals, 31, nullptr);
+        if (rc) return rc;
+    }
+    CU(read_back(ctx, &Misc::gc, st));
+    ctx->rs.n_units = hm->gc.n_units;
+    if (hm->gc.overflow) {  // a unit did not fit shared memory: this batch goes through pipeline v1
+        ctx->fallbacks++;
+        return GBIN_OK;
+    }
+    const uint64_t S = hm->gc.total_kmers, NS = hm->gc.total_ids;
+    uint64_t B = 0;
+    const int rc = emit_bucket_directory(ctx, S, NS, st, launches, &B);
+    if (rc) return rc;
+    *out = device_table(ctx, n, hm->gc.distinct, S, NS, B);
+    *done = true;
+    return GBIN_OK;
 }
 
-// Bucket directory over the n_kmers emitted k-mers. bucket_excl: [n_kmers] scratch. *n_buckets_dev receives B.
-int skr_emit_buckets(const uint32_t *kmer_mmer, uint64_t n_kmers, uint64_t n_ids, uint32_t *bucket_excl, uint32_t *scratch,
-                     uint32_t *mmer_codes, uint64_t *mmer_kmer_off, uint64_t *kmer_id_off, uint32_t *n_buckets_dev, cudaStream_t st) {
-    if (n_kmers == 0) {
-        cudaMemsetAsync(n_buckets_dev, 0, sizeof(uint32_t), st);
-        empty_table_kernel2<<<1, 1, 0, st>>>(mmer_kmer_off, kmer_id_off);
-        return 1;
+int emit_bucket_directory(gbin_ctx *ctx, uint64_t S, uint64_t NS, cudaStream_t st, int *launches, uint64_t *B) {
+    Misc *dm = ctx->misc.as<Misc>();
+    Misc *hm = static_cast<Misc *>(ctx->h_misc.p);
+    CU(ctx->bucket_excl.ensure((S + 1) * 4));
+    CU(ctx->o_mmer_codes.ensure((S + 1) * sizeof(uint32_t)));
+    CU(ctx->o_mmer_kmer_off.ensure((S + 2) * sizeof(uint64_t)));
+    CU(ctx->scan_scratch.ensure(group_scan_scratch_bytes(S + 1024)));
+    const bool on = ctx->prof.begin(KK_EMIT, st);
+    int lp = 1;
+    if (S == 0) {
+        cudaMemsetAsync(&dm->n_buckets_dev, 0, sizeof(uint32_t), st);
+        empty_table_kernel2<<<1, 1, 0, st>>>(ctx->o_mmer_kmer_off.as<uint64_t>(), ctx->o_kmer_id_off.as<uint64_t>());
+    } else {
+        const uint32_t *kmer_mmer = ctx->o_kmer_mmer.as<uint32_t>();
+        lp += exclusive_scan<uint32_t, KmerBucketHead>(KmerBucketHead{kmer_mmer}, ctx->bucket_excl.as<uint32_t>(), S, ctx->scan_scratch.as<uint32_t>(),
+                                                       &dm->n_buckets_dev, st);
+        emit_buckets_kernel<<<(unsigned)((S + 255) / 256), 256, 0, st>>>(kmer_mmer, ctx->bucket_excl.as<uint32_t>(), S, NS, ctx->o_mmer_codes.as<uint32_t>(),
+                                                                        ctx->o_mmer_kmer_off.as<uint64_t>(), ctx->o_kmer_id_off.as<uint64_t>());
     }
-    int l = exclusive_scan<uint32_t, KmerBucketHead>(KmerBucketHead{kmer_mmer}, bucket_excl, n_kmers, scratch, n_buckets_dev, st);
-    emit_buckets_kernel<<<(unsigned)((n_kmers + 255) / 256), 256, 0, st>>>(kmer_mmer, bucket_excl, n_kmers, n_ids, mmer_codes, mmer_kmer_off,
-                                                                          kmer_id_off);
-    return l + 1;
+    ctx->prof.end(on, lp, st);
+    *launches += lp;
+    CU(cudaGetLastError());
+    CU(read_back(ctx, &Misc::n_buckets_dev, st));
+    *B = hm->n_buckets_dev;
+    return GBIN_OK;
 }
 
 }  // namespace gbin
